@@ -205,3 +205,111 @@ def load_sentis(path_or_bytes) -> SentisModel:
         operators=operators,
         blob=blob,
     )
+
+
+class _FBWriter:
+    """Minimal FlatBuffer builder for the layout _FB reads: objects are prepended (children before the tables that point
+    at them, so every offset points forward); positions are counted from the end of the buffer."""
+
+    def __init__(self):
+        self.parts, self.size = [], 0
+
+    def _prepend(self, data: bytes) -> int:
+        self.parts.append(bytes(data))
+        self.size += len(data)
+        return self.size
+
+    def scalars(self, fmt: str, items) -> int:
+        items = list(items)
+        return self._prepend(struct.pack("<I%d%s" % (len(items), fmt), len(items), *items))
+
+    def bytes_(self, data: bytes) -> int:
+        return self._prepend(struct.pack("<I", len(data)) + bytes(data))
+
+    def string(self, s: str) -> int:
+        return self.bytes_(s.encode("utf-8"))
+
+    def offsets(self, targets) -> int:
+        targets = list(targets)
+        pos = self.size + 4 + 4 * len(targets)
+        return self._prepend(struct.pack("<I%dI" % len(targets), len(targets),
+                                         *(pos - 4 - 4 * i - q for i, q in enumerate(targets))))
+
+    def table(self, fields) -> int:
+        """fields[i]: None (absent), (struct format, value), or the position of an object written earlier."""
+        body, slots, refs = bytearray(), [], []
+        for f in fields:
+            if f is None:
+                slots.append(0)
+                continue
+            slots.append(4 + len(body))
+            if isinstance(f, tuple):
+                body += struct.pack("<" + f[0], f[1])
+            else:
+                refs.append((4 + len(body), f))
+                body += bytes(4)
+        pos = self.size + 4 + len(body)
+        for off, q in refs:
+            struct.pack_into("<I", body, off - 4, pos - off - q)
+        vt = struct.pack("<HH%dH" % len(slots), 4 + 2 * len(slots), 4 + len(body), *slots)
+        self._prepend(vt + struct.pack("<i", len(vt)) + bytes(body))
+        return pos
+
+    def finish(self, root: int) -> bytes:
+        self._prepend(struct.pack("<I", self.size + 4 - root))
+        return b"".join(reversed(self.parts))
+
+
+def write_sentis(convs, iou_threshold: float, score_threshold: float, chunk_bytes: int = 1 << 20) -> bytes:
+    """A `.sentis` container in the layout load_sentis reads, holding what the loaders take from the reference's asset:
+    per convolution a DequantizeUint8 chain for the weights and one for the bias feeding a Conv / ConvTranspose chain,
+    the bias-free DFL convolution (weights 0..15), and a NonMaxSuppression chain whose iou / score thresholds are 0-d
+    f32 constants.  convs[i] = (w_q uint8, w_scale, w_zp, b_q uint8, b_scale, b_zp, transposed).  The weight blob is
+    split into chunks of `chunk_bytes`."""
+    fb, blob = _FBWriter(), bytearray()
+    operators = ["DequantizeUint8", "Conv", "ConvTranspose", "NonMaxSuppression"]
+    values, chains = [], []
+
+    def tensor(dtype, shape, data=None):           # -> value id; data: bytes of a constant
+        if data is not None:
+            off = len(blob)
+            blob.extend(data)
+        body = fb.table([("B", dtype), ("i", len(data) if data is not None else 0), fb.scalars("i", shape),
+                         ("I", int(data is not None)), ("i", off if data is not None else 0), ("B", 0)])
+        values.append(fb.table([("B", 6), body]))
+        return len(values) - 1
+
+    def number(v):
+        values.append(fb.table([("B", 3), fb.table([("f", v)])]) if isinstance(v, float) else
+                      fb.table([("B", 2), fb.table([("i", v)])]))
+        return len(values) - 1
+
+    def chain(op, ins, outs, args=()):
+        call = fb.table([("i", operators.index(op)), fb.scalars("i", args)])
+        chains.append(fb.table([fb.scalars("i", ins), fb.scalars("i", outs), fb.offsets([fb.table([None, call])])]))
+
+    def dequant(q, scale, zp):
+        q = np.ascontiguousarray(q, np.uint8)
+        out = tensor(0, q.shape)
+        chain("DequantizeUint8", [tensor(3, q.shape, q.tobytes())], [out], [number(float(scale)), number(int(zp))])
+        return out
+
+    x = tensor(0, [1, 3, 640, 640])
+    for i, (wq, ws, wz, bq, bs, bz, transposed) in enumerate(convs):
+        w, b = dequant(wq, ws, wz), dequant(bq, bs, bz)
+        chain("ConvTranspose" if transposed else "Conv", [x, w, b], [tensor(0, [])])
+        if i == len(convs) - 1:
+            chain("Conv", [x, dequant(np.arange(16, dtype=np.uint8).reshape(1, 16, 1, 1), 1.0, 0)], [tensor(0, [])])
+    thr = [tensor(0, [], np.float32(t).tobytes()) for t in (iou_threshold, score_threshold)]
+    chain("NonMaxSuppression", [x, x, -1] + thr, [tensor(1, [])])
+
+    ops = [fb.table([fb.string(op)]) for op in operators]
+    plan = fb.table([None, fb.offsets(values), fb.scalars("i", [x]), fb.offsets([fb.string("images")]), fb.scalars("i", []),
+                     fb.offsets([]), fb.offsets(chains), fb.offsets(ops)])
+    program = fb.finish(fb.table([("I", 1), plan]))
+    out = [struct.pack("<I", len(program)), program]
+    for start in range(0, len(blob), chunk_bytes):
+        cw = _FBWriter()
+        chunk = cw.finish(cw.table([cw.bytes_(blob[start:start + chunk_bytes])]))
+        out += [struct.pack("<I", len(chunk)), chunk]
+    return b"".join(out)

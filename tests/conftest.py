@@ -42,6 +42,25 @@ def golden(lib):
 
 
 @pytest.fixture(scope="session")
+def golden_sentis(golden):
+    """The golden XRSW pack (the reference asset's uint8 tensors with their scale / zero point) put back into a .sentis
+    container with the asset's NMS thresholds (SURVEY.md fact 3): what the asset's loaders read, without the asset."""
+    from oracle.sentis import write_sentis
+    from xr_image_segmentation_b200 import weights as W
+    pack = golden["model"].pack
+    _, _, n, _, payload, _ = W.HEADER.unpack_from(pack, 0)
+    convs = []
+    for i in range(n):
+        (_, cout, cin_g, k, _, _, _, tr, dtype, ws, wz, bs, bz, w_off, b_off) = \
+            W.RECORD.unpack_from(pack, W.HEADER.size + i * W.RECORD.size)
+        assert dtype == 3
+        shape = (cin_g, cout, k, k) if tr else (cout, cin_g, k, k)
+        wq = np.frombuffer(pack, np.uint8, int(np.prod(shape)), payload + w_off).reshape(shape)
+        convs.append((wq, ws, wz, np.frombuffer(pack, np.uint8, cout, payload + b_off), bs, bz, bool(tr)))
+    return write_sentis(convs, 0.43, 0.301)
+
+
+@pytest.fixture(scope="session")
 def golden_weights(golden):
     from xr_image_segmentation_b200 import weights as W
     scale, layers = W.read_pack(golden["model"].pack)

@@ -135,18 +135,14 @@ def test_shard_range_and_merge():
 
 
 # ---- .sentis loader inside the library (SURVEY.md §8f N2) ------------------------------------------------------------
-SENTIS = "/root/reference/Assets/Resources/Model/yolo11n-seg-sentis.sentis"
-
-
-@pytest.mark.skipif(not os.path.exists(SENTIS), reason="the reference asset only exists in the build container")
-def test_sentis_loader_matches_oracle_reader_and_golden_pack(lib, golden):
+def test_sentis_loader_matches_oracle_reader_and_golden_pack(lib, golden, golden_sentis):
     """The C++ FlatBuffer walk + uint8 dequantization (csrc/sentis.cuh) against the oracle's Python reader and the committed
-    XRSW re-container of the same asset: every convolution, bit for bit; thresholds as decoded in SURVEY.md fact 3."""
+    XRSW pack the container was written from: every convolution, bit for bit; thresholds as decoded in SURVEY.md fact 3."""
     import ctypes as C
 
     from oracle.sentis import load_sentis
     from xr_image_segmentation_b200 import weights as W
-    data = open(SENTIS, "rb").read()
+    data = golden_sentis
     buf = C.create_string_buffer(data, len(data))
     ptr = C.cast(buf, C.c_void_p)
     n, iou, sc = C.c_int32(), C.c_float(), C.c_float()
@@ -174,10 +170,9 @@ def test_sentis_loader_matches_oracle_reader_and_golden_pack(lib, golden):
     assert I.ModelLoader.Load(data).scale == "n"
 
 
-@pytest.mark.skipif(not os.path.exists(SENTIS), reason="the reference asset only exists in the build container")
-def test_sentis_loader_rejects_corrupt_input(lib):
+def test_sentis_loader_rejects_corrupt_input(lib, golden_sentis):
     import ctypes as C
-    data = bytearray(open(SENTIS, "rb").read())
+    data = bytearray(golden_sentis)
     n = C.c_int32()
 
     def info(b):

@@ -1,8 +1,6 @@
 """CPU tests pinning the ORACLE: (1) against the committed golden vectors, which were produced by the interpreter
-over the reference asset's own 499-chain graph (tests/golden/make_golden.py); (2) against the reference asset itself
-when /root/reference is present (build container only); (3) properties / hand-computed cases of the restated C#."""
-import os
-
+over the reference asset's own 499-chain graph (tests/golden/make_golden.py); (2) its .sentis reader against the golden
+weight pack; (3) properties / hand-computed cases of the restated C#."""
 import numpy as np
 import pytest
 import torch
@@ -11,7 +9,6 @@ from oracle import postprocess as pp
 from oracle import preprocess as pre
 from oracle import yolo11seg as Y
 
-REF_SENTIS = "/root/reference/Assets/Resources/Model/yolo11n-seg-sentis.sentis"
 NAMES = ["coco139", "coco632", "coco2006", "coco4495", "coco7108", "bus"]   # all six sample frames of the reference
 
 
@@ -55,31 +52,14 @@ def test_csharp_postprocess_matches_golden(golden, oracle_runs, name):
     assert np.mean(np.unpackbits(np.packbits(dm.astype(bool), axis=-1) ^ exp[f"{name}.draw_mask_bits"])) <= 1e-4
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SENTIS), reason="reference asset only exists in the build container")
-def test_graph_interpreter_vs_generic_on_reference_asset(golden):
-    from oracle.graph import GraphInterpreter, V_HEAD_RAW, V_KEEP, V_PROTO
+def test_xrsw_pack_roundtrip_matches_reference_dequant(golden_sentis, golden_weights):
+    """The pack keeps the asset's uint8 tensors: put back into a .sentis container, the oracle's own dequantization of
+    them gives the pack's weights."""
     from oracle.sentis import load_sentis
-    m = load_sentis(REF_SENTIS)
-    assert len(m.chains) == 499 and len(m.values) == 1990 and m.output_names == ["output_0", "output_1", "output_2", "output_3"]
-    w = Y.weights_from_sentis(m)
-    x = torch.from_numpy(pre.to_tensor(golden["inputs"]["coco632"]))
-    out = GraphInterpreter(m).run(x, keep={V_HEAD_RAW, V_KEEP, V_PROTO})
-    res, raw = Y.run_model(w, x, "n")
-    assert res[0]["keep"].tolist() == out[V_KEEP].tolist()
-    head = torch.cat([raw["box_logits"][0], raw["cls_logits"][0]], 1).T
-    assert torch.equal(head, out[V_HEAD_RAW][0])
-    np.testing.assert_allclose(res[0]["boxes"], out[m.outputs[0]].numpy(), atol=1e-3)
-    np.testing.assert_allclose(res[0]["masks"], out[m.outputs[3]].numpy(), atol=1e-5)
-
-
-def test_xrsw_pack_roundtrip_matches_reference_dequant(golden, golden_weights):
-    """The pack keeps the asset's uint8 tensors: dequantized values must equal the oracle's own dequantization."""
-    if os.path.exists(REF_SENTIS):
-        from oracle.sentis import load_sentis
-        ref = Y.weights_from_sentis(load_sentis(REF_SENTIS))
-        assert len(ref) == len(golden_weights) == 100
-        for (w0, b0), (w1, b1) in zip(ref, golden_weights):
-            assert np.array_equal(w0, w1) and np.array_equal(b0, b1)
+    ref = Y.weights_from_sentis(load_sentis(golden_sentis))
+    assert len(ref) == len(golden_weights) == 100
+    for (w0, b0), (w1, b1) in zip(ref, golden_weights):
+        assert np.array_equal(w0, w1) and np.array_equal(b0, b1)
     assert sum(w.size + b.size for w, b in golden_weights) == 2868648
 
 
