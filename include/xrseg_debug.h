@@ -45,12 +45,7 @@ int xrseg_debug_conv(int device, int impl, const float* x, int b, int cin, int h
  * Channel triples: 16-8-16 and 32-16-32 (after padding). */
 int xrseg_debug_bottleneck(int device, const float* x, int b, int c1, int h, int w, const float* w1, const float* b1,
                            int cm, const float* w2, const float* b2, int c2, int residual, float* y);
-/* The whole-block C3k2 kernel (graph chains X.cv1, X.m0.cv1, X.m0.cv2, X.cv2 in one launch; built for the n-scale b2
- * block: 32 -> [16|16] -> 8 -> 16 -> 64 channels) on caller tensors, fp32 NCHW on the host. */
-int xrseg_debug_c3k2(int device, const float* x, int b, int cin, int h, int w, int c, int cm, int cout,
-                     const float* w_cv1, const float* b_cv1, const float* w_m1, const float* b_m1, const float* w_m2,
-                     const float* b_m2, const float* w_cv2, const float* b_cv2, float* y);
-/* Host-only: weight packing of the fused Bottleneck / C3k2 kernels into mma.sync B-fragment order (CPU layout tests). */
+/* Host-only: weight packing of the fused Bottleneck kernel into mma.sync B-fragment order (CPU layout tests). */
 int xrseg_debug_pack_bneck(const float* w, int cin, int cout, int C, int N, int taps, uint32_t* out, size_t cap_words);
 /* Host-side emulation of the UMMA conv kernel's data movement (slot mapping, weight packing, tap shifts)
  * in fp32 -- used by CPU tests to validate index math without a GPU.  NOT a product path. */

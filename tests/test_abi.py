@@ -240,18 +240,17 @@ def test_every_conv_plan_respects_the_hardware_limits(plan_dump, batch, scale):
     assert paired == (["b1"] if scale == "n" else []), paired
 
 
-@pytest.mark.parametrize("scale,whole_block,expect", [
-    ("n", "0", {"stem": 1, "conv": 79, "dw": 6, "sppf": 1, "up": 2, "attn": 1, "bneck": 3}),
-    ("n", "1", {"stem": 1, "conv": 77, "dw": 6, "sppf": 1, "up": 2, "attn": 1, "bneck": 2, "c3k2": 1}),
-    ("s", "0", {"stem": 1, "conv": 84, "dw": 6, "sppf": 1, "up": 2, "attn": 1, "bneck": 1}),
+@pytest.mark.parametrize("scale,expect", [
+    ("n", {"stem": 1, "conv": 79, "dw": 6, "sppf": 1, "up": 2, "attn": 1, "bneck": 3}),
+    ("s", {"stem": 1, "conv": 84, "dw": 6, "sppf": 1, "up": 2, "attn": 1, "bneck": 1}),
 ])
-def test_fusion_passes_produce_the_expected_launch_list(plan_dump, scale, whole_block, expect):
-    """model.cuh: fuse_siblings / fuse_bottlenecks / fuse_c3k2_blocks / fuse_attention_pe / fuse_tail_1x1.  n scale: 100 layers ->
-    93 network launches (six sibling pairs, the Bottlenecks of b2 / b4 / n16, the C2PSA positional encoding inside the attention
-    kernel, proto.cv3 inside proto.cv2's launch); the opt-in whole-block kernel takes b2; the s scale has one supported
-    Bottleneck (b2: 32-16-32).  Every fused Bottleneck keeps its residual and stays on the main stream."""
+def test_fusion_passes_produce_the_expected_launch_list(plan_dump, scale, expect):
+    """model.cuh: fuse_siblings / fuse_bottlenecks / fuse_attention_pe / fuse_tail_1x1.  n scale: 100 layers -> 93 network
+    launches (six sibling pairs, the Bottlenecks of b2 / b4 / n16, the C2PSA positional encoding inside the attention kernel,
+    proto.cv3 inside proto.cv2's launch); the s scale has one supported Bottleneck (b2: 32-16-32).  Every fused Bottleneck
+    keeps its residual and stays on the main stream."""
     import subprocess
-    out = subprocess.run([plan_dump, "64", scale, "ops", whole_block], capture_output=True, text=True, check=True).stdout
+    out = subprocess.run([plan_dump, "64", scale, "ops"], capture_output=True, text=True, check=True).stdout
     rows = [l.split() for l in out.splitlines() if l.startswith("op ")]
     kinds = {}
     for r in rows:

@@ -3,7 +3,6 @@
 libxrseg_debug.so) against the oracle's fp32 tensor of the same layer, on the committed golden frames.
 
   python tools/layer_sweep.py [--out gpurun_out/layer_sweep.md] [--frames coco139,coco632,bus]
-  XRSEG_LIB_VARIANT=silu16 python tools/layer_sweep.py ...        (the packed-fp16-SiLU A/B build of `make variants`)
 
 Per layer: relative L2 error ||gpu - ref|| / ||ref|| and max abs error over the sampled frames, plus the error of the
 layer's INPUT (so one can see whether a layer adds error or only passes it on).  Layers whose tensor does not exist in the
@@ -80,8 +79,7 @@ def main():
         h[0] += float((d.astype(np.float64) ** 2).sum()); h[1] += float((ref.astype(np.float64) ** 2).sum())
         h[2] = max(h[2], float(np.abs(d).max()))
     r.close()
-    variant = os.environ.get("XRSEG_LIB_VARIANT", "") or "product build"
-    lines = [f"# Per-layer error of the GPU network vs the fp32 oracle ({variant}; frames: {args.frames})", "",
+    lines = [f"# Per-layer error of the GPU network vs the fp32 oracle (product build; frames: {args.frames})", "",
              "relative L2 = ||gpu - oracle|| / ||oracle|| over the whole tensor, fp16 storage on the GPU side.", "",
              "| layer | rel L2 | max abs | note |", "|---|---|---|---|"]
     worst = 0.0

@@ -3,37 +3,15 @@
 //   /tmp/plan_dump [batch] [n|s]
 #include <math.h>
 #include "../xr_image_segmentation_b200/csrc/conv_tma.cuh"
-#include "../xr_image_segmentation_b200/csrc/conv_chain.cuh"
 #include "../xr_image_segmentation_b200/csrc/model.cuh"
 using namespace xrseg;
 int main(int argc, char** argv) {
   const int B = argc > 1 ? atoi(argv[1]) : 64;
   const int scale = argc > 2 ? argv[2][0] : 'n';
   if (argc > 3 && argv[3][0] == 'o') {   // "ops": the fused launch list (one line per network launch) instead of the conv plans
-    Net fused(scale, B, 640, true, true, argc > 4 && argv[4][0] == '1');
-    const char* kind_name[] = {"stem", "conv", "dw", "sppf", "up", "attn", "bneck", "c3k2", "chain"};
-    auto desc_of = [&](const Op& o) {
-      ConvDesc cd{};
-      cd.B = B; cd.H = o.x.H; cd.W = o.x.W; cd.Cin = o.x.Cp; cd.in_pitch = o.x.pitch; cd.Cout = o.y.Cp + (o.layer2 >= 0 ? o.y2.Cp : 0);
-      cd.out_pitch = o.y.pitch; cd.k = o.k; cd.stride = o.stride; cd.act = o.act; cd.transposed = o.transposed;
-      cd.res_pitch = o.has_res ? o.res.pitch : 0;
-      return cd;
-    };
-    if (argc > 5 && argv[5][0] == 'c')     // "chains": the launch list of the product (chain kernel for the 20x20 / 40x40 stages)
-      fused.fuse_chains([&](const Op& o) { ConvParams t; return plan_chain_layer(desc_of(o), t); });
+    Net fused(scale, B, 640, true, true);
+    const char* kind_name[] = {"stem", "conv", "dw", "sppf", "up", "attn", "bneck"};
     for (const Op& o : fused.ops) {
-      if (o.kind == OP_CHAIN) {
-        printf("op chain  %s .. %s  (%zu convolutions) branch %d wait %d signal %d\n", fused.layers[o.chain.front().layer].name.c_str(),
-               fused.layers[o.chain.back().layer].name.c_str(), o.chain.size(), o.branch, o.wait_tag, o.signal_tag);
-        for (const Op& s : o.chain) {
-          ConvParams p;
-          plan_chain_layer(desc_of(s), p);
-          printf("     %-18s %3dx%-3d %3d->%-3d k%d s%d mode %d cb %2d kps %d nks %2d R %2d nsub %d tpi %d ntiles %d S %d smem %6d tmem %3d bres %d\n",
-                 fused.layers[s.layer].name.c_str(), s.x.H, s.x.W, s.x.Cp, p.Cout, s.k, s.stride, p.mode, p.cb, p.kps, p.nks, p.R, p.nsub,
-                 p.tpi, p.n_tiles, p.S, p.smem_bytes, 2 * p.nsub * p.Ntile, p.b_resident);
-        }
-        continue;
-      }
       std::string name = o.layer >= 0 ? fused.layers[o.layer].name : std::string("-");
       if (o.kind == OP_CONV && o.layer2 >= 0) name += "+" + fused.layers[o.layer2].name;
       printf("op %-6s %-28s in %3dx%-3d c%-3d out c%-3d res %d branch %d\n", kind_name[o.kind], name.c_str(), o.x.H, o.x.W, o.x.Cp,

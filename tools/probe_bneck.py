@@ -15,10 +15,3 @@ for (B, c1, cm, c2, h, w) in [(64, 16, 8, 16, 160, 160), (64, 32, 16, 32, 80, 80
     w2 = rng.standard_normal((c2, cm, 3, 3), dtype=np.float32) * 0.1
     y = I.debug_bottleneck(x, w1, np.zeros(cm, np.float32), w2, np.zeros(c2, np.float32), residual=True)
     print(B, c1, cm, c2, h, w, "finite", bool(np.isfinite(y).all()), flush=True)
-
-B, cin, c, cm, cout, h, w = 64, 32, 16, 8, 64, 160, 160
-x = rng.standard_normal((B, cin, h, w), dtype=np.float32)
-mk = lambda co, ci, k: rng.standard_normal((co, ci, k, k) if k > 1 else (co, ci), dtype=np.float32) * 0.1
-y = I.debug_c3k2(x, mk(2 * c, cin, 1), np.zeros(2 * c, np.float32), mk(cm, c, 3), np.zeros(cm, np.float32), mk(c, cm, 3),
-                 np.zeros(c, np.float32), mk(cout, 3 * c, 1), np.zeros(cout, np.float32))
-print("c3k2", B, h, w, "finite", bool(np.isfinite(y).all()), flush=True)

@@ -114,7 +114,6 @@ DEBUG_SIGNATURES = {
                                    C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
     "xrseg_debug_bottleneck": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
                                          C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
-    "xrseg_debug_c3k2": (C.c_int, [C.c_int, C.c_void_p] + [C.c_int] * 7 + [C.c_void_p] * 9),
     "xrseg_debug_pack_bneck": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t]),
     "xrseg_debug_emulate_conv": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int,
                                            C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
@@ -125,9 +124,7 @@ SIGNATURES = {**PRODUCT_SIGNATURES, **DEBUG_SIGNATURES}   # what libxrseg_debug.
 
 
 def library_path(debug: bool = False) -> str:
-    variant = os.environ.get("XRSEG_LIB_VARIANT", "")          # A/B builds of `make variants` (e.g. silu16: the packed-fp16 SiLU); default: none
-    name = ("libxrseg_debug" if debug else "libxrseg") + (f"_{variant}" if variant else "")
-    return os.path.join(_HERE, name + ".so")
+    return os.path.join(_HERE, ("libxrseg_debug" if debug else "libxrseg") + ".so")
 
 
 def build_library(verbose: bool = False) -> str:

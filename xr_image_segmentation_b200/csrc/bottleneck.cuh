@@ -236,282 +236,6 @@ __global__ void __launch_bounds__(256) bottleneck_mma_kernel(const BneckParams p
 
 #endif  // __CUDACC__
 
-// ------------------------------------------------------------------------------------------------------------------
-// A whole C3k2 block (c3k = False) in one launch:  [a|b] = cv1(x) (1x1),  m = b + cv2'(cv1'(b)) (the Bottleneck above),
-// y = cv2([a|b|m]) (1x1)  -- graph chains X.cv1, X.m0.cv1, X.m0.cv2, X.cv2 (SURVEY.md Appendix A).  Built for the
-// high-resolution block b2 (32 -> [16|16] -> 8 -> 16 -> 64 channels at 160 x 160), where the four separate launches move
-// the 48-channel concat buffer through HBM three times; here only x is read and y written.  Same tiling as the
-// Bottleneck kernel (TH x 14 output pixels, 18-pixel-wide input window); cv1 is evaluated on the whole window (its
-// halo is recomputed by the neighbouring CTAs), positions outside the frame are forced to zero because they are the
-// 3x3 convolutions' padding.  The input window's shared memory is re-used for the Bottleneck's intermediates.
-// ------------------------------------------------------------------------------------------------------------------
-struct C3k2Params {
-  const __half* in; int in_pitch;      // [B,H,W,>=CIN]
-  __half* out; int out_pitch;          // [B,H,W,>=COUT]
-  const uint2 *w_cv1, *w_m1, *w_m2, *w_cv2;   // fragment-ordered fp16 weights
-  const float* bias;                   // [2C | CM | C | COUT]
-  int B, H, W;
-};
-
-template <int CIN, int C, int CM, int COUT, int TH>
-struct C3k2Cfg {
-  static constexpr int TW = BNECK_TW, IW = TW + 4, IH = TH + 4, MW = TW + 2, MH = TH + 2, NPIX = IH * IW;
-  static constexpr int PX = CIN * 2 + 16, PAB = 4 * C + 16, PMID = CM * 2 + (CM >= 16 ? 16 : 0), PMO = 2 * C + 16;
-  static constexpr int KS_CV1 = CIN / 16, NT_CV1 = 2 * C / 8;
-  static constexpr int KS_M1 = (9 * C + 15) / 16, NT_M1 = CM / 8, KS_M2 = (9 * CM + 15) / 16, NT_M2 = C / 8;
-  static constexpr int KS_CV2 = 3 * C / 16, NT_CV2 = COUT / 8;
-  static constexpr int X_BYTES = (NPIX * PX + 127) / 128 * 128, AB_BYTES = (NPIX * PAB + 127) / 128 * 128;
-  static constexpr int MID_BYTES = ((MH * MW + 2) * PMID + 127) / 128 * 128, MO_BYTES = (TH * 16 * PMO + 127) / 128 * 128;
-  static constexpr int W_CV1 = KS_CV1 * NT_CV1 * 256, W_M1 = KS_M1 * NT_M1 * 256, W_M2 = KS_M2 * NT_M2 * 256, W_CV2 = KS_CV2 * NT_CV2 * 256;
-  static constexpr int NBIAS = 2 * C + CM + C + COUT;
-  static constexpr int SMEM_BYTES = X_BYTES + AB_BYTES + W_CV1 + W_M1 + W_M2 + W_CV2 + NBIAS * 4;
-  static_assert(CIN % 16 == 0 && C % 16 == 0 && CM % 8 == 0 && COUT % 32 == 0 && TH % 2 == 0, "channel counts");
-  static_assert(MID_BYTES + MO_BYTES <= X_BYTES, "the Bottleneck's intermediates live in the input window's space");
-};
-
-#ifdef __CUDACC__
-
-template <int CIN, int C, int CM, int COUT, int TH>
-__global__ void __launch_bounds__(256) c3k2_mma_kernel(const C3k2Params p) {
-  using Cfg = C3k2Cfg<CIN, C, CM, COUT, TH>;
-  constexpr int TW = Cfg::TW, IW = Cfg::IW, IH = Cfg::IH, MW = Cfg::MW, MH = Cfg::MH, NPIX = Cfg::NPIX;
-  constexpr int PX = Cfg::PX, PAB = Cfg::PAB, PMID = Cfg::PMID, PMO = Cfg::PMO;
-  extern __shared__ __align__(128) uint8_t bneck_smem[];
-  uint8_t* s_x = bneck_smem;
-  uint8_t* s_mid = s_x;                        // aliases s_x (dead after cv1)
-  uint8_t* s_m = s_x + Cfg::MID_BYTES;
-  uint8_t* s_ab = s_x + Cfg::X_BYTES;
-  uint2* s_wcv1 = reinterpret_cast<uint2*>(s_ab + Cfg::AB_BYTES);
-  uint2* s_wm1 = reinterpret_cast<uint2*>(reinterpret_cast<uint8_t*>(s_wcv1) + Cfg::W_CV1);
-  uint2* s_wm2 = reinterpret_cast<uint2*>(reinterpret_cast<uint8_t*>(s_wm1) + Cfg::W_M1);
-  uint2* s_wcv2 = reinterpret_cast<uint2*>(reinterpret_cast<uint8_t*>(s_wm2) + Cfg::W_M2);
-  float* s_bias = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(s_wcv2) + Cfg::W_CV2);
-  const float *s_bcv1 = s_bias, *s_bm1 = s_bias + 2 * C, *s_bm2 = s_bm1 + CM, *s_bcv2 = s_bm2 + C;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3, hi = lane >> 4;
-  const int tx0 = blockIdx.x * TW, ty0 = blockIdx.y * TH, b = blockIdx.z;
-
-  pdl_launch_dependents();
-  {
-    auto fetch = [&](uint2* dst, const uint2* src, int bytes) {
-      for (int i = tid; i < bytes / 16; i += 256) cp_async16(smem_u32(dst) + 16 * i, reinterpret_cast<const uint8_t*>(src) + 16 * i, 16);
-    };
-    fetch(s_wcv1, p.w_cv1, Cfg::W_CV1);
-    fetch(s_wm1, p.w_m1, Cfg::W_M1);
-    fetch(s_wm2, p.w_m2, Cfg::W_M2);
-    fetch(s_wcv2, p.w_cv2, Cfg::W_CV2);
-    cp_async_commit();
-    for (int i = tid; i < Cfg::NBIAS; i += 256) s_bias[i] = p.bias[i];
-  }
-  pdl_wait();
-
-  // 1. input window (zero outside the frame)
-  {
-    constexpr int CH = CIN / 8, ROW = IW * CH, TOTAL = IH * ROW, ITERS = (TOTAL + 255) / 256;
-    const __half* img = p.in + static_cast<size_t>(b) * p.H * p.W * p.in_pitch;
-    uint4 v[ITERS];
-#pragma unroll
-    for (int k = 0; k < ITERS; ++k) {
-      const int i = tid + 256 * k;
-      const int r = i / ROW, j = i - r * ROW;
-      const int col = j / CH, c = j - col * CH;
-      const int y = ty0 - 2 + r, x = tx0 - 2 + col;
-      v[k] = make_uint4(0u, 0u, 0u, 0u);
-      if (i < TOTAL && y >= 0 && y < p.H && x >= 0 && x < p.W)
-        v[k] = __ldcg(reinterpret_cast<const uint4*>(img + (static_cast<size_t>(y) * p.W + x) * p.in_pitch + c * 8));
-    }
-#pragma unroll
-    for (int k = 0; k < ITERS; ++k) {
-      const int i = tid + 256 * k;
-      const int r = i / ROW, j = i - r * ROW;
-      const int col = j / CH, c = j - col * CH;
-      if (i < TOTAL) *reinterpret_cast<uint4*>(s_x + (r * IW + col) * PX + c * 16) = v[k];
-    }
-    cp_async_wait<0>();
-  }
-  __syncthreads();
-
-  // 2. cv1 (1x1, CIN -> 2C) on every pixel of the window -> s_ab; M-tiles are 16 consecutive pixels of the flattened window
-  {
-    constexpr int NT = Cfg::NT_CV1, KS = Cfg::KS_CV1, MT = (NPIX + 15) / 16, UNITS = (MT + 1) / 2;
-    for (int u = warp; u < UNITS; u += 8) {
-      float acc[2][NT][4];
-      uint32_t a_base[2];
-#pragma unroll
-      for (int m = 0; m < 2; ++m) {
-#pragma unroll
-        for (int nt = 0; nt < NT; ++nt) acc[m][nt][0] = acc[m][nt][1] = acc[m][nt][2] = acc[m][nt][3] = 0.f;
-        a_base[m] = smem_u32(s_x) + min((2 * u + m) * 16 + (lane & 15), NPIX - 1) * PX + hi * 16;
-      }
-#pragma unroll
-      for (int s = 0; s < KS; ++s) {
-        uint32_t a[2][4];
-        bneck_ldmatrix_x4(a[0], a_base[0] + s * 32);
-        bneck_ldmatrix_x4(a[1], a_base[1] + s * 32);
-#pragma unroll
-        for (int nt = 0; nt < NT; ++nt) {
-          const uint2 bw = s_wcv1[(s * NT + nt) * 32 + lane];
-          bneck_hmma(acc[0][nt], a[0], bw.x, bw.y);
-          bneck_hmma(acc[1][nt], a[1], bw.x, bw.y);
-        }
-      }
-#pragma unroll
-      for (int m = 0; m < 2; ++m)
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int q = (2 * u + m) * 16 + g + 8 * h;
-          if (q < NPIX) {
-            const int r = q / IW, col = q - r * IW;
-            const int y = ty0 - 2 + r, x = tx0 - 2 + col;
-            const bool ok = y >= 0 && y < p.H && x >= 0 && x < p.W;
-            uint8_t* dst = s_ab + q * PAB + 4 * t;
-#pragma unroll
-            for (int nt = 0; nt < NT; ++nt) {
-              const uint32_t v = silu_pack_h2(acc[m][nt][2 * h] + s_bcv1[nt * 8 + 2 * t], acc[m][nt][2 * h + 1] + s_bcv1[nt * 8 + 2 * t + 1]);
-              *reinterpret_cast<uint32_t*>(dst + nt * 16) = ok ? v : 0u;
-            }
-          }
-        }
-    }
-  }
-  __syncthreads();
-
-  // 3. Bottleneck conv 1 (3x3, C -> CM) on b = channels [C, 2C) of s_ab -> s_mid (zero outside the frame)
-  {
-    constexpr int NT = Cfg::NT_M1;
-    float bias[NT][2];
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) { bias[nt][0] = s_bm1[nt * 8 + 2 * t]; bias[nt][1] = s_bm1[nt * 8 + 2 * t + 1]; }
-    for (int u = warp; u < MH / 2; u += 8) {
-      float acc[2][NT][4];
-      uint32_t a_base[2];
-#pragma unroll
-      for (int m = 0; m < 2; ++m) {
-#pragma unroll
-        for (int nt = 0; nt < NT; ++nt) acc[m][nt][0] = acc[m][nt][1] = acc[m][nt][2] = acc[m][nt][3] = 0.f;
-        a_base[m] = smem_u32(s_ab) + ((2 * u + m) * IW + (lane & 15)) * PAB + 2 * C;
-      }
-      bneck_conv_tiles<C, NT, IW, PAB>(acc, a_base, s_wm1, lane);
-#pragma unroll
-      for (int m = 0; m < 2; ++m) {
-        const int qy = 2 * u + m, y = ty0 - 1 + qy;
-        const bool row_ok = y >= 0 && y < p.H;
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int qx = g + 8 * h, x = tx0 - 1 + qx;
-          const bool ok = row_ok && x >= 0 && x < p.W;
-          uint8_t* dst = s_mid + (qy * MW + qx) * PMID + 4 * t;
-#pragma unroll
-          for (int nt = 0; nt < NT; ++nt) {
-            const uint32_t v = silu_pack_h2(acc[m][nt][2 * h] + bias[nt][0], acc[m][nt][2 * h + 1] + bias[nt][1]);
-            *reinterpret_cast<uint32_t*>(dst + nt * 16) = ok ? v : 0u;
-          }
-        }
-      }
-    }
-  }
-  __syncthreads();
-
-  // 4. Bottleneck conv 2 (3x3, CM -> C) + b -> s_m (rows of 16 pixels; pixels 14, 15 are never used)
-  {
-    constexpr int NT = Cfg::NT_M2;
-    float bias[NT][2];
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) { bias[nt][0] = s_bm2[nt * 8 + 2 * t]; bias[nt][1] = s_bm2[nt * 8 + 2 * t + 1]; }
-    for (int u = warp; u < TH / 2; u += 8) {
-      float acc[2][NT][4];
-      uint32_t a_base[2];
-#pragma unroll
-      for (int m = 0; m < 2; ++m) {
-#pragma unroll
-        for (int nt = 0; nt < NT; ++nt) acc[m][nt][0] = acc[m][nt][1] = acc[m][nt][2] = acc[m][nt][3] = 0.f;
-        a_base[m] = smem_u32(s_mid) + ((2 * u + m) * MW + (lane & 15)) * PMID;
-      }
-      bneck_conv_tiles<CM, NT, MW, PMID>(acc, a_base, s_wm2, lane);
-#pragma unroll
-      for (int m = 0; m < 2; ++m) {
-        const int oy = 2 * u + m;
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int ox = g + 8 * h;
-          const uint8_t* res = s_ab + ((oy + 2) * IW + min(ox, TW - 1) + 2) * PAB + 2 * C + 4 * t;
-          uint8_t* dst = s_m + (oy * 16 + ox) * PMO + 4 * t;
-#pragma unroll
-          for (int nt = 0; nt < NT; ++nt) {
-            const uint32_t v = silu_pack_h2(acc[m][nt][2 * h] + bias[nt][0], acc[m][nt][2 * h + 1] + bias[nt][1]);
-            const uint32_t rr = *reinterpret_cast<const uint32_t*>(res + nt * 16);
-            const __half2 s2 = __hadd2(*reinterpret_cast<const __half2*>(&v), *reinterpret_cast<const __half2*>(&rr));
-            *reinterpret_cast<uint32_t*>(dst + nt * 16) = *reinterpret_cast<const uint32_t*>(&s2);
-          }
-        }
-      }
-    }
-  }
-  __syncthreads();
-
-  // 5. cv2 (1x1, [a|b|m] = 3C -> COUT) on the tile -> global; four n-tiles at a time keep the accumulators at 32 registers
-  {
-    constexpr int NT = Cfg::NT_CV2, KS_AB = 2 * C / 16, KS_M = C / 16;
-    __half* img = p.out + static_cast<size_t>(b) * p.H * p.W * p.out_pitch;
-    for (int u = warp; u < TH / 2; u += 8) {
-      uint32_t ab_base[2], m_base[2];
-#pragma unroll
-      for (int m = 0; m < 2; ++m) {
-        const int oy = 2 * u + m, ox = min(lane & 15, TW - 1);
-        ab_base[m] = smem_u32(s_ab) + ((oy + 2) * IW + ox + 2) * PAB + hi * 16;
-        m_base[m] = smem_u32(s_m) + (oy * 16 + ox) * PMO + hi * 16;
-      }
-#pragma unroll
-      for (int nh = 0; nh < NT / 4; ++nh) {
-        float acc[2][4][4];
-#pragma unroll
-        for (int m = 0; m < 2; ++m)
-#pragma unroll
-          for (int nt = 0; nt < 4; ++nt) acc[m][nt][0] = acc[m][nt][1] = acc[m][nt][2] = acc[m][nt][3] = 0.f;
-#pragma unroll
-        for (int s = 0; s < KS_AB + KS_M; ++s) {
-          uint32_t a[2][4];
-          bneck_ldmatrix_x4(a[0], s < KS_AB ? ab_base[0] + s * 32 : m_base[0] + (s - KS_AB) * 32);
-          bneck_ldmatrix_x4(a[1], s < KS_AB ? ab_base[1] + s * 32 : m_base[1] + (s - KS_AB) * 32);
-#pragma unroll
-          for (int nt = 0; nt < 4; ++nt) {
-            const uint2 bw = s_wcv2[(s * NT + nh * 4 + nt) * 32 + lane];
-            bneck_hmma(acc[0][nt], a[0], bw.x, bw.y);
-            bneck_hmma(acc[1][nt], a[1], bw.x, bw.y);
-          }
-        }
-#pragma unroll
-        for (int m = 0; m < 2; ++m) {
-          const int oy = 2 * u + m, y = ty0 + oy;
-          __half* row = img + (static_cast<size_t>(y) * p.W + tx0) * p.out_pitch + nh * 32;
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-            const int ox = g + 8 * h, x = tx0 + ox;
-            const bool ok = y < p.H && ox < TW && x < p.W;
-            uint32_t v[4];
-#pragma unroll
-            for (int nt = 0; nt < 4; ++nt) {
-              const int c = (nh * 4 + nt) * 8 + 2 * t;
-              v[nt] = silu_pack_h2(acc[m][nt][2 * h] + s_bcv2[c], acc[m][nt][2 * h + 1] + s_bcv2[c + 1]);
-            }
-            __half* dst = row + ox * p.out_pitch;
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-              const uint32_t send = (t & 1) ? v[2 * j] : v[2 * j + 1];
-              const uint32_t recv = __shfl_xor_sync(0xffffffffu, send, 1);
-              if (ok) {
-                if (t & 1) *reinterpret_cast<uint2*>(dst + (2 * j + 1) * 8 + 2 * (t - 1)) = make_uint2(recv, v[2 * j + 1]);
-                else *reinterpret_cast<uint2*>(dst + (2 * j) * 8 + 2 * t) = make_uint2(v[2 * j], recv);
-              }
-            }
-          }
-        }
-      }
-    }
-  }
-}
-
-#endif  // __CUDACC__
-
 // B-fragment order of mma.sync m16n8k16 for W[k][n], k = tap * C + c (tap-major over the C channels of the shared-memory
 // window, zero beyond the real channel counts and beyond K = 9 C): per (k-step, n-tile, lane) two 32-bit words
 //   b0 = { W[16 s + 2 t][n], W[16 s + 2 t + 1][n] },  b1 = { W[16 s + 2 t + 8][n], W[16 s + 2 t + 9][n] },  n = 8 nt + lane / 4,

@@ -60,22 +60,14 @@ __device__ __forceinline__ float silu_f(float y) { return __fdividef(y, 1.0f + _
 // output, SURVEY.md fact 6).  Measured on B200 against the packed-fp16 form (tanh.approx.f16x2 + HFMA2, half the MUFU
 // work but three roundings): no launch changes by more than noise (profiles/r2a_*), while the per-layer relative L2 error
 // against the fp32 oracle drops by a third to a half and the worst class-logit error from 0.21 to 0.08
-// (profiles/r2a_layer_sweep_*.md).  -DXRSEG_SILU_F16X2 (make variants) rebuilds the packed form for A/B runs.
+// (profiles/r2a_layer_sweep_*.md).
 __device__ __forceinline__ uint32_t silu_pack_h2(float a, float b) {
-#ifdef XRSEG_SILU_F16X2
-  __half2 h = __floats2half2_rn(0.5f * a, 0.5f * b);
-  uint32_t hu = *reinterpret_cast<uint32_t*>(&h), tu;
-  asm("tanh.approx.f16x2 %0, %1;" : "=r"(tu) : "r"(hu));
-  __half2 r = __hfma2(h, *reinterpret_cast<__half2*>(&tu), h);
-  return *reinterpret_cast<uint32_t*>(&r);
-#else
   const float ha = 0.5f * a, hb = 0.5f * b;
   float ta, tb;
   asm("tanh.approx.f32 %0, %1;" : "=f"(ta) : "f"(ha));
   asm("tanh.approx.f32 %0, %1;" : "=f"(tb) : "f"(hb));
   __half2 r = __floats2half2_rn(fmaf(ha, ta, ha), fmaf(hb, tb, hb));
   return *reinterpret_cast<uint32_t*>(&r);
-#endif
 }
 
 // 256-bit global accesses (sm_100): one full 32-byte sector per lane and instruction.
@@ -141,19 +133,11 @@ __device__ __forceinline__ void epilogue_chunk16(const uint32_t (&v)[16], const 
 // half-argument of silu(y) = h tanh(h) + h is ONE FFMA on the accumulator (h = 0.5 acc + 0.5 bias): three FP32-pipe
 // instructions and one MUFU per output, plus half a pack.
 __device__ __forceinline__ uint32_t silu_pack_from_half_arg(float ha, float hb) {
-#ifdef XRSEG_SILU_F16X2
-  __half2 h = __floats2half2_rn(ha, hb);
-  uint32_t hu = *reinterpret_cast<uint32_t*>(&h), tu;
-  asm("tanh.approx.f16x2 %0, %1;" : "=r"(tu) : "r"(hu));
-  __half2 r = __hfma2(h, *reinterpret_cast<__half2*>(&tu), h);
-  return *reinterpret_cast<uint32_t*>(&r);
-#else
   float ta, tb;
   asm("tanh.approx.f32 %0, %1;" : "=f"(ta) : "f"(ha));
   asm("tanh.approx.f32 %0, %1;" : "=f"(tb) : "f"(hb));
   __half2 r = __floats2half2_rn(fmaf(ha, ta, ha), fmaf(hb, tb, hb));
   return *reinterpret_cast<uint32_t*>(&r);
-#endif
 }
 // probe (PROBE instantiation of the kernel only; 0 in the product): 1 = compute but do not store, 2 = store without the
 // bias / SiLU math (raw accumulators rounded to fp16)

@@ -28,9 +28,8 @@ namespace xrseg {
 enum { MODE_HALO_TMA = 2, MODE_FLAT_TMA = 3, MODE_S2_TMA = 4 };
 
 // Up to four tensor maps per launch (MODE_S2_TMA reads four parity planes of the input; the other modes use m[0]).
-// m[4] / m[5]: output tensor maps of the TMA-store epilogue (out / out2), unused otherwise.
 struct TmapSet {
-  CUtensorMap m[6];
+  CUtensorMap m[4];
 };
 // warp 0: TMA producer; warps 1-4: MMA issuers (one per 128-row sub-tile: a single thread cannot issue tcgen05.mma faster
 // than one per ~50-65 cycles, which bounded every thin layer); warps 5 .. 5 + TMA_EPI_WARPS - 1: epilogue.  The epilogue
@@ -39,15 +38,8 @@ struct TmapSet {
 // dependency stalls, not by issue slots or the MUFU (tools/probe_mufu.cu: 15.4 SiLU / clk / SM with eight warps), so more
 // warps per scheduler hide more of them -- 8 / 12 / 16 / 20 / 24 warps: 31.7k / 32.6k / 33.4k / 32.2k / 29.5k frames/s
 // (past 16 the register cap of a 1-CTA-per-SM launch, 65536 / threads, forces spills).
-#ifndef XRSEG_EPI_WARPS
-#define XRSEG_EPI_WARPS 16
-#endif
-#ifndef XRSEG_BIAS_PREFETCH
-#define XRSEG_BIAS_PREFETCH 0   // 1: fetch the bias of non-fixed chunks one unit ahead (needs 16 more registers: spills at the 80-register cap of a 21-warp CTA, measured slower)
-#endif
-enum { TMA_EPI_WARPS = XRSEG_EPI_WARPS, TMA_EPI_GROUPS = XRSEG_EPI_WARPS / 4, TMA_THREADS = 32 * (5 + XRSEG_EPI_WARPS),
-       TMA_TAIL_PAD = 4096, TMA_FIRST_EPI_WARP = 5 };
-static_assert(XRSEG_EPI_WARPS % 4 == 0 && XRSEG_EPI_WARPS >= 8 && XRSEG_EPI_WARPS <= 24, "whole groups of four epilogue warps");
+enum { TMA_EPI_WARPS = 16, TMA_EPI_GROUPS = TMA_EPI_WARPS / 4, TMA_THREADS = 32 * (5 + TMA_EPI_WARPS), TMA_TAIL_PAD = 4096,
+       TMA_FIRST_EPI_WARP = 5 };
 
 struct TmaPlanExtra {
   int R, nsub, tpi, hbox, slots_box;
@@ -91,18 +83,6 @@ static inline CUtensorMap make_halo_tensor_map(const __half* base, int B, int H,
 }
 
 // ---- planning --------------------------------------------------------------------------------------------------
-// Shared-memory budget of the TMA planners.  tma_smem_budget() is CONV_SMEM_MAX unless XRSEG_SMEM_KB asks for a smaller
-// PREFERRED footprint (e.g. 113 = half an SM, so that consecutive kernels can be co-resident under programmatic
-// dependent launch); plan_conv_*_tma first try the preferred budget and fall back to the full one.
-static inline int& tma_budget_ref() {
-  static thread_local int b = CONV_SMEM_MAX;
-  return b;
-}
-static inline int tma_preferred_budget() {
-  static const int kb = [] { const char* e = getenv("XRSEG_SMEM_KB"); return e ? atoi(e) : 0; }();
-  return kb > 0 && kb * 1024 < CONV_SMEM_MAX ? kb * 1024 : CONV_SMEM_MAX;
-}
-#define XR_TMA_BUDGET (tma_budget_ref())
 // Few work items (batch-1 streaming: a 20x20 layer is one or two items): a layer with >= 128 output channels whose items would
 // keep at most half the SMs busy is planned as TWO N tiles -- twice the CTAs, half the MMAs (and half the streamed weights) on
 // each one's critical path.  Set by the plan_conv_*_tma wrappers for a second planning pass; XRSEG_SPLIT_SMALL=0 turns it off.
@@ -119,29 +99,17 @@ static inline void tma_apply_split(ConvParams& p, int ncols) {
 }
 // 0: no split; 2 / 4: N tiles for the second planning pass (four only for 256 output channels on at most a quarter of the SMs)
 static inline int tma_wants_split(const ConvParams& p, int num_sms) {
-  static const int mode = [] { const char* e = getenv("XRSEG_SPLIT_SMALL"); return e ? atoi(e) : 4; }();   // 0 off, 2: halves only
-  if (!mode || p.n_tiles != 1 || p.Ntile < 128 || p.transposed || 2 * p.m_tiles > num_sms) return 0;
-  if (mode >= 4 && p.Ntile == 256 && 4 * p.m_tiles <= num_sms) return 4;
+  static const bool on = [] { const char* e = getenv("XRSEG_SPLIT_SMALL"); return !(e && e[0] == '0'); }();
+  if (!on || p.n_tiles != 1 || p.Ntile < 128 || p.transposed || 2 * p.m_tiles > num_sms) return 0;
+  if (p.Ntile == 256 && 4 * p.m_tiles <= num_sms) return 4;
   return (p.Ntile / 2) % 16 == 0 ? 2 : 0;
 }
 
 // A CTA never has more than ceil(work / grid) * nks stages to fetch: a deeper ring only costs shared memory, and a small
 // footprint is what lets the next kernel's CTAs become co-resident early (programmatic dependent launch) so that their
 // prologue -- barrier init, TMEM allocation, weight fetch -- overlaps this kernel's tail.
-// Accumulator sets in TMEM: the MMA -> commit -> epilogue -> release round trip of one item is several microseconds, so
-// thin layers (few columns per item) ring up to four sets instead of two; CTAs with little work keep two, which leaves
-// TMEM columns for a co-resident CTA of the next kernel.
-static inline int choose_nbuf(int nsub, int ntile, int work, int num_sms) {
-  const int grid = work < num_sms ? work : num_sms;
-  int nbuf = 512 / (nsub * ntile);
-  if (nbuf > 4) nbuf = 4;
-  if (nbuf < 2) nbuf = 2;
-  if (ceil_div(work, grid) < 4) nbuf = 2;
-  // Measured on B200 (YOLO11n-seg, batch 64): ringing 4 sets instead of 2 changes no layer by more than noise -- the
-  // round trip is not what bounds the thin layers -- so two sets stay the default (XRSEG_NBUF=4 re-enables the ring).
-  static const bool deep = [] { const char* e = getenv("XRSEG_NBUF"); return e && e[0] == '4'; }();
-  return deep ? nbuf : 2;
-}
+// Accumulator sets in TMEM: every plan takes two.  Measured on B200 (YOLO11n-seg, batch 64): ringing four sets for thin
+// layers changes no layer by more than noise -- the MMA -> epilogue round trip is not what bounds them.
 static inline int clamp_stages(int S, int work, int num_sms, int nks) {
   const int grid = work < num_sms ? work : num_sms;
   int need = ceil_div(work, grid) * nks;
@@ -176,12 +144,6 @@ static inline bool plan_conv_halo_tma_impl(const ConvDesc& d, int num_sms, ConvP
   p.Hp1 = d.H + 1;
   int nsub_max = 256 / p.Ntile;
   if (nsub_max > 4) nsub_max = 4;
-  {
-    // experiment switch: smaller items (more items per CTA -> the fill / drain of the MMA <-> epilogue pipeline weighs less)
-    static const int cap = [] { const char* e = getenv("XRSEG_HALO_NSUB_MAX"); return e ? atoi(e) : 0; }();
-    static const int cap_w = [] { const char* e = getenv("XRSEG_HALO_NSUB_MAX_W"); return e ? atoi(e) : 100000; }();
-    if (cap > 0 && nsub_max > cap && d.W <= cap_w) nsub_max = cap;
-  }
   if (nsub_max < 1 || p.Wp > 256) return false;
   int R = (128 * nsub_max) / p.Wp;
   if (R > d.H) R = d.H;
@@ -220,19 +182,17 @@ static inline bool plan_conv_halo_tma_impl(const ConvDesc& d, int num_sms, ConvP
       const bool res = (p.n_tiles == 1 && total_b <= 114688);
       const int fixed = round_up(CONV_HDR_BYTES, 1024) + 1024 + 128 * rb + 1024 +
                         (res ? round_up(static_cast<int>(total_b), 1024) : 0);
-      int S = (XR_TMA_BUDGET - fixed) / (a_stage + (res ? 0 : round_up(b_stage, 1024)));
+      int S = (CONV_SMEM_MAX - fixed) / (a_stage + (res ? 0 : round_up(b_stage, 1024)));
       if (S > CONV_MAX_STAGES) S = CONV_MAX_STAGES;
       if (S > 2 * (d.Cin / cb) + 2) S = 2 * (d.Cin / cb) + 2;
       // The TMA unit delivers one box ROW per ~1.5 cycles whatever its width (tools/probe_tma_rate.cu: 21 / 42 / 85 B/clk per SM
       // for 32 / 64 / 128-byte rows), so a layer that splits its channels into narrow K-blocks pays the row cost Cin / cb
-      // times.  XRSEG_HALO_MIN_S=2 takes the WIDEST K-block that still leaves a two-stage ring; measured on the network
-      // (proto.cv2 148 -> 154 us, h4.box.0 33 -> 35 us, n13/n19.m0.cv1 equal) the deeper three-stage ring with narrower
-      // blocks is still the better trade, so 3 stays the default.
-      static const int min_S = [] { const char* e = getenv("XRSEG_HALO_MIN_S"); return e ? atoi(e) : 3; }();
-      if (S >= min_S || (S == 2 && best_S < 2)) {
+      // times.  Taking the WIDEST K-block that still leaves a two-stage ring was measured on the network (proto.cv2 148 -> 154
+      // us, h4.box.0 33 -> 35 us, n13/n19.m0.cv1 equal): the deeper three-stage ring with narrower blocks is the better trade.
+      if (S >= 3 || (S == 2 && best_S < 2)) {
         best_cb = cb;
         best_S = S;
-        if (S >= min_S) break;
+        if (S >= 3) break;
       }
     }
     if (best_S < 2) return false;
@@ -241,7 +201,7 @@ static inline bool plan_conv_halo_tma_impl(const ConvDesc& d, int num_sms, ConvP
     const int rb = cb * 2;
     p.cb = cb; p.cps = cb / 8; p.nks = d.Cin / cb;
     p.taps = 9; p.K_total = 9 * d.Cin;
-    p.nbuf = choose_nbuf(p.nsub, p.Ntile, d.B * p.tpi * p.n_tiles, num_sms);
+    p.nbuf = 2;
     p.tmem_cols = pow2_ceil(p.nbuf * p.nsub * p.Ntile);
     p.a_stage_bytes = round_up(p.slots * rb, 1024);
     p.b_stage_bytes = 9 * p.Ntile * rb;
@@ -257,7 +217,7 @@ static inline bool plan_conv_halo_tma_impl(const ConvDesc& d, int num_sms, ConvP
     // one tail pad BEFORE the A stages too: tap (0,0) of position 0 reads the row before the stage
     p.smem_off_a = p.smem_off_b + round_up(b_region, 1024) + 1024;
     p.smem_bytes = p.smem_off_a + S * p.a_stage_bytes + 128 * rb + 1024;
-    if (p.smem_bytes > XR_TMA_BUDGET) return false;
+    if (p.smem_bytes > CONV_SMEM_MAX) return false;
     const int work = p.m_tiles * p.n_tiles;
     p.grid = work < num_sms ? work : num_sms;
     p.fd_wp = make_fastdiv(p.Wp);
@@ -272,7 +232,7 @@ static inline bool plan_conv_halo_tma_impl(const ConvDesc& d, int num_sms, ConvP
   p.K_total = 9 * d.Cin;
   p.nbuf = 2;
   p.tmem_cols = pow2_ceil(2 * p.nsub * p.Ntile);
-  const int budget = XR_TMA_BUDGET - CONV_HDR_BYTES - TMA_TAIL_PAD;
+  const int budget = CONV_SMEM_MAX - CONV_HDR_BYTES - TMA_TAIL_PAD;
   const long total_b = 9L * d.Cin * p.Ntile * 2;
   p.b_resident = (p.n_tiles == 1 && total_b <= 114688) ? 1 : 0;
   int best_cb = 0, best_S = 0;
@@ -304,7 +264,7 @@ static inline bool plan_conv_halo_tma_impl(const ConvDesc& d, int num_sms, ConvP
   const int b_region = p.b_resident ? p.nks * p.b_stage_bytes : p.S * p.b_stage_bytes;
   p.smem_off_a = CONV_HDR_BYTES + round_up(b_region, 128);
   p.smem_bytes = p.smem_off_a + p.S * p.a_stage_bytes + TMA_TAIL_PAD;
-  if (p.smem_bytes > XR_TMA_BUDGET) return false;
+  if (p.smem_bytes > CONV_SMEM_MAX) return false;
   const int work = p.m_tiles * p.n_tiles;
   p.grid = work < num_sms ? work : num_sms;
   p.fd_wp = make_fastdiv(p.Wp);
@@ -377,27 +337,19 @@ static inline bool plan_conv_s2_tma_impl(const ConvDesc& d, int num_sms, ConvPar
       const int plane = round_up((R + 1) * p.Wp * rb, 1024);
       const int b_stage = 9 * p.Ntile * rb;
       const int fixed = round_up(CONV_HDR_BYTES, 1024) + 1024 + 128 * rb + 1024 + p.Wp * rb + round_up(resident, 1024);
-      int S = (XR_TMA_BUDGET - fixed) / (4 * plane + (p.b_resident ? 0 : round_up(b_stage, 1024)));
+      int S = (CONV_SMEM_MAX - fixed) / (4 * plane + (p.b_resident ? 0 : round_up(b_stage, 1024)));
       if (S > CONV_MAX_STAGES) S = CONV_MAX_STAGES;
       if (S > 2 * (d.Cin / cb) + 2) S = 2 * (d.Cin / cb) + 2;
       if (S < 2) continue;
       const int nks = d.Cin / cb, nsub = ceil_div(R * p.Wp, 128);
-      // operand fetch.  XRSEG_S2_ROWCOST=1 models it as ~1.5 cycles per TMA box row whatever its width
-      // (tools/probe_tma_rate.cu), four plane boxes per K-block, and the MMA issue as parallel over the sub-tile warps;
-      // measured on the network (gpurun_out s17, s19): n17 (80 -> 40) alone 40.7 -> 27.4 us, b5 51 -> 50 us, b3 (160 -> 80) 64 -> 69 us;
-      // restricted to output maps up to 40 x 40 (XRSEG_S2_ROWCOST=2) one runner alone gains 1 %, but four runners LOSE 2 % (38.1k ->
-      // 37.3k frames/s, three A/B pairs): n17's new plan has 512 items and leaves the half-width rule of the small launches
-      // (xrseg_api.cu), and side by side beats faster.  The bytes / 40 B/clk estimate stays the default.
-      static const int rowcost_env = [] { const char* e = getenv("XRSEG_S2_ROWCOST"); return e ? atoi(e) : 0; }();
-      const bool rowcost = rowcost_env == 1 || (rowcost_env == 2 && Ho <= 40);
-      // one issuing warp per sub-tile: the issue cost (~50 cycles per MMA, ~600 per stage hand-over) is paid in parallel,
-      // the tensor pipe (128 x N x 16 MACs per MMA at 4096 MACs / cycle) is shared
-      const double t_issue = nks * 600.0 + 9.0 * (d.Cin / 16) * 50.0;
-      const double t_pipe = 9.0 * (d.Cin / 16) * nsub * (p.Ntile / 2.0 > 16.0 ? p.Ntile / 2.0 : 16.0);
-      const double t_mma = rowcost ? (t_issue > t_pipe ? t_issue : t_pipe)
-                                   : nks * 600.0 + 9.0 * (d.Cin / 16) * nsub * (p.Ntile / 2.0 > 50.0 ? p.Ntile / 2.0 : 50.0);
+      // operand fetch at ~40 bytes per clock.  A row-cost model (~1.5 cycles per TMA box row whatever its width, MMA issue
+      // parallel over the sub-tile warps) was measured on the network: n17 (80 -> 40) alone 40.7 -> 27.4 us, b5 51 -> 50 us,
+      // b3 (160 -> 80) 64 -> 69 us; restricted to output maps up to 40 x 40 one runner alone gains 1 %, but four runners LOSE
+      // 2 % (38.1k -> 37.3k frames/s, three A/B pairs): n17's plan then has 512 items and leaves the half-width rule of the small
+      // launches (xrseg_api.cu), and side by side beats faster.
+      const double t_mma = nks * 600.0 + 9.0 * (d.Cin / 16) * nsub * (p.Ntile / 2.0 > 50.0 ? p.Ntile / 2.0 : 50.0);
       const double t_epi = nsub * ceil_div(p.Ntile, 32) * 650.0;
-      const double t_mem = rowcost ? 1.5 * 4.0 * (R + 1) * p.Wp * nks : 4.0 * (R + 1) * p.Wp * d.Cin * 2 / 40.0;
+      const double t_mem = 4.0 * (R + 1) * p.Wp * d.Cin * 2 / 40.0;
       double t = t_mma > t_epi ? t_mma : t_epi;
       if (t_mem > t) t = t_mem;
       t = (t + 800.0) * (S >= 3 ? 1.0 : 1.15);
@@ -419,7 +371,7 @@ static inline bool plan_conv_s2_tma_impl(const ConvDesc& d, int num_sms, ConvPar
   p.lbo_a = round_up(p.slots * rb, 1024);          // bytes of one plane buffer
   p.a_stage_bytes = 4 * p.lbo_a;
   p.b_stage_bytes = 9 * p.Ntile * rb;
-  p.nbuf = choose_nbuf(p.nsub, p.Ntile, d.B * p.tpi * p.n_tiles, num_sms);
+  p.nbuf = 2;
   p.tmem_cols = pow2_ceil(p.nbuf * p.nsub * p.Ntile);
   p.M_total = d.B * p.tpi;
   p.m_tiles = p.M_total;
@@ -427,7 +379,7 @@ static inline bool plan_conv_s2_tma_impl(const ConvDesc& d, int num_sms, ConvPar
   const int b_region = p.b_resident ? resident : p.S * round_up(p.b_stage_bytes, 1024);
   p.smem_off_a = p.smem_off_b + round_up(b_region, 1024) + 1024;        // one pad row block before the stages (offset -1)
   p.smem_bytes = p.smem_off_a + p.S * p.a_stage_bytes + 128 * rb + p.Wp * rb + 1024;   // tail: rows read past the last plane
-  if (p.smem_bytes > XR_TMA_BUDGET) return false;
+  if (p.smem_bytes > CONV_SMEM_MAX) return false;
   // PIXEL-PAIR rows: when a K-block is the whole pixel (cb == Cin == pixel pitch, <= 32 channels) the even and the odd pixel of
   // a column pair are 2 * rb contiguous bytes in global memory, so the two x-parity planes of a row parity become ONE plane whose
   // rows are [even pixel | odd pixel]: two TMA boxes per K-block with rows twice as wide instead of four -- the TMA unit
@@ -439,7 +391,7 @@ static inline bool plan_conv_s2_tma_impl(const ConvDesc& d, int num_sms, ConvPar
     const int rba = 2 * rb;
     const int lbo = round_up(p.slots * rba, 1024);
     const int bytes = p.smem_off_a + p.S * 2 * lbo + 128 * rba + p.Wp * rba + 1024;
-    if (bytes <= XR_TMA_BUDGET) {
+    if (bytes <= CONV_SMEM_MAX) {
       p.pair = 1;
       p.lbo_a = lbo;
       p.a_stage_bytes = 2 * lbo;
@@ -488,7 +440,7 @@ static inline TmapSet make_s2_tensor_maps(const __half* base, int B, int H, int 
 // its time in its own arrive/wait traffic there (tools/probe_umma.py).  Channels beyond Cin inside the last K-block are
 // out of bounds for the tensor map and arrive as zeros, so Cin only has to be a multiple of 16 (e.g. the 48-channel
 // C3k2 concat).
-static inline bool plan_conv_flat_tma_impl(const ConvDesc& d, int num_sms, ConvParams& p, bool chain = false) {
+static inline bool plan_conv_flat_tma_impl(const ConvDesc& d, int num_sms, ConvParams& p) {
   // also the 2x2 stride-2 ConvTranspose: the same GEMM with N = 4 positions x Cout, scattered by the epilogue
   const bool convt = d.transposed && d.k == 2 && d.stride == 2 && d.res_pitch == 0;
   if (!((d.k == 1 && d.stride == 1 && !d.transposed) || convt)) return false;
@@ -523,11 +475,7 @@ static inline bool plan_conv_flat_tma_impl(const ConvDesc& d, int num_sms, ConvP
   if (nsub > 4) nsub = 4;
   if (nsub == 3) nsub = 2;                         // an item is one or two FULL boxes of <= 256 rows: power-of-two sub-tiles only
   if (nsub < 1) nsub = 1;                          // (N = 80 at more than 64 frames picked 3: two 256-row boxes into 384 slots)
-  if (chain) {                                     // one CTA walks the whole frame: as many sub-tiles per item as it has rows for
-    while (nsub > 1 && 128 * (nsub >> 1) >= p.flat_rows) nsub >>= 1;
-  } else {
-    while (nsub > 1 && ceil_div(tiles128, nsub) < 8 * num_sms) nsub >>= 1;  // keep >= 8 items per CTA for balance
-  }
+  while (nsub > 1 && ceil_div(tiles128, nsub) < 8 * num_sms) nsub >>= 1;  // keep >= 8 items per CTA for balance
   for (;; nsub >>= 1) {
     p.nsub = nsub;
     p.slots = 128 * nsub;
@@ -542,7 +490,7 @@ static inline bool plan_conv_flat_tma_impl(const ConvDesc& d, int num_sms, ConvP
       p.a_stage_bytes = kps * p.slots * rb;          // multiple of 1024 for every cb
       p.b_stage_bytes = kps * b_block;
       const int fixed = round_up(CONV_HDR_BYTES, 1024) + (p.b_resident ? round_up(resident, 1024) : 0);
-      S = (XR_TMA_BUDGET - fixed) / (p.a_stage_bytes + (p.b_resident ? 0 : round_up(p.b_stage_bytes, 1024)));
+      S = (CONV_SMEM_MAX - fixed) / (p.a_stage_bytes + (p.b_resident ? 0 : round_up(p.b_stage_bytes, 1024)));
       if (S > CONV_MAX_STAGES) S = CONV_MAX_STAGES;
       if (S >= 2) break;                             // streamed weights of a wide layer: fewer K-blocks per stage
     }
@@ -552,7 +500,7 @@ static inline bool plan_conv_flat_tma_impl(const ConvDesc& d, int num_sms, ConvP
       break;
     }
   }
-  p.nbuf = choose_nbuf(p.nsub, p.Ntile, ceil_div(p.flat_rows, p.slots) * p.n_tiles, num_sms);
+  p.nbuf = 2;
   p.tmem_cols = pow2_ceil(p.nbuf * p.nsub * p.Ntile);
   p.lbo_a = p.a_stage_bytes;
   p.M_total = ceil_div(p.flat_rows, p.slots);
@@ -561,7 +509,7 @@ static inline bool plan_conv_flat_tma_impl(const ConvDesc& d, int num_sms, ConvP
   const int b_region = p.b_resident ? resident : p.S * round_up(p.b_stage_bytes, 1024);
   p.smem_off_a = p.smem_off_b + round_up(b_region, 1024);
   p.smem_bytes = p.smem_off_a + p.S * p.a_stage_bytes;
-  if (p.smem_bytes > XR_TMA_BUDGET) return false;
+  if (p.smem_bytes > CONV_SMEM_MAX) return false;
   const int work = p.m_tiles * p.n_tiles;
   p.grid = work < num_sms ? work : num_sms;
   p.Wp = 1; p.Hp1 = 1; p.R = 0; p.tpi = 1;
@@ -574,143 +522,27 @@ static inline bool plan_conv_flat_tma_impl(const ConvDesc& d, int num_sms, ConvP
   return true;
 }
 
-// Preferred-budget wrappers (see tma_budget_ref): the smaller footprint is taken only when it costs nothing but ring
-// depth -- same K-block, rows per item, sub-tiles and K-blocks per stage as the unconstrained plan.
-static inline bool same_tiling(const ConvParams& a, const ConvParams& b) {
-  return a.cb == b.cb && a.R == b.R && a.nsub == b.nsub && a.kps == b.kps && a.b_resident == b.b_resident && a.S >= 2;
-}
-static inline bool plan_conv_halo_tma(const ConvDesc& d, int num_sms, ConvParams& p, bool swizzled = true, int max_budget = CONV_SMEM_MAX) {
-  tma_budget_ref() = max_budget;
-  bool ok = plan_conv_halo_tma_impl(d, num_sms, p, swizzled);
-  if (ok && swizzled && tma_wants_split(p, num_sms)) {
+// Planning with the few-work-items split (tma_wants_split): a second pass of the same planner with the N tiles forced.
+template <typename Plan>
+static inline bool plan_with_split(ConvParams& p, int num_sms, Plan plan) {
+  if (!plan(p)) return false;
+  if (const int f = tma_wants_split(p, num_sms)) {
     ConvParams q;
-    tma_force_split_ref() = tma_wants_split(p, num_sms);
-    if (plan_conv_halo_tma_impl(d, num_sms, q, swizzled)) p = q;
+    tma_force_split_ref() = f;
+    if (plan(q)) p = q;
     tma_force_split_ref() = 0;
   }
-  tma_budget_ref() = CONV_SMEM_MAX;
-  if (!ok) return false;
-  if (max_budget != CONV_SMEM_MAX) return true;
-  if (tma_preferred_budget() < CONV_SMEM_MAX) {
-    ConvParams q;
-    tma_budget_ref() = tma_preferred_budget();
-    if (plan_conv_halo_tma_impl(d, num_sms, q, swizzled) && same_tiling(q, p)) p = q;
-    tma_budget_ref() = CONV_SMEM_MAX;
-  }
   return true;
 }
-static inline bool plan_conv_s2_tma(const ConvDesc& d, int num_sms, ConvParams& p, int max_budget = CONV_SMEM_MAX) {
-  tma_budget_ref() = max_budget;
-  bool ok = plan_conv_s2_tma_impl(d, num_sms, p);
-  if (ok && tma_wants_split(p, num_sms)) {
-    ConvParams q;
-    tma_force_split_ref() = tma_wants_split(p, num_sms);
-    if (plan_conv_s2_tma_impl(d, num_sms, q)) p = q;
-    tma_force_split_ref() = 0;
-  }
-  tma_budget_ref() = CONV_SMEM_MAX;
-  if (!ok) return false;
-  if (max_budget != CONV_SMEM_MAX) return true;
-  if (tma_preferred_budget() < CONV_SMEM_MAX) {
-    ConvParams q;
-    tma_budget_ref() = tma_preferred_budget();
-    if (plan_conv_s2_tma_impl(d, num_sms, q) && same_tiling(q, p)) p = q;
-    tma_budget_ref() = CONV_SMEM_MAX;
-  }
-  return true;
+static inline bool plan_conv_halo_tma(const ConvDesc& d, int num_sms, ConvParams& p, bool swizzled = true) {
+  if (!swizzled) return plan_conv_halo_tma_impl(d, num_sms, p, false);
+  return plan_with_split(p, num_sms, [&](ConvParams& q) { return plan_conv_halo_tma_impl(d, num_sms, q); });
 }
-static inline bool plan_conv_flat_tma(const ConvDesc& d, int num_sms, ConvParams& p, int max_budget = CONV_SMEM_MAX) {
-  tma_budget_ref() = max_budget;
-  bool ok = plan_conv_flat_tma_impl(d, num_sms, p);
-  if (ok && tma_wants_split(p, num_sms)) {
-    ConvParams q;
-    tma_force_split_ref() = tma_wants_split(p, num_sms);
-    if (plan_conv_flat_tma_impl(d, num_sms, q)) p = q;
-    tma_force_split_ref() = 0;
-  }
-  tma_budget_ref() = CONV_SMEM_MAX;
-  if (!ok) return false;
-  if (max_budget != CONV_SMEM_MAX) return true;
-  if (tma_preferred_budget() < CONV_SMEM_MAX) {
-    ConvParams q;
-    tma_budget_ref() = tma_preferred_budget();
-    if (plan_conv_flat_tma_impl(d, num_sms, q) && same_tiling(q, p)) p = q;
-    tma_budget_ref() = CONV_SMEM_MAX;
-  }
-  return true;
+static inline bool plan_conv_s2_tma(const ConvDesc& d, int num_sms, ConvParams& p) {
+  return plan_with_split(p, num_sms, [&](ConvParams& q) { return plan_conv_s2_tma_impl(d, num_sms, q); });
 }
-
-// ---- TMA-store epilogue -------------------------------------------------------------------------------------------
-// Direct epilogue stores are one 32-byte sector per lane at the pixel pitch: a warp instruction touches 32 different
-// 128-byte lines and every line is visited once per 16-channel chunk -- the L1 tag stage, not HBM, bounded the wide thin
-// layers (tools/probe_tma.py: b2.cv2 84 us with stores, 73 us without).  With st_tma the epilogue warps write their
-// 16-channel units into a shared-memory image of the item's output tile (conflict-free 16-byte stores in the hardware
-// swizzle) and ONE thread hands the tile to the TMA unit, which writes whole lines.  The destination is always seen as the
-// flat matrix [pixels, channels]: flat mode stores boxes of <= 256 rows; the halo / stride-2 modes store one box per IMAGE
-// ROW (W pixels, starting one tile row after the padding column), because a TMA store that starts at a negative coordinate
-// faults (tools/probe_tma_store.cu: "illegal instruction"; boxes that run past the upper bound are clipped as expected).
-// A store's shared-memory source must be 128-byte aligned: tiles with 64-byte rows are written one row down (st_shift) so
-// that every image row starts on an even tile row (needs an even W + 2, halo mode only).
-// Applies when every epilogue group owns one fixed chunk (Ntile 16 / 32 / 64), one N tile, no ConvTranspose scatter, and the
-// tile fits next to the operand ring without changing the tiling (fewer stages are accepted down to 2).
-// MEASURED (B200, batch 64, profiles/r2_experiments.md): correct on every parity test, but SLOWER than the direct stores in
-// this form -- b2.cv1 42 -> 60 us, b4.cv1 26 -> 35 us, 35.6k -> 34.1k frames/s: one tile per CTA means the epilogue of item
-// i + 1 waits for the TMA unit to have read item i, plus two 512-thread barriers per item, which costs more than the L1 tag
-// cycles it saves.  Opt-in (XRSEG_ST_TMA=1) until the tile is double-buffered.
-// The store path is compiled into the kernel only with -DXRSEG_ST_TMA_BUILD=1 (make variant NAME=sttma FLAGS=-DXRSEG_ST_TMA_BUILD=1):
-// in the product build its address arithmetic and the two extra live registers per unit cost the direct-store epilogue spills
-// and instruction-cache misses in its hot loop (ncu: "no instruction" was the second largest stall of the thin layers).
-#ifndef XRSEG_ST_TMA_BUILD
-#define XRSEG_ST_TMA_BUILD 0
-#endif
-static inline bool tma_store_enabled() {
-  static const bool on = [] { const char* e = getenv("XRSEG_ST_TMA"); return XRSEG_ST_TMA_BUILD && e && e[0] == '1'; }();
-  return on;
-}
-static inline int tma_store_tile_bytes(const ConvParams& p) { return 128 * p.nsub * p.Ntile * 2 + 1024; }
-static inline int tma_store_cw(const ConvParams& p, int split_n) {
-  int cw = p.Ntile < 64 ? p.Ntile : 64;                       // channels per column block (row = 32 / 64 / 128 bytes)
-  if (split_n) while (split_n % cw || (p.Ntile - split_n) % cw) cw >>= 1;
-  return cw;
-}
-static inline bool tma_store_shape_ok(const ConvParams& p, int split_n) {
-  if (!(p.mode == MODE_HALO_TMA || p.mode == MODE_FLAT_TMA || p.mode == MODE_S2_TMA) || !p.sw || p.transposed) return false;
-  const int nch = p.Ntile >> 4;
-  if (p.n_tiles != 1 || !(nch == 1 || nch == 2 || nch == 4)) return false;
-  if (split_n && (split_n % 16 || split_n >= p.Ntile)) return false;
-  if (p.mode != MODE_FLAT_TMA) {
-    const int rbw = tma_store_cw(p, split_n) * 2;
-    if (p.W > 256) return false;
-    if (!(rbw == 128 || (rbw == 64 && p.mode == MODE_HALO_TMA && p.Wp % 2 == 0))) return false;
-  }
-  return true;
-}
-// Adds the output tile to a finished plan (call after plan_conv_*_tma and before packing weights; `replan` re-runs the same
-// planner under a smaller budget).  Returns true when the launch will use the TMA-store epilogue.
-template <typename Replan>
-static inline bool plan_tma_store(ConvParams& p, int split_n, Replan replan) {
-  p.st_tma = 0;
-  if (!tma_store_enabled() || !tma_store_shape_ok(p, split_n)) return false;
-  const int tile = tma_store_tile_bytes(p);
-  if (round_up(p.smem_bytes, 1024) + tile > CONV_SMEM_MAX) {
-    ConvParams q;
-    if (!replan(q, CONV_SMEM_MAX - tile - 1024) || !same_tiling(q, p) || q.Ntile != p.Ntile || q.mode != p.mode) return false;
-    p = q;
-  }
-  p.st_tma = 1;
-  p.st_cw = tma_store_cw(p, split_n);
-  p.st_nblk = p.Ntile / p.st_cw;
-  p.st_shift = (p.mode != MODE_FLAT_TMA && p.st_cw == 32) ? 1 : 0;
-  p.smem_off_o = round_up(p.smem_bytes, 1024);
-  p.smem_bytes = p.smem_off_o + tile;
-  return true;
-}
-// Output tensor map of the TMA-store epilogue for destination `base` (an NHWC slice of C channels, pixel pitch `pitch`,
-// B frames): the flat matrix (C, B*H*W); box = st_cw channels x (<= 256 rows | one image row of W pixels).
-static inline CUtensorMap make_store_tensor_map(const __half* base, const ConvParams& p, int B, int C, int pitch) {
-  const int sw = p.st_cw == 64 ? 3 : (p.st_cw == 32 ? 2 : 1);
-  const int rows_box = p.mode == MODE_FLAT_TMA ? (p.slots < 256 ? p.slots : 256) : p.W;   // s2: p.H / p.W are output geometry
-  return make_halo_tensor_map(base, 1, 1, B * p.H * p.W, C, pitch, rows_box, 1, p.st_cw, sw);
+static inline bool plan_conv_flat_tma(const ConvDesc& d, int num_sms, ConvParams& p) {
+  return plan_with_split(p, num_sms, [&](ConvParams& q) { return plan_conv_flat_tma_impl(d, num_sms, q); });
 }
 
 // Tensor map of the flat mode: the activation matrix [rows, C] (pixel pitch `pitch`) as (C, rows, 1, 1).
@@ -805,20 +637,6 @@ __device__ __forceinline__ void prefetch_tensormap(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(map)) : "memory");
 }
 
-__device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, uint32_t src_smem, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(
-                   reinterpret_cast<uint64_t>(map)),
-               "r"(src_smem), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_group_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_group0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, %0;" ::"n"(32 * TMA_EPI_WARPS) : "memory"); }
-__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-  asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
-}
-
 // MMAs of one pipeline stage for ONE 128-row sub-tile, issued by one thread.  MODE: 0 halo (3x3 s1), 1 parity planes
 // (3x3 s2), 2 flat (1x1 / ConvT, kps K-blocks of one tap).  KJ = k16 steps per K-block.  a_sub / b_lo: low descriptor
 // words (start address >> 4 | LBO field) of the sub-tile's first row and of the stage's first weight tile.
@@ -866,7 +684,7 @@ __device__ __forceinline__ void issue_taps(uint32_t d_tmem, uint32_t a_sub, uint
 // 256-bit store.  hb16 (shared memory) holds 0.5 * bias when ACT (h = 0.5 acc + 0.5 bias is ONE FFMA).
 template <bool ACT, bool RES>
 __device__ __forceinline__ void tma_epilogue_unit(const uint32_t (&v)[16], const float (&hbr)[16], const __half* res, __half* out,
-                                                  int probe, bool valid = true, uint32_t smem0 = 0, uint32_t smem1 = 0) {
+                                                  int probe, bool valid = true) {
   uint32_t o[8];
   if (probe & 2) {                         // PROBE builds only: store the raw accumulators
 #pragma unroll
@@ -928,11 +746,6 @@ __device__ __forceinline__ void tma_epilogue_unit(const uint32_t (&v)[16], const
     if ((o[0] ^ o[1] ^ o[2] ^ o[3] ^ o[4] ^ o[5] ^ o[6] ^ o[7]) == 0x12345678u) st_global_256(out, o);
     return;
   }
-  if (smem0) {                             // TMA-store epilogue: the unit's two 16-byte chunks of the shared-memory tile
-    st_shared_v4(smem0, o[0], o[1], o[2], o[3]);
-    st_shared_v4(smem1, o[4], o[5], o[6], o[7]);
-    return;
-  }
   if (valid) st_global_256(out, o);
 }
 
@@ -944,8 +757,7 @@ __device__ __forceinline__ void tma_epilogue_unit(const uint32_t (&v)[16], const
 // hoisted out of the unit loop: a unit is one TMEM load, the math, one address and one store.
 template <bool PROBE, int KIND, bool ACT, bool RES, bool BREG>
 __device__ __forceinline__ void tma_epilogue_loop(const ConvParams& p, uint32_t tmem_base, uint64_t* tfull, uint64_t* tempty,
-                                                  const float* bias_s, int nbuf, int warp, int lane, int total_work,
-                                                  uint32_t tile_u32, const CUtensorMap* tmap_out, const CUtensorMap* tmap_out2) {
+                                                  const float* bias_s, int nbuf, int warp, int lane, int total_work) {
   constexpr int G = TMA_EPI_GROUPS;
   const int ew = warp - TMA_FIRST_EPI_WARP;
   const int q = warp & 3;              // TMEM lane quadrant this warp may access
@@ -1043,12 +855,6 @@ __device__ __forceinline__ void tma_epilogue_loop(const ConvParams& p, uint32_t 
       __half* const gbase = breg_gbase;
       const int gpitch = breg_gpitch;
       const uint32_t acc_g = acc + static_cast<uint32_t>(gc0 * 16);
-      const bool st_tma = XRSEG_ST_TMA_BUILD && KIND != 2 && p.st_tma != 0;
-      if (st_tma) {
-        // the previous item's tile must have left shared memory before anyone overwrites it
-        if (ew == 0 && lane == 0) bulk_wait_group_read0();
-        epi_bar_sync();
-      }
       uint32_t va[16], vb[16];
       if (!ld_on) {
 #pragma unroll
@@ -1065,66 +871,27 @@ __device__ __forceinline__ void tma_epilogue_loop(const ConvParams& p, uint32_t 
         if (!pipelined) tmem_ld_wait();
         const int px = u == 0 ? pix[0] : (u == 1 ? pix[1] : (u == 2 ? pix[2] : pix[3]));
         const size_t pxs = static_cast<size_t>(px < 0 ? 0 : px);
-        uint32_t s0 = 0, s1 = 0;
-        if (st_tma) {                                  // row 128 u + 32 q + lane of column block n / st_cw, swizzled
-          const uint32_t rbw = static_cast<uint32_t>(p.st_cw) * 2u;
-          const uint32_t blk = static_cast<uint32_t>(n) / static_cast<uint32_t>(p.st_cw);
-          const uint32_t off = static_cast<uint32_t>(128 * u + q * 32 + lane + p.st_shift) * rbw + (static_cast<uint32_t>(n) * 2u) % rbw;
-          const uint32_t mask = rbw == 128u ? 7u : (rbw == 64u ? 3u : 1u);
-          const uint32_t base = tile_u32 + blk * static_cast<uint32_t>(128 * nsub) * rbw;   // (the shifted last row spills into the pad)
-          s0 = base + (off ^ (((off >> 7) & mask) << 4));
-          s1 = base + ((off + 16u) ^ ((((off + 16u) >> 7) & mask) << 4));
-        }
         tma_epilogue_unit<ACT, RES>((j & 1) ? vb : va, hbr, RES ? resp + pxs * res_pitch + n : nullptr, gbase + pxs * gpitch, probe_epi,
-                                    px >= 0, s0, s1);
+                                    px >= 0);
       }
       tc_fence_before();
       __syncwarp();
       if (elect_one()) mbar_arrive(&tempty[buf]);
-      if (st_tma) {
-        fence_proxy_async_smem();                      // generic-proxy writes of the tile -> visible to the TMA unit
-        epi_bar_sync();
-        if (ew == 0 && lane == 0 && !no_store) {
-          for (int blk = 0; blk < p.st_nblk; ++blk) {
-            const int n0 = blk * p.st_cw;
-            const bool second = KIND == 1 && n0 >= split_n;
-            const CUtensorMap* map = second ? tmap_out2 : tmap_out;
-            const int c0 = second ? n0 - split_n : n0;
-            const uint32_t rbw = static_cast<uint32_t>(p.st_cw) * 2u;
-            const uint32_t src = tile_u32 + static_cast<uint32_t>(blk) * static_cast<uint32_t>(128 * nsub) * rbw;
-            if (flat) {
-              for (int r0 = 0; r0 < slots; r0 += 256)
-                tma_store_4d(map, src + static_cast<uint32_t>(r0) * rbw, c0, tile * slots + r0, 0, 0);
-            } else {                                   // one box per image row: W pixels from tile row yy * Wp + 1 (+ shift)
-              for (int yy = 0; yy < Rr && y0 + yy < Hh; ++yy)
-                tma_store_4d(map, src + static_cast<uint32_t>(yy * Wp + 1 + p.st_shift) * rbw, c0, (b * Hh + y0 + yy) * Ww, 0, 0);
-            }
-          }
-          bulk_commit_group();
-        }
-      }
       if (PROBE) e_work += clock64() - t0;
       continue;
     }
-    auto finish_unit = [&](const uint32_t (&v)[16], const float (&hb_in)[16], int u, int c) {
+    // generic path (chunks not fixed per group): the bias of a unit is read from shared memory at the point of use -- fetching
+    // it one unit ahead needs 16 more registers and spills at the 80-register cap of a 21-warp CTA (measured slower)
+    auto finish_unit = [&](const uint32_t (&v)[16], int u, int c) {
       const int px = u == 0 ? pix[0] : (u == 1 ? pix[1] : (u == 2 ? pix[2] : pix[3]));
       if (px < 0) return;
       const int n = n_base + c * 16;
-#if XRSEG_BIAS_PREFETCH
-      const float (&hb)[16] = hb_in;
-#else
-      float hb[16];                                  // A/B build: bias fetched at the point of use
-      if (!BREG) {
+      float hb[16];
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const float4 b4 = reinterpret_cast<const float4*>(bias_s + n)[i];
-          hb[4 * i] = b4.x; hb[4 * i + 1] = b4.y; hb[4 * i + 2] = b4.z; hb[4 * i + 3] = b4.w;
-        }
-      } else {
-#pragma unroll
-        for (int i = 0; i < 16; ++i) hb[i] = hb_in[i];
+      for (int i = 0; i < 4; ++i) {
+        const float4 b4 = reinterpret_cast<const float4*>(bias_s + n)[i];
+        hb[4 * i] = b4.x; hb[4 * i + 1] = b4.y; hb[4 * i + 2] = b4.z; hb[4 * i + 3] = b4.w;
       }
-#endif
       __half* dst;
       if (KIND == 2) {                               // column chunk -> output position (pos >> 1, pos & 1) and channel
         const int pos = fd_div(fd_cout, n);
@@ -1137,51 +904,31 @@ __device__ __forceinline__ void tma_epilogue_loop(const ConvParams& p, uint32_t 
       }
       tma_epilogue_unit<ACT, RES>(v, hb, RES ? resp + static_cast<size_t>(px) * res_pitch + n : nullptr, dst, probe_epi);
     };
-    // bias of a unit: fixed per group (BREG, loaded once above) or fetched from shared memory ONE UNIT AHEAD, together with the
-    // unit's TMEM load, so that the LDS latency (long while the tensor core streams operands) hides under the previous unit
-    auto load_bias = [&](float (&h)[16], int cc) {
-      if (BREG || !XRSEG_BIAS_PREFETCH) return;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const float4 b4 = reinterpret_cast<const float4*>(bias_s + n_base + cc * 16)[i];
-        h[4 * i] = b4.x; h[4 * i + 1] = b4.y; h[4 * i + 2] = b4.z; h[4 * i + 3] = b4.w;
-      }
-    };
     // software pipeline over this group's units (unit k = u * nch + c lives at accumulator column 16 k): the TMEM load of
     // the next unit is in flight while the current one is converted and stored
     int u = gu0, c = gc0, k = grp;
     uint32_t va[16], vb[16];
-    float ha[16], hb[16];
     if (!ld_on) {
 #pragma unroll
       for (int i = 0; i < 16; ++i) va[i] = vb[i] = 0x3f000000u + i + lane;
     }
-    if (k < n_units) {
-      if (ld_on) tmem_ld16(acc + static_cast<uint32_t>(16 * k), va);
-      load_bias(ha, c);
-    }
+    if (k < n_units && ld_on) tmem_ld16(acc + static_cast<uint32_t>(16 * k), va);
     while (k < n_units) {
       int u2 = u, c2 = c + G;
       while (c2 >= nch) { c2 -= nch; ++u2; }
       if (ld_on) tmem_ld_wait();
-      if (k + G < n_units) {
-        if (ld_on) tmem_ld16(acc + static_cast<uint32_t>(16 * (k + G)), vb);
-        load_bias(hb, c2);
-      }
+      if (k + G < n_units && ld_on) tmem_ld16(acc + static_cast<uint32_t>(16 * (k + G)), vb);
       if (!pipelined) tmem_ld_wait();
-      finish_unit(va, BREG ? hbr : ha, u, c);
+      finish_unit(va, u, c);
       k += G;
       if (k >= n_units) break;
       u = u2; c = c2;
       c2 = c + G;
       while (c2 >= nch) { c2 -= nch; ++u2; }
       if (ld_on) tmem_ld_wait();
-      if (k + G < n_units) {
-        if (ld_on) tmem_ld16(acc + static_cast<uint32_t>(16 * (k + G)), va);
-        load_bias(ha, c2);
-      }
+      if (k + G < n_units && ld_on) tmem_ld16(acc + static_cast<uint32_t>(16 * (k + G)), va);
       if (!pipelined) tmem_ld_wait();
-      finish_unit(vb, BREG ? hbr : hb, u, c);
+      finish_unit(vb, u, c);
       k += G;
       u = u2; c = c2;
     }
@@ -1190,25 +937,21 @@ __device__ __forceinline__ void tma_epilogue_loop(const ConvParams& p, uint32_t 
     if (elect_one()) mbar_arrive(&tempty[buf]);
     if (PROBE) e_work += clock64() - t0;
   }
-  if (XRSEG_ST_TMA_BUILD && BREG && KIND != 2 && p.st_tma && ew == 0 && lane == 0) bulk_wait_group0();   // the last tile is in global memory before the CTA exits
   if (PROBE && p.dbg_clk && warp == TMA_FIRST_EPI_WARP && lane == 0) {
     p.dbg_clk[blockIdx.x * 12 + 6] = e_wait;
     p.dbg_clk[blockIdx.x * 12 + 7] = e_work;
   }
 }
 
-// Epilogue of a launch with a fused trailing 1x1 convolution (ConvParams::tail_n; main layer 3x3 stride 1 or 2 with Ntile = N1 in
-// {32, 64}, the 1x1 with N2 = tail_n in {32, 64}).  Group g owns chunk g % (N1/16) of the sub-tiles g / (N1/16), + 4/(N1/16), ...:
+// Epilogue of a launch with a fused trailing 1x1 convolution (ConvParams::tail_n; main layer 3x3 stride 1 with Ntile = N1 = 64,
+// the 1x1 with N2 = tail_n = 32).  Group g owns chunk g % (N1/16) of the sub-tiles g / (N1/16), + 4/(N1/16), ...:
 //   pass 1: 16 accumulator columns -> + bias, SiLU -> 16 fp16 values = 8 packed columns, written BACK into tensor memory inside
 //           the group's own, already consumed, 16-column range -> tready;
 //   the sub-tile's MMA warp then runs D2 = A[TMEM] x W2^T (issue_tail in the kernel);
 //   pass 2 (after t2full): 16 channels of the 1x1 per unit -> + bias2, (SiLU) -> one 32-byte store -> tempty.
-// In-place form (proto.cv2 -> cv3, N1 = 64, N2 = 32, TMEM full): packed columns 64u + {0, 24, 32, 56}, D2 as two N = 16 halves
-// in the freed runs [8, 24) and [40, 56) of the same 64 columns.  Separate form (b1 -> b2.cv1, b3 -> b4.cv1): packed columns
-// N1 u + 16 c, D2 in its own region behind the main accumulators.  The intermediate never reaches shared or global memory.
-__device__ __forceinline__ uint32_t tail_pack_col(int inplace, int c) {
-  return inplace ? (c == 0 ? 0u : (c == 1 ? 24u : (c == 2 ? 32u : 56u))) : static_cast<uint32_t>(16 * c);
-}
+// In place (proto.cv2 -> cv3, TMEM full): packed columns 64u + {0, 24, 32, 56}, D2 as two N = 16 halves in the freed runs
+// [8, 24) and [40, 56) of the same 64 columns.  The intermediate never reaches shared or global memory.
+__device__ __forceinline__ uint32_t tail_pack_col(int c) { return c == 0 ? 0u : (c == 1 ? 24u : (c == 2 ? 32u : 56u)); }
 template <bool PROBE>
 __device__ __forceinline__ void tma_epilogue_loop_tail(const ConvParams& p, uint32_t tmem_base, uint64_t* tfull, uint64_t* tempty,
                                                        uint64_t* tready, uint64_t* t2full, const float* bias_s, int warp, int lane,
@@ -1217,7 +960,7 @@ __device__ __forceinline__ void tma_epilogue_loop_tail(const ConvParams& p, uint
   const int ew = warp - TMA_FIRST_EPI_WARP;
   const int q = warp & 3;
   const int g = ew >> 2;
-  const int nsub = p.nsub, N1 = p.Ntile, N2 = p.tail_n, inplace = p.tail_inplace;
+  const int nsub = p.nsub, N1 = p.Ntile, N2 = p.tail_n;
   const int nch1 = N1 >> 4, nch2 = N2 >> 4;
   const int c1 = g % nch1, u1 = g / nch1, step1 = G / nch1;     // pass 1: chunk c1 of sub-tiles u1, u1 + step1, ...
   const int c2 = g % nch2, u2 = g / nch2, step2 = G / nch2;     // pass 2: chunk c2 of the 1x1's channels, sub-tiles u2, ...
@@ -1226,8 +969,7 @@ __device__ __forceinline__ void tma_epilogue_loop_tail(const ConvParams& p, uint
   __half* const outp = p.out;
   const FastDiv fd_wp = p.fd_wp, fd_tpi = p.fd_hp1;
   const uint32_t lane_taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
-  const uint32_t pk_col = tail_pack_col(inplace, c1);
-  const uint32_t d2_region = static_cast<uint32_t>(2 * nsub * N1);          // separate form: behind the two main accumulator sets
+  const uint32_t pk_col = tail_pack_col(c1);
   float hbr[16];
 #pragma unroll
   for (int i = 0; i < 16; ++i) hbr[i] = bias_s[c1 * 16 + i];
@@ -1293,8 +1035,7 @@ __device__ __forceinline__ void tma_epilogue_loop_tail(const ConvParams& p, uint
     for (int k = 0; k < 4; ++k) {
       const int u = u2 + k * step2;
       if (u >= nsub) break;
-      const uint32_t d2 = inplace ? acc + static_cast<uint32_t>(u * N1) + (c2 ? 40u : 8u)
-                                  : lane_taddr + d2_region + static_cast<uint32_t>((buf * nsub + u) * N2 + 16 * c2);
+      const uint32_t d2 = acc + static_cast<uint32_t>(u * N1) + (c2 ? 40u : 8u);
       uint32_t v[16];
       tmem_ld16(d2, v);
       tmem_ld_wait();
@@ -1363,10 +1104,6 @@ conv_halo_tma_kernel(const __grid_constant__ ConvParams p, const __grid_constant
     prefetch_tensormap(&tmap);
     if (p.mode == MODE_S2_TMA)
       for (int i = 1; i < (p.pair ? 2 : 4); ++i) prefetch_tensormap(&tmaps.m[i]);
-    if (XRSEG_ST_TMA_BUILD && p.st_tma) {
-      prefetch_tensormap(&tmaps.m[4]);
-      if (p.split_n) prefetch_tensormap(&tmaps.m[5]);
-    }
     if (p.b_resident) {
       // resident weights: fetched first thing (they are constants: no dependence on the previous kernel), so the copy
       // runs while warp 1 allocates TMEM -- which may have to wait for a co-resident CTA of the previous kernel
@@ -1511,28 +1248,20 @@ conv_halo_tma_kernel(const __grid_constant__ ConvParams p, const __grid_constant
         else if (!__any_sync(0xffffffffu, mbar_test_wait(&tready[jb], ph))) return false;
         tc_fence_after();
         if (elect_one()) {
-          const int N1 = p.Ntile, N2 = p.tail_n, nch1 = N1 >> 4;
+          const int N1 = p.Ntile;
           const uint32_t accj = tmem_base + static_cast<uint32_t>((jb * p.nsub + my_u) * N1);
           const uint32_t w2 = smem_u32(smem + p.smem_off_w2);
           // W2: [N2 rows][N1 channels] fp16, K-major, rows of N1 * 2 bytes in the hardware swizzle of that width
           const uint32_t rb2 = static_cast<uint32_t>(N1) * 2u;
           const uint64_t hi2 = static_cast<uint64_t>(((8u * rb2) >> 4) | (1u << 14) | ((rb2 == 128u ? 2u : 4u) << 29)) << 32;
-          if (p.tail_inplace) {
-            const uint32_t idesc16 = umma_idesc_f16(16, 0);
+          const uint32_t idesc16 = umma_idesc_f16(16, 0);
 #pragma unroll
-            for (int hh = 0; hh < 2; ++hh) {
-              const uint32_t b_lo2 = (((w2 + static_cast<uint32_t>(hh) * 16u * rb2) >> 4) & 0x3FFFu) | (1u << 16);
-              const uint32_t d2 = accj + (hh ? 40u : 8u);
+          for (int hh = 0; hh < 2; ++hh) {
+            const uint32_t b_lo2 = (((w2 + static_cast<uint32_t>(hh) * 16u * rb2) >> 4) & 0x3FFFu) | (1u << 16);
+            const uint32_t d2 = accj + (hh ? 40u : 8u);
 #pragma unroll
-              for (int j2 = 0; j2 < 4; ++j2)
-                umma_f16_ts(d2, accj + tail_pack_col(1, j2), hi2 | (b_lo2 + 2u * j2), idesc16, j2 > 0 ? 1u : 0u);
-            }
-          } else {
-            const uint32_t idesc2 = umma_idesc_f16(N2, 0);
-            const uint32_t b_lo2 = ((w2 >> 4) & 0x3FFFu) | (1u << 16);
-            const uint32_t d2 = tmem_base + static_cast<uint32_t>(2 * p.nsub * N1 + (jb * p.nsub + my_u) * N2);
-            for (int j2 = 0; j2 < nch1; ++j2)
-              umma_f16_ts(d2, accj + static_cast<uint32_t>(16 * j2), hi2 | (b_lo2 + 2u * j2), idesc2, j2 > 0 ? 1u : 0u);
+            for (int j2 = 0; j2 < 4; ++j2)
+              umma_f16_ts(d2, accj + tail_pack_col(j2), hi2 | (b_lo2 + 2u * j2), idesc16, j2 > 0 ? 1u : 0u);
           }
           umma_commit(&t2full[jb]);
         }
@@ -1670,8 +1399,7 @@ conv_halo_tma_kernel(const __grid_constant__ ConvParams p, const __grid_constant
     const bool breg = p.n_tiles == 1 && nch_ <= TMA_EPI_GROUPS && TMA_EPI_GROUPS % nch_ == 0;
     const int sel = (breg ? 16 : 0) + kind * 4 + (p.act ? 2 : 0) + (p.res ? 1 : 0);
 #define XR_EPI_CASE(id, K, A, R, B) \
-  case id: tma_epilogue_loop<PROBE, K, A, R, B>(p, tmem_base, tfull, tempty, bias_s, nbuf, warp, lane, total_work, \
-                                                smem_u32(smem + p.smem_off_o), &tmaps.m[4], &tmaps.m[5]); break;
+  case id: tma_epilogue_loop<PROBE, K, A, R, B>(p, tmem_base, tfull, tempty, bias_s, nbuf, warp, lane, total_work); break;
     switch (sel) {
       XR_EPI_CASE(0, 0, false, false, false) XR_EPI_CASE(1, 0, false, true, false) XR_EPI_CASE(2, 0, true, false, false)
       XR_EPI_CASE(3, 0, true, true, false) XR_EPI_CASE(4, 1, false, false, false) XR_EPI_CASE(6, 1, true, false, false)

@@ -100,22 +100,13 @@ struct ConvParams {
   // output columns >= split_n go to out2 (pixel pitch out2_pitch), relative to split_n.  split_n == 0: single output.
   __half* out2;
   int split_n, out2_pitch;
-  // TMA-store epilogue (conv_tma.cuh: plan_tma_store): the epilogue writes the item's fp16 output tile into shared memory
-  // ([st_nblk column blocks][128 * nsub rows][st_cw channels], hardware swizzle of the row width) and one thread stores it
-  // with cp.async.bulk.tensor (tensor maps TmapSet::m[4] / m[5]); 0 = direct 32-byte stores from registers.
-  int st_tma, st_cw, st_nblk, smem_off_o, st_shift;   // st_shift: tile rows are written one row down (128-byte aligned image rows)
   // Fused trailing 1x1 convolution (conv_tma.cuh "tail"): the 64-channel output of a 3x3 layer never leaves the SM -- the epilogue
   // writes it back into tensor memory as packed fp16, a second set of MMAs (A from TMEM, W2 from shared memory) produces the
   // tail_n = 32 output channels of the 1x1 layer in the freed accumulator columns, a second epilogue pass stores those.
   // `out` / `out_pitch` are then the TAIL's destination.  tail_n == 0: off.
   int tail_n, tail_act, smem_off_w2;
-  int tail_inplace;                 // 1: Ntile 64 -> 32 inside the sub-tile's own 64 columns (TMEM full); 0: the 1x1's accumulators live in
-                                    // their own TMEM region behind the main ones (column nbuf * nsub * Ntile + (buf * nsub + u) * tail_n)
   const __half* tail_w;             // [32][64] fp16, K-major 128-byte swizzle (pack_conv_weights_sw image of the 1x1 layer)
   const float* tail_bias;           // [32]
-  // Chain kernel (conv_chain.cuh), flat mode: rows of ONE frame (H * W); a work item is `slots` rows of one frame and
-  // tpi = ceil(frame_rows / slots) items make a frame.  0 outside chains.
-  int frame_rows;
 };
 
 struct ConvDesc {

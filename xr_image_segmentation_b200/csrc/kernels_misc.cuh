@@ -238,9 +238,10 @@ __device__ __forceinline__ void dw_fma8(float (&acc)[8], const uint4 v, const fl
 // added in fp32.  Against a full fp32 accumulation this adds ~1e-3 relative error (the output is rounded to fp16 anyway)
 // and cuts the instruction count per 8 outputs from ~150 (72 conversions + 72 FMAs) to ~50; with the weights held as
 // 36 half2 registers the kernel also fits more blocks per SM.
-// NV = half2 lanes per thread: a thread owns 2*NV channels of one pixel column.  NV = 2 (four channels, 8-byte accesses)
-// halves the per-thread state (~60 registers) and doubles the threads: the kernel is latency-bound at the 25 %
-// occupancy the 8-channel version reaches.
+// NV = half2 lanes per thread: a thread owns 2*NV channels of one pixel column; the network launches NV = 4 (eight channels,
+// 16-byte accesses).  NV = 2 halves the per-thread state (~60 registers) and doubles the occupancy: measured equal.  Staging
+// the input tile in shared memory (fetched once by cp.async) was measured slower on B200: h3.cls.0dw / 1dw 51.5 / 59.9 us
+// against 48.2 / 51.6 us -- the barrier between fill and compute costs more than the L1 re-reads it saves.
 template <int NV>
 struct alignas(NV * 4) DwVec {
   uint32_t v[NV];
@@ -346,131 +347,6 @@ __global__ void __launch_bounds__(128, NV == 2 ? 8 : 4) dwconv3x3_kernel(const D
     // roll: the row below becomes the middle row, the middle row becomes the row above
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
-      s_up0[i] = s_mid0[i];
-      s_mid0[i] = s_dn0[i];
-      s_mid1[i] = s_dn1[i];
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// The same depthwise convolution with the input tile staged in shared memory (opt-in, XRSEG_DW_SMEM=1; measured SLOWER than
-// the register version above on B200: h3.cls.0dw / 1dw 51.5 / 59.9 us against 48.2 / 51.6 us, 32.5k against 33.0k frames/s,
-// gpurun_out r2i -- the barrier between fill and compute costs more than the L1 re-reads it saves).  The register version keeps three 16-byte loads per thread in flight and re-reads every input
-// pixel three times through L1: ~24 KB in flight per SM at its 25 % occupancy, a third of what HBM needs, and it ran at a
-// third of the HBM roofline (h3.cls.1dw 51 us for 131 MB).  Here a block owns TR output rows x the full width x CG groups of
-// 8 channels; its (TR + 2) x (W + 2) x CG halo tile is fetched ONCE with 16-byte cp.async (zero fill outside the image =
-// the convolution's padding, so the compute loop has no bounds checks), all of it in flight at once, six or more blocks
-// per SM.  Arithmetic and rounding are those of the register version.
-// ------------------------------------------------------------------------------------------------
-struct DwSmemGeom {
-  int TR, CG, threads, smem_bytes;
-};
-static inline DwSmemGeom dw_smem_geom(int W, int C) {
-  DwSmemGeom g;
-  const int groups = C / 8;
-  g.CG = W >= 80 ? 2 : (W >= 40 ? 4 : 8);
-  if (g.CG > groups) g.CG = groups;
-  while (groups % g.CG) --g.CG;                      // whole blocks of channel groups (C = 80: 10 groups -> CG 2 / 2 / 5)
-  g.TR = W >= 40 ? 8 : 10;
-  g.threads = ((W * g.CG + 31) / 32) * 32;
-  g.smem_bytes = (g.TR + 2) * (W + 2) * g.CG * 16;
-  return g;
-}
-
-__global__ void __launch_bounds__(192, 4) dwconv3x3_smem_kernel(const DwParams p, int TR, int CG) {
-  XR_PDL_ENTRY();
-  extern __shared__ __align__(16) uint8_t dw_tile[];            // [(TR+2)][(W+2)][CG] x 16 bytes
-  const int Wp = p.W + 2;
-  const int b = blockIdx.z, y0 = blockIdx.y * TR, g0 = blockIdx.x * CG;
-  const size_t row_elems = static_cast<size_t>(p.W) * p.in_pitch;
-  const __half* img = p.in + static_cast<size_t>(b) * p.H * row_elems;
-  // stage the halo tile: element (r, cx, g) = input pixel (y0 - 1 + r, cx - 1), channels of group g0 + g
-  const int n_chunks = (TR + 2) * Wp * CG;
-  for (int i = threadIdx.x; i < n_chunks; i += blockDim.x) {
-    const int g = i % CG, rc = i / CG;
-    const int cx = rc % Wp, r = rc / Wp;
-    const int y = y0 - 1 + r, x = cx - 1;
-    const int c = (g0 + g) * 8;
-    const int cin = p.in_grp > 0 ? (c / p.in_grp) * p.in_grp_stride + p.in_grp_off + c % p.in_grp : c;
-    const bool in = y >= 0 && y < p.H && x >= 0 && x < p.W;
-    const __half* src = in ? img + static_cast<size_t>(y) * row_elems + static_cast<size_t>(x) * p.in_pitch + cin : img;
-    cp_async16(smem_u32(dw_tile + static_cast<size_t>(i) * 16), src, in ? 16u : 0u);
-  }
-  cp_async_commit();
-  // weights of this thread's channel group while the tile is in flight
-  const int col = threadIdx.x;                                   // (x, g), g fastest
-  const bool active = col < p.W * CG;
-  const int x = col / CG, g = col - x * CG;
-  const int c = (g0 + g) * 8;
-  __half2 w[9][4];
-  float bias[8];
-  if (active) {
-#pragma unroll
-    for (int t = 0; t < 9; ++t)
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const float2 wf = *reinterpret_cast<const float2*>(p.w + t * p.C + c + 2 * i);
-        w[t][i] = __floats2half2_rn(wf.x, wf.y);
-      }
-#pragma unroll
-    for (int i = 0; i < 8; ++i) bias[i] = p.bias[c + i];
-  }
-  cp_async_wait<0>();
-  __syncthreads();
-  if (!active) return;
-  const uint4* tile = reinterpret_cast<const uint4*>(dw_tile);
-  auto sums_of = [&](int r, __half2 (&a0)[4], __half2 (&a1)[4], __half2 (&a2)[4]) {     // input row y0 - 1 + r of the tile
-    const uint4* q = tile + (static_cast<size_t>(r) * Wp + x) * CG + g;                  // left neighbour (cx = x)
-    const uint4 vl = q[0], vc = q[CG], vr = q[2 * CG];
-    const __half2* hl = reinterpret_cast<const __half2*>(&vl);
-    const __half2* hc = reinterpret_cast<const __half2*>(&vc);
-    const __half2* hr = reinterpret_cast<const __half2*>(&vr);
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      a0[i] = __hfma2(hr[i], w[2][i], __hfma2(hc[i], w[1][i], __hmul2(hl[i], w[0][i])));
-      a1[i] = __hfma2(hr[i], w[5][i], __hfma2(hc[i], w[4][i], __hmul2(hl[i], w[3][i])));
-      a2[i] = __hfma2(hr[i], w[8][i], __hfma2(hc[i], w[7][i], __hmul2(hl[i], w[6][i])));
-    }
-  };
-  __half2 s_up0[4], s_mid0[4], s_mid1[4], s_dn0[4], s_dn1[4], s_dn2[4], dummy[4];
-  sums_of(0, s_up0, dummy, dummy);
-  sums_of(1, s_mid0, s_mid1, dummy);
-  const int y1 = min(y0 + TR, p.H);
-  size_t opix = (static_cast<size_t>(b) * p.H + y0) * p.W + x;
-  for (int y = y0; y < y1; ++y, opix += p.W) {
-    sums_of(y - y0 + 2, s_dn0, s_dn1, s_dn2);
-    float acc[8];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const float2 a = __half22float2(s_up0[i]), m = __half22float2(s_mid1[i]), d = __half22float2(s_dn2[i]);
-      acc[2 * i] = bias[2 * i] + a.x + m.x + d.x;
-      acc[2 * i + 1] = bias[2 * i + 1] + a.y + m.y + d.y;
-    }
-    uint4 o;
-    uint32_t* ov = reinterpret_cast<uint32_t*>(&o);
-    if (p.act) {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) ov[i] = silu_pack_h2(acc[2 * i], acc[2 * i + 1]);
-    } else {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        __half2 hh = __floats2half2_rn(acc[2 * i], acc[2 * i + 1]);
-        ov[i] = *reinterpret_cast<uint32_t*>(&hh);
-      }
-    }
-    if (p.res) {
-      const uint4 raw = *reinterpret_cast<const uint4*>(p.res + opix * p.res_pitch + c);
-      const uint32_t* rv = reinterpret_cast<const uint32_t*>(&raw);
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        __half2 sum = __hadd2(*reinterpret_cast<__half2*>(&ov[i]), *reinterpret_cast<const __half2*>(&rv[i]));
-        ov[i] = *reinterpret_cast<uint32_t*>(&sum);
-      }
-    }
-    *reinterpret_cast<uint4*>(p.out + opix * p.out_pitch + c) = o;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
       s_up0[i] = s_mid0[i];
       s_mid0[i] = s_dn0[i];
       s_mid1[i] = s_dn1[i];

@@ -9,7 +9,6 @@
 
 #include <string.h>
 
-#include <functional>
 #include <map>
 #include <string>
 #include <vector>
@@ -29,7 +28,7 @@ struct LayerRec {
   int cin, cout, k, stride, groups, act, transposed, h_in, w_in;
 };
 
-enum OpKind { OP_STEM, OP_CONV, OP_DW, OP_SPPF, OP_UP, OP_ATTN, OP_BNECK, OP_C3K2, OP_CHAIN };
+enum OpKind { OP_STEM, OP_CONV, OP_DW, OP_SPPF, OP_UP, OP_ATTN, OP_BNECK };
 
 struct Op {
   OpKind kind;
@@ -50,17 +49,10 @@ struct Op {
   // the kernel; ytail is its destination (y stays the never-materialised intermediate)
   int tail_layer = -1, tail_act = 0;
   TV ytail;
-  // OP_C3K2 (whole-block fusion): layer = X.cv1, layer2 = X.m0.cv1, layer3 = X.m0.cv2, layer4 = X.cv2
-  int layer3 = -1, layer4 = -1;
-  // OP_CHAIN (conv_chain.cuh): consecutive convolutions of the 20x20 / 40x40 stages run by one launch, a CTA per frame;
-  // `chain` holds the OP_CONV ops in order (x / y of the chain op itself are those of its first / last convolution)
-  std::vector<Op> chain;
 };
 
 // Channel triples (input, middle, output; as laid out in shared memory) the fused Bottleneck kernel is built for
 // (bottleneck.cuh).  Anything else keeps its two tcgen05 launches.
-// (input, split width c, bottleneck middle, output) of the C3k2 blocks the whole-block kernel is built for
-static inline bool c3k2_supported(int cin, int c, int cm, int cout) { return cin == 32 && c == 16 && cm == 8 && cout == 64; }
 static inline bool bneck_supported(int c1, int cm, int c2) {
   return (c1 == 16 && cm == 8 && c2 == 16) || (c1 == 32 && cm == 16 && c2 == 32);
 }
@@ -100,13 +92,12 @@ class Net {
   bool fuse_bneck = true;                 // Bottleneck fusion (fuse_bottlenecks)
   bool fuse_pe = true;                    // C2PSA positional encoding inside the attention kernel (fuse_attention_pe)
   bool fuse_tail = true;                  // proto.cv3 (1x1, 64 -> 32) inside proto.cv2's launch (fuse_tail_1x1)
-  bool fuse_c3k2 = false;                 // whole-block fusion (fuse_c3k2_blocks); measured slower, opt-in (XRSEG_FUSE_C3K2=1)
   TV input;                 // [B,640,640,4] fp16
   TV box[3], cls[3], coef[3], protos;
   int fh[3], fw[3];
 
-  Net(int scale, int batch, int in_hw = 640, bool fuse = true, bool bneck = true, bool c3k2_blocks = false)
-      : B(batch), sp(make_spec(scale)), fuse_enabled(fuse), fuse_bneck(fuse && bneck), fuse_tail(fuse), fuse_c3k2(c3k2_blocks) { build(in_hw); }
+  Net(int scale, int batch, int in_hw = 640, bool fuse = true, bool bneck = true)
+      : B(batch), sp(make_spec(scale)), fuse_enabled(fuse), fuse_bneck(fuse && bneck), fuse_tail(fuse) { build(in_hw); }
 
   TV alloc(int H, int W, int C, int pitch_override = 0) {
     TV t;
@@ -252,17 +243,12 @@ class Net {
 
   // A 3x3 convolution whose ONLY consumer is a 1x1 convolution (rows are independent for a 1x1) runs that 1x1 inside its own
   // launch as a second set of MMAs on the epilogue's fp16 tile kept in tensor memory (ConvParams::tail_n, conv_tma.cuh): the
-  // intermediate tensor is never written to HBM or read back.  The kernel side handles 32 / 64 channels on either side; the
-  // pairs below are the ones whose TMEM budget works out on the n scale:
-  //   proto.cv2 (64) -> proto.cv3 (32)   in place (512 accumulator columns are all in use)
-  //   b1 (32) -> b2.cv1 (32),  b3 (64) -> b4.cv1 (64)   the stride-2 stage convs feed only the next C3k2 block's cv1;
-  //                                                      256 + 256 columns
-  // Anything else keeps its two launches.
+  // intermediate tensor is never written to HBM or read back.  The one pair is proto.cv2 (64) -> proto.cv3 (32), in place (512
+  // accumulator columns are all in use).  The stride-2 stage pairs b1 -> b2.cv1 and b3 -> b4.cv1 were measured too: 76 + 43 ->
+  // 113 us and 66 + 27 -> 88 us, frames/s unchanged -- these layers are bound by their epilogue, and two epilogue passes in one
+  // launch cost what the second launch did.  Anything else keeps its two launches.
   void fuse_tail_1x1() {
     static const bool env_on = [] { const char* e = getenv("XRSEG_FUSE_TAIL"); return !(e && e[0] == '0'); }();
-    // the stage pairs are opt-in: measured b1 + b2.cv1 76 + 43 -> 113 us, b3 + b4.cv1 66 + 27 -> 88 us, frames/s unchanged -- these
-    // layers are bound by their epilogue, and two epilogue passes in one launch cost what the second launch did
-    static const bool env_stage = [] { const char* e = getenv("XRSEG_FUSE_TAIL_STAGE"); return e && e[0] == '1'; }();
     if (!fuse_tail || !env_on) return;
     for (size_t i = 0; i + 1 < ops.size(); ++i) {
       Op& a = ops[i];
@@ -270,10 +256,7 @@ class Net {
       if (a.kind != OP_CONV || b.kind != OP_CONV || a.layer2 >= 0 || b.layer2 >= 0 || a.tail_layer >= 0) continue;
       const std::string &na = layers[a.layer].name, &nb = layers[b.layer].name;
       const bool proto = na == "proto.cv2" && nb == "proto.cv3" && a.stride == 1 && a.y.Cp == 64 && b.y.Cp == 32;
-      const bool stage = env_stage && a.stride == 2 &&
-                         ((na == "b1" && nb == "b2.cv1" && a.y.Cp == 32 && b.y.Cp == 32 && a.y.W == 160) ||
-                          (na == "b3" && nb == "b4.cv1" && a.y.Cp == 64 && b.y.Cp == 64 && a.y.W == 80));
-      if (!proto && !stage) continue;
+      if (!proto) continue;
       const bool ok = a.k == 3 && !a.transposed && a.act && !a.has_res && b.k == 1 && b.stride == 1 && !b.transposed && !b.has_res &&
                       b.x.off == a.y.off && b.x.pitch == a.y.pitch && b.x.Cp == a.y.Cp && a.branch == b.branch && b.wait_tag == 0 &&
                       a.signal_tag == 0;
@@ -331,63 +314,6 @@ class Net {
       a.signal_tag = b.signal_tag;
       ops.erase(ops.begin() + i + 1);
     }
-  }
-
-  // X.cv1 (1x1) -> fused Bottleneck -> X.cv2 (1x1) over the block's concat buffer become ONE launch when the channel
-  // counts are small enough for everything to stay in shared memory (b2 of the n scale): the concat buffer is never
-  // materialised.  Runs after fuse_bottlenecks().
-  void fuse_c3k2_blocks() {
-    if (!fuse_bneck || !fuse_c3k2) return;
-    for (size_t i = 0; i + 2 < ops.size(); ++i) {
-      Op& a = ops[i];
-      const Op m = ops[i + 1], z = ops[i + 2];
-      if (a.kind != OP_CONV || m.kind != OP_BNECK || z.kind != OP_CONV || a.layer2 >= 0 || z.layer2 >= 0) continue;
-      const int c = m.x.Cp;
-      const bool chain = a.k == 1 && z.k == 1 && a.stride == 1 && z.stride == 1 && a.act && z.act && !a.has_res && !z.has_res &&
-                         !a.transposed && !z.transposed && m.has_res && a.y.Cp == 2 * c && m.x.off == a.y.off + c &&
-                         m.y.off == a.y.off + 2 * c && z.x.off == a.y.off && z.x.Cp == 3 * c && z.x.pitch == a.y.pitch &&
-                         a.branch == m.branch && m.branch == z.branch && m.wait_tag == 0 && z.wait_tag == 0 &&
-                         a.signal_tag == 0 && m.signal_tag == 0 && layers[a.layer].cout == 2 * c && layers[z.layer].cin == 3 * c;
-      if (!chain || !c3k2_supported(a.x.Cp, c, round_up(layers[m.layer].cout, 8), z.y.Cp)) continue;
-      a.kind = OP_C3K2;
-      a.layer2 = m.layer; a.layer3 = m.layer2; a.layer4 = z.layer;
-      a.y = z.y;
-      a.signal_tag = z.signal_tag;
-      ops.erase(ops.begin() + i + 1, ops.begin() + i + 3);
-    }
-  }
-
-  // Consecutive OP_CONV ops on small maps (input <= 40x40) of the same branch become one OP_CHAIN launch: a CTA walks the
-  // whole chain for one frame (frames are independent, so no grid-wide dependency exists inside these stages).  `can_chain`
-  // says whether the chain kernel has a plan for a convolution.  A chain starts at an op that waits for an event (or at any
-  // eligible op) and ends at an op that signals one, so the branch / event structure of the graph is unchanged.
-  void fuse_chains(const std::function<bool(const Op&)>& can_chain, int max_pixels = 1600) {
-    std::vector<Op> out;
-    for (size_t i = 0; i < ops.size();) {
-      auto eligible = [&](const Op& o) {
-        return o.kind == OP_CONV && !o.transposed && o.x.H * o.x.W <= max_pixels && can_chain(o);
-      };
-      if (!eligible(ops[i])) { out.push_back(ops[i++]); continue; }
-      size_t j = i + 1;
-      if (ops[i].signal_tag == 0)
-        while (j < ops.size() && eligible(ops[j]) && ops[j].branch == ops[i].branch && ops[j].wait_tag == 0) {
-          ++j;
-          if (ops[j - 1].signal_tag != 0) break;     // a signalling op ends its chain
-        }
-      if (j - i < 2) { out.push_back(ops[i++]); continue; }
-      Op c;
-      c.kind = OP_CHAIN;
-      c.layer = ops[i].layer;
-      c.x = ops[i].x;
-      c.y = ops[j - 1].y;
-      c.branch = ops[i].branch;
-      c.wait_tag = ops[i].wait_tag;
-      c.signal_tag = ops[j - 1].signal_tag;
-      c.chain.assign(ops.begin() + i, ops.begin() + j);
-      out.push_back(c);
-      i = j;
-    }
-    ops.swap(out);
   }
 
   void build(int hw) {
@@ -477,7 +403,6 @@ class Net {
     named["p3"] = p3; named["p4"] = p4; named["p5"] = p5;
     fuse_siblings();
     fuse_bottlenecks();
-    fuse_c3k2_blocks();
     fuse_attention_pe();
     fuse_tail_1x1();
     fh[0] = p3.H; fw[0] = p3.W; fh[1] = p4.H; fw[1] = p4.W; fh[2] = p5.H; fw[2] = p5.W;

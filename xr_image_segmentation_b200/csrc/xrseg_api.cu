@@ -17,7 +17,6 @@
 
 #include "common.cuh"
 #include "conv_tma.cuh"
-#include "conv_chain.cuh"
 #include "conv_umma.cuh"
 #include "kernels_misc.cuh"
 #include "model.cuh"
@@ -48,19 +47,6 @@ struct DevLayer {
   __half* w16_rows = nullptr;      // stem_rows_kernel weights
 };
 
-// one OP_CHAIN launch (conv_chain.cuh): the per-layer plans + tensor maps in device memory
-struct ChainDev {
-  ChainLayer* d_layers = nullptr;
-  int n = 0, smem = 0;
-};
-
-// XRSEG_CHAIN=1: the convolutions of the 20x20 / 40x40 stages as per-frame chain launches (conv_chain.cuh).  Parity-tested,
-// but measured no faster than one launch per layer (DESIGN.md section 4, dead ends): off unless asked for.
-bool chains_disabled() {
-  const char* e = getenv("XRSEG_CHAIN");
-  return !(e && e[0] == '1');
-}
-
 // ---- fused Bottleneck (bottleneck.cuh): one instantiation per supported channel triple ---------------------------------
 template <int C1, int CM, int C2, int TH>
 void bneck_launch_t(const BneckParams& p, bool res, cudaStream_t st) {
@@ -79,14 +65,6 @@ void bneck_prepare_device() {
   bneck_prepare_t<16, 8, 16, 14>();
   bneck_prepare_t<32, 16, 32, 14>();
 }
-void c3k2_prepare_device() {
-  XR_CUDA(cudaFuncSetAttribute(c3k2_mma_kernel<32, 16, 8, 64, 14>, cudaFuncAttributeMaxDynamicSharedMemorySize, C3k2Cfg<32, 16, 8, 64, 14>::SMEM_BYTES));
-}
-void launch_c3k2(int cin, int c, int cm, int cout, const C3k2Params& p, cudaStream_t st) {
-  XR_CHECK(c3k2_supported(cin, c, cm, cout), "no fused C3k2 kernel for %d-%d-%d-%d channels", cin, c, cm, cout);
-  const dim3 grid(ceil_div(p.W, BNECK_TW), ceil_div(p.H, 14), p.B);
-  launch_k(c3k2_mma_kernel<32, 16, 8, 64, 14>, grid, 256, C3k2Cfg<32, 16, 8, 64, 14>::SMEM_BYTES, st, p);
-}
 void launch_bneck(int c1, int cm, int c2, const BneckParams& p, bool res, cudaStream_t st) {
   if (c1 == 16 && cm == 8 && c2 == 16) bneck_launch_t<16, 8, 16, 14>(p, res, st);
   else if (c1 == 32 && cm == 16 && c2 == 32) bneck_launch_t<32, 16, 32, 14>(p, res, st);
@@ -102,10 +80,6 @@ bool flat_tma_disabled() {
 bool branches_disabled() {   // XRSEG_BRANCHES=0: everything on one stream (A/B measurements)
   const char* e = getenv("XRSEG_BRANCHES");
   return e && e[0] == '0';
-}
-bool dw_wide() {   // 8 channels per thread unless XRSEG_DW_NARROW=1 (4 channels, twice the occupancy: measured equal)
-  const char* e = getenv("XRSEG_DW_NARROW");
-  return !(e && e[0] == '1');
 }
 bool mask_mma_enabled() {
   const char* e = getenv("XRSEG_MASK_MMA");
@@ -141,7 +115,6 @@ struct xrseg_runner {
   int mb = 1;                      // frames per network pass
   int A = 8400;
   std::vector<DevLayer> dl;
-  std::vector<ChainDev> chains;    // indexed like net->ops (empty entries for everything but OP_CHAIN)
   __half* arena = nullptr;
   uint8_t* d_frames = nullptr;
   size_t d_frames_cap = 0;
@@ -192,83 +165,11 @@ inline __half* ptr_of(xrseg_runner* r, const TV& t) { return r->arena + t.off; }
 // ------------------------------------------------------------------------------------------------
 // weights -> device, per layer kind
 // ------------------------------------------------------------------------------------------------
-ConvDesc conv_desc_of(const Op& o, int batch) {
-  ConvDesc cd{};
-  cd.B = batch; cd.H = o.x.H; cd.W = o.x.W; cd.Cin = o.x.Cp; cd.in_pitch = o.x.pitch;
-  cd.Cout = o.y.Cp + (o.layer2 >= 0 ? o.y2.Cp : 0); cd.out_pitch = o.y.pitch;
-  cd.k = o.k; cd.stride = o.stride; cd.act = o.act; cd.transposed = o.transposed;
-  cd.res_pitch = o.has_res ? o.res.pitch : 0;
-  return cd;
-}
-
-// weights of a convolution op (with its fused sibling, if any) as one [Cout_a padded | Cout_b] x Cin x k x k matrix
-const HostLayerWeights& conv_weights_of(const Net& net, const Op& o, const std::vector<HostLayerWeights>& hw, HostLayerWeights& fused,
-                                        int* cout_real) {
-  const LayerRec& l = net.layers[o.layer];
-  *cout_real = l.cout;
-  if (o.layer2 < 0) return hw[o.layer];
-  const LayerRec& l2 = net.layers[o.layer2];
-  const HostLayerWeights &w = hw[o.layer], &w2 = hw[o.layer2];
-  const size_t per = static_cast<size_t>(l.cin) * l.k * l.k;
-  fused.w.assign((static_cast<size_t>(o.y.Cp) + l2.cout) * per, 0.f);
-  fused.b.assign(static_cast<size_t>(o.y.Cp) + l2.cout, 0.f);
-  std::copy(w.w.begin(), w.w.end(), fused.w.begin());
-  std::copy(w.b.begin(), w.b.end(), fused.b.begin());
-  std::copy(w2.w.begin(), w2.w.end(), fused.w.begin() + static_cast<size_t>(o.y.Cp) * per);
-  std::copy(w2.b.begin(), w2.b.end(), fused.b.begin() + o.y.Cp);
-  *cout_real = o.y.Cp + l2.cout;
-  return fused;
-}
-
-// OP_CHAIN: plan every convolution of the chain for the chain kernel, pack its weights, build its tensor maps, and put the
-// resulting ChainLayer array into device memory
-void upload_chain(xrseg_runner* r, size_t op_index, const Op& o, const std::vector<HostLayerWeights>& hw) {
-  Net& net = *r->net;
-  std::vector<ChainLayer> host;
-  int smem = 0;
-  for (const Op& s : o.chain) {
-    const LayerRec& l = net.layers[s.layer];
-    DevLayer& d = r->dl[s.layer];
-    XR_CHECK(plan_chain_layer(conv_desc_of(s, r->mb), d.cp), "no chain plan for %s", l.name.c_str());
-    d.use_tma = true;
-    if (d.cp.mode == MODE_HALO_TMA)
-      d.tmaps.m[0] = make_halo_tensor_map(ptr_of(r, s.x), r->mb, s.x.H, s.x.W, s.x.Cp, s.x.pitch, d.cp.Wp, d.cp.hbox, d.cp.cb, d.cp.sw);
-    else if (d.cp.mode == MODE_FLAT_TMA)
-      d.tmaps.m[0] = make_flat_tensor_map(ptr_of(r, s.x), static_cast<long>(r->mb) * s.x.H * s.x.W, s.x.Cp, s.x.pitch, d.cp);
-    else
-      d.tmaps = make_s2_tensor_maps(ptr_of(r, s.x), r->mb, s.x.H, s.x.W, s.x.Cp, s.x.pitch, d.cp);
-    HostLayerWeights fused;
-    int cout_real = 0;
-    const HostLayerWeights& wsrc = conv_weights_of(net, s, hw, fused, &cout_real);
-    std::vector<__half> wp;
-    std::vector<float> bp;
-    pack_conv_weights_sw<__half>(d.cp, wsrc.w.data(), wsrc.b.data(), l.cin, cout_real, wp, bp);
-    d.wpack = dev_upload(wp);
-    d.bias = dev_upload(bp);
-    ChainLayer cl{};
-    cl.tmaps = d.tmaps;
-    cl.p = d.cp;
-    cl.p.in = ptr_of(r, s.x); cl.p.out = ptr_of(r, s.y);
-    if (s.layer2 >= 0) { cl.p.out2 = ptr_of(r, s.y2); cl.p.split_n = s.y.Cp; cl.p.out2_pitch = s.y2.pitch; }
-    cl.p.res = s.has_res ? ptr_of(r, s.res) : nullptr;
-    cl.p.wpack = d.wpack; cl.p.bias = d.bias;
-    host.push_back(cl);
-    smem = std::max(smem, d.cp.smem_bytes);
-  }
-  ChainDev& c = r->chains[op_index];
-  c.n = static_cast<int>(host.size());
-  c.smem = smem;
-  XR_CUDA(cudaMalloc(&c.d_layers, host.size() * sizeof(ChainLayer)));
-  XR_CUDA(cudaMemcpy(c.d_layers, host.data(), host.size() * sizeof(ChainLayer), cudaMemcpyHostToDevice));
-}
-
 void upload_layers(xrseg_runner* r, const std::vector<HostLayerWeights>& hw) {
   Net& net = *r->net;
   r->dl.resize(net.layers.size());
-  r->chains.assign(net.ops.size(), ChainDev{});
   for (size_t oi = 0; oi < net.ops.size(); ++oi) {
     const Op& o = net.ops[oi];
-    if (o.kind == OP_CHAIN) { upload_chain(r, oi, o, hw); continue; }
     if (o.layer < 0) continue;
     const LayerRec& l = net.layers[o.layer];
     const HostLayerWeights& w = hw[o.layer];
@@ -305,21 +206,6 @@ void upload_layers(xrseg_runner* r, const std::vector<HostLayerWeights>& hw) {
       }
       d.w32 = dev_upload(ws);
       d.bias = dev_upload(bs);
-    } else if (o.kind == OP_C3K2) {
-      const int ids[4] = {o.layer, o.layer2, o.layer3, o.layer4};
-      const int c = net.layers[o.layer].cout / 2, cm = round_up(net.layers[o.layer2].cout, 8);
-      const int kdim[4] = {o.x.Cp, c, cm, 3 * c}, ndim[4] = {2 * c, cm, c, o.y.Cp}, taps[4] = {1, 9, 9, 1};
-      std::vector<float> bias;
-      for (int j = 0; j < 4; ++j) {
-        const LayerRec& lj = net.layers[ids[j]];
-        std::vector<uint32_t> f;
-        pack_bneck_weights(hw[ids[j]].w.data(), lj.cin, lj.cout, kdim[j], ndim[j], f, taps[j]);
-        r->dl[ids[j]].wfrag = reinterpret_cast<uint2*>(dev_upload(f));
-        std::vector<float> bj(ndim[j], 0.f);
-        std::copy(hw[ids[j]].b.begin(), hw[ids[j]].b.end(), bj.begin());
-        bias.insert(bias.end(), bj.begin(), bj.end());
-      }
-      d.bias = dev_upload(bias);
     } else if (o.kind == OP_BNECK) {
       const LayerRec& l2 = net.layers[o.layer2];
       const HostLayerWeights& w2 = hw[o.layer2];
@@ -370,34 +256,15 @@ void upload_layers(xrseg_runner* r, const std::vector<HostLayerWeights>& hw) {
       } else {
         d.cp = plan_conv(cd, r->num_sms, 0);
       }
-      if (d.use_tma) {
-        // TMA-store epilogue where the shape allows it (conv_tma.cuh: plan_tma_store); output maps m[4] (out) / m[5] (out2)
-        const int split_n = o.layer2 >= 0 ? o.y.Cp : 0;
-        const int mode = d.cp.mode;
-        const int nsm = r->num_sms;
-        if (plan_tma_store(d.cp, split_n, [&](ConvParams& q, int budget) {
-              return mode == MODE_HALO_TMA ? plan_conv_halo_tma(cd, nsm, q, true, budget)
-                     : mode == MODE_FLAT_TMA ? plan_conv_flat_tma(cd, nsm, q, budget) : plan_conv_s2_tma(cd, nsm, q, budget);
-            })) {
-          d.tmaps.m[4] = make_store_tensor_map(ptr_of(r, o.y), d.cp, r->mb, o.y.Cp, o.y.pitch);
-          if (o.layer2 >= 0) d.tmaps.m[5] = make_store_tensor_map(ptr_of(r, o.y2), d.cp, r->mb, o.y2.Cp, o.y2.pitch);
-        }
-      }
       if (o.tail_layer >= 0) {
         // fused trailing 1x1 (model.cuh: fuse_tail_1x1): W2 as the 128-byte-swizzled image of a 1x1 layer with Ntile = 32, cb = 64
         const LayerRec& lt = net.layers[o.tail_layer];
         const HostLayerWeights& wt = hw[o.tail_layer];
         const int N1 = d.cp.Ntile, N2 = o.ytail.Cp;
-        XR_CHECK(d.use_tma && (d.cp.mode == MODE_HALO_TMA || d.cp.mode == MODE_S2_TMA) && d.cp.sw && (N1 == 32 || N1 == 64) &&
-                     (N2 == 32 || N2 == 64) && d.cp.n_tiles == 1 && d.cp.b_resident && (d.cp.nbuf == 0 || d.cp.nbuf == 2) &&
-                     !d.cp.st_tma && lt.cin <= N1,
-                 "fused trailing 1x1 needs a halo / stride-2 TMA plan with Ntile 32 / 64, resident weights and two accumulator sets (%s)",
+        XR_CHECK(d.use_tma && d.cp.mode == MODE_HALO_TMA && d.cp.sw && N1 == 64 && N2 == 32 && d.cp.n_tiles == 1 && d.cp.b_resident &&
+                     d.cp.nbuf == 2 && lt.cin <= N1,
+                 "fused trailing 1x1 needs a halo TMA plan with Ntile 64, a 32-channel 1x1, resident weights and two accumulator sets (%s)",
                  l.name.c_str());
-        // TMEM: in place when the main accumulators fill all 512 columns (64 -> 32 only), else a region of its own behind them
-        const int main_cols = 2 * d.cp.nsub * N1, tail_cols = 2 * d.cp.nsub * N2;
-        const bool inplace = main_cols + tail_cols > 512;
-        XR_CHECK(!inplace || (N1 == 64 && N2 == 32), "no tensor-memory room for the fused 1x1 (%s: %d + %d columns)", l.name.c_str(),
-                 main_cols, tail_cols);
         ConvParams t{};
         t.Ntile = N2; t.n_tiles = 1; t.cb = N1; t.sw = N1 == 64 ? 3 : 2; t.taps = 1; t.nks = 1; t.kps = 1; t.b_stage_bytes = N2 * N1 * 2;
         t.Cout = N2;
@@ -408,15 +275,10 @@ void upload_layers(xrseg_runner* r, const std::vector<HostLayerWeights>& hw) {
         r->dl[o.tail_layer].tail_bias = dev_upload(bp2);
         d.cp.tail_n = N2;
         d.cp.tail_act = o.tail_act;
-        d.cp.tail_inplace = inplace ? 1 : 0;
-        if (!inplace) d.cp.tmem_cols = pow2_ceil(main_cols + tail_cols);
         d.cp.smem_off_w2 = round_up(d.cp.smem_bytes, 1024);
         d.cp.smem_bytes = d.cp.smem_off_w2 + N2 * N1 * 2;
         XR_CHECK(d.cp.smem_bytes <= CONV_SMEM_MAX, "no room for the tail's weights (%s)", l.name.c_str());
       }
-#ifdef XRSEG_DEBUG_API
-      if (const char* e = getenv("XRSEG_EPI")) d.cp.dbg_skip |= (e[0] == '1') ? 8 : 0;   // A/B of the TMA kernel's epilogue
-#endif
       if (r->cfg.conv_impl == XRSEG_CONV_UMMA) {
         std::vector<__half> wp;
         std::vector<float> bp;
@@ -487,12 +349,11 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
         mq.B = nb; mq.H = o.x.H; mq.W = o.x.W; mq.in_scale = 1.0f / 255.0f;
         const int nt = o.y.Cp / 8;
         const __half* w16_rows = r->dl[o.layer].w16_rows;
-        static const bool stem_rows_off = [] { const char* e = getenv("XRSEG_STEM_ROWS"); return e && e[0] == '0'; }();
         L.fn = [r, p, q, mq, nt, total, smem, smem_u8, nb, w16_rows](cudaStream_t st) {
           const bool aligned = (reinterpret_cast<uintptr_t>(r->fused_src) % 4 == 0) && (r->fused_stride % 4 == 0);
           const bool wide = (reinterpret_cast<uintptr_t>(r->fused_src) % 16 == 0) && (r->fused_stride % 16 == 0) &&
                             (mq.W * 3) % 16 == 0 && r->fused_bpp == 3;
-          if (r->fused_src && wide && !stem_rows_off && (nt == 2 || nt == 4) && r->cfg.conv_impl == XRSEG_CONV_UMMA) {
+          if (r->fused_src && wide && (nt == 2 || nt == 4) && r->cfg.conv_impl == XRSEG_CONV_UMMA) {
             StemMmaParams u = mq;                        // packed RGB rows: raw-byte staging (stem_rows_kernel)
             u.src = r->fused_src; u.stride_bytes = r->fused_stride; u.bpp = 3; u.w16 = w16_rows; u.flip = r->fused_flip;
             const dim3 grid(ceil_div(u.W / 2, STEM2_COLS), ceil_div(u.H / 2, STEM2_ROWS), nb);
@@ -531,30 +392,21 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
           ConvParams p = d.cp;
           if (nb != p.B) p = replan_for_batch(d.cp, nb, r->num_sms);   // partial last chunk: same layout, fewer frames
           {
-            // Small launches use at most HALF the SMs (XRSEG_TINY_GRID, 0 = off): 3x3 layers with at most two work items per SM
-            // (XRSEG_TINY_WORK = 296: every 20x20 layer, the 3x3 convs of the 40x40 stage) and 1x1 layers with at most
-            // XRSEG_TINY_FLAT_WORK = 800 items (the 40x40 stage).  These kernels are latency-bound -- most of their ~10 us is fill
+            // Small launches use at most HALF the SMs (XRSEG_TINY_GRID=0 turns it off): 3x3 layers with at most two work items
+            // per SM (296: every 20x20 layer, the 3x3 convs of the 40x40 stage) and 1x1 layers with at most 800 items (the 40x40
+            // stage).  These kernels are latency-bound -- most of their ~10 us is fill
             // and drain -- and a throughput caller keeps several runners in flight: with half-width grids the small kernels of
             // two steps sit side by side on disjoint SMs instead of taking turns on all of them.  Measured (B200, batch 64, four
             // runners, profiles/r2_experiments.md): 34.5k -> 36.7k frames/s, e2e 32.4k -> 34.0k; one runner alone 30.2k -> 29.9k;
             // batch-1 latency unchanged (its grids are smaller than the cap anyway).
-            static const int tiny_grid = [] { const char* e = getenv("XRSEG_TINY_GRID"); return e ? atoi(e) : -1; }();
-            static const int tiny_work = [] { const char* e = getenv("XRSEG_TINY_WORK"); return e ? atoi(e) : 296; }();
-            static const int tiny_flat = [] { const char* e = getenv("XRSEG_TINY_FLAT_WORK"); return e ? atoi(e) : 800; }();
-            // XRSEG_TINY_MMA_CYC (experiment switch, default off): keep tensor-heavy layers at full width -- few items say nothing
-            // about their size (b7: 256 items of 72 N = 256 MMAs each, 21 us of tensor time on half the SMs against 10.5 us on all
-            // of them; h5.box.0, n20, h4.box.1, n13.cv1, b9.cv2 likewise).  Value = largest tensor time (cycles) of the busiest CTA
-            // of a half-width launch.  Measured with 9000 (gpurun_out s18): those launches alone 43 -> 28, 30 -> 21, 27 -> 21,
-            // 27 -> 19, 37 -> 28, 24 -> 21 us and one runner alone 32.0k -> 32.5k frames/s, but four runners 39.1k -> 38.2k and
-            // e2e 35.9k -> 35.6k: side by side on disjoint SMs beats taking turns even for these.
-            static const long tiny_mma = [] { const char* e = getenv("XRSEG_TINY_MMA_CYC"); return e ? atol(e) : (1L << 60); }();
-            const int cap = tiny_grid < 0 ? r->num_sms / 2 : tiny_grid;
+            // Tensor-heavy layers stay at half width too: keeping them on all SMs (b7: 256 items of 72 N = 256 MMAs each, 21 us of
+            // tensor time on half the SMs against 10.5 us on all of them; h5.box.0, n20, h4.box.1, n13.cv1, b9.cv2 likewise) made
+            // those launches alone 43 -> 28, 30 -> 21, 27 -> 21, 27 -> 19, 37 -> 28, 24 -> 21 us and one runner alone 32.0k -> 32.5k
+            // frames/s, but four runners 39.1k -> 38.2k and e2e 35.9k -> 35.6k: side by side on disjoint SMs beats taking turns.
+            static const bool tiny_on = [] { const char* e = getenv("XRSEG_TINY_GRID"); return !(e && e[0] == '0'); }();
+            const int cap = r->num_sms / 2;
             const int work = p.m_tiles * p.n_tiles;
-            if (cap > 0 && d.use_tma && p.grid > cap && work <= (p.mode == MODE_FLAT_TMA ? tiny_flat : tiny_work)) {
-              const long mma_item = static_cast<long>(p.nks) * (p.kps > 1 ? p.kps : 1) * (p.taps > 0 ? p.taps : 1) * (p.cb / 16) * p.nsub *
-                                    (p.Ntile / 2 > 16 ? p.Ntile / 2 : 16);
-              if (ceil_div(work, cap) * mma_item <= tiny_mma) p.grid = cap;
-            }
+            if (tiny_on && d.use_tma && p.grid > cap && work <= (p.mode == MODE_FLAT_TMA ? 800 : 296)) p.grid = cap;
           }
           p.in = ptr_of(r, o.x); p.out = ptr_of(r, o.y);
           if (o.layer2 >= 0) { p.out2 = ptr_of(r, o.y2); p.split_n = o.y.Cp; p.out2_pitch = o.y2.pitch; }
@@ -586,64 +438,6 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
         }
         break;
       }
-      case OP_CHAIN: {
-        const ChainDev c = r->chains[oi];
-        const int num_sms = r->num_sms;
-        L.name = "chain:" + net.layers[o.chain.front().layer].name + ".." + net.layers[o.chain.back().layer].name;
-        if (L.name.size() > 31) L.name.resize(31);
-        for (const Op& s : o.chain) {               // algorithmic work: the sum over the chain's convolutions
-          const LayerRec& l = net.layers[s.layer];
-          const double pin = static_cast<double>(nb) * s.x.H * s.x.W, pout = static_cast<double>(nb) * s.y.H * s.y.W;
-          const int cout_alg = l.cout + (s.layer2 >= 0 ? net.layers[s.layer2].cout : 0);
-          L.flops += 2.0 * pout * cout_alg * l.cin * s.k * s.k;
-          L.bytes += (pin * l.cin + pout * cout_alg * (s.has_res ? 2 : 1) + static_cast<double>(cout_alg) * l.cin * s.k * s.k) * 2;
-        }
-#ifdef XRSEG_DEBUG_API
-        if (getenv("XRSEG_CHAIN_PROBE")) {
-          // per-layer phase clocks of CTA 0 (printed after a synchronous launch; timing experiments only)
-          std::vector<std::string> names;
-          for (const Op& s : o.chain) names.push_back(net.layers[s.layer].name);
-          L.fn = [c, nb, num_sms, names](cudaStream_t st) {
-            cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-            cudaStreamIsCapturing(st, &cs);
-            if (cs != cudaStreamCaptureStatusNone) { launch_conv_chain(c.d_layers, c.n, nb, c.smem, num_sms, st); return; }
-            long long* d = nullptr;
-            cudaMalloc(&d, sizeof(long long) * 8 * c.n);
-            cudaMemset(d, 0, sizeof(long long) * 8 * c.n);
-            launch_conv_chain(c.d_layers, c.n, nb, c.smem, num_sms, st, d);
-            cudaStreamSynchronize(st);
-            std::vector<long long> h(8 * c.n);
-            cudaMemcpy(h.data(), d, sizeof(long long) * h.size(), cudaMemcpyDeviceToHost);
-            cudaFree(d);
-            for (int l = 0; l < c.n; ++l) {
-              const long long* t = &h[8 * l];
-              const long long next = l + 1 < c.n ? h[8 * (l + 1)] : t[4];
-              // all relative to the moment MMA warp 1 has its weights (same SM sub-partition clock as the epilogue thread)
-              (void)next;
-              fprintf(stderr, "chain probe %-18s data +%5lld  mma-done +%5lld  prefetch-issued +%5lld  first-ld +%5lld  epi-done +%5lld  fenced +%5lld cycles\n",
-                      names[l].c_str(), t[1] - t[5], t[2] - t[1], t[6] - t[2], t[7] - t[6], t[3] - t[7], t[4] - t[3]);
-            }
-          };
-        } else
-#endif
-        L.fn = [c, nb, num_sms](cudaStream_t st) { launch_conv_chain(c.d_layers, c.n, nb, c.smem, num_sms, st); };
-        break;
-      }
-      case OP_C3K2: {
-        const LayerRec &l = net.layers[o.layer], &l2 = net.layers[o.layer2], &l3 = net.layers[o.layer3], &l4 = net.layers[o.layer4];
-        C3k2Params p{};
-        p.in = ptr_of(r, o.x); p.in_pitch = o.x.pitch; p.out = ptr_of(r, o.y); p.out_pitch = o.y.pitch;
-        p.w_cv1 = r->dl[o.layer].wfrag; p.w_m1 = r->dl[o.layer2].wfrag; p.w_m2 = r->dl[o.layer3].wfrag; p.w_cv2 = r->dl[o.layer4].wfrag;
-        p.bias = r->dl[o.layer].bias;
-        p.B = nb; p.H = o.x.H; p.W = o.x.W;
-        const int cin = o.x.Cp, c = l.cout / 2, cm = round_up(l2.cout, 8), cout = o.y.Cp;
-        const double macs = static_cast<double>(l.cin) * l.cout + 9.0 * (l2.cin * l2.cout + l3.cin * l3.cout) + static_cast<double>(l4.cin) * l4.cout;
-        L.name = l.name.substr(0, l.name.size() - 4);          // "b2"
-        L.flops = 2.0 * px_out * macs;
-        L.bytes = (px_in * l.cin + px_out * l4.cout + macs) * 2;
-        L.fn = [p, cin, c, cm, cout](cudaStream_t st) { launch_c3k2(cin, c, cm, cout, p, st); };
-        break;
-      }
       case OP_BNECK: {
         const LayerRec &l = net.layers[o.layer], &l2 = net.layers[o.layer2];
         BneckParams p{};
@@ -667,24 +461,11 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
         p.B = nb; p.H = o.x.H; p.W = o.x.W; p.C = o.y.Cp; p.act = o.act;
         p.in_grp = o.in_grp; p.in_grp_stride = o.in_grp_stride; p.in_grp_off = o.in_grp_off;
         p.rows = o.x.H >= 40 ? 16 : 10;
-        {
-          static const int dw_rows = [] { const char* e = getenv("XRSEG_DW_ROWS"); return e ? atoi(e) : 0; }();
-          if (dw_rows > 0) p.rows = dw_rows;
-        }
         L.name = l.name;
         L.flops = 2.0 * px_out * l.cout * 9;
         L.bytes = (px_in * l.cin + px_out * l.cout * (o.has_res ? 2 : 1)) * 2;
-        const bool narrow = !dw_wide();             // 8 channels per thread (default) or 4 (XRSEG_DW_NARROW=1)
-        const dim3 grid(ceil_div(p.W * (p.C / (narrow ? 4 : 8)), 128), ceil_div(p.H, p.rows), nb);
-        static const bool dw_smem = [] { const char* e = getenv("XRSEG_DW_SMEM"); return e && e[0] == '1'; }();   // opt-in: measured slower
-        const DwSmemGeom geo = dw_smem_geom(p.W, p.C);
-        if (dw_smem && p.C % 8 == 0 && geo.threads <= 192 && geo.smem_bytes <= 48 * 1024) {
-          const dim3 sgrid((p.C / 8) / geo.CG, ceil_div(p.H, geo.TR), nb);
-          L.fn = [p, sgrid, geo](cudaStream_t st) {
-            launch_k(dwconv3x3_smem_kernel, sgrid, geo.threads, static_cast<size_t>(geo.smem_bytes), st, p, geo.TR, geo.CG);
-          };
-        } else if (narrow) L.fn = [p, grid](cudaStream_t st) { launch_k(dwconv3x3_kernel<2>, grid, 128, 0, st, p); };
-        else L.fn = [p, grid](cudaStream_t st) { launch_k(dwconv3x3_kernel<4>, grid, 128, 0, st, p); };
+        const dim3 grid(ceil_div(p.W * (p.C / 8), 128), ceil_div(p.H, p.rows), nb);
+        L.fn = [p, grid](cudaStream_t st) { launch_k(dwconv3x3_kernel<4>, grid, 128, 0, st, p); };
         break;
       }
       case OP_SPPF: {
@@ -1188,7 +969,6 @@ xrseg_runner::~xrseg_runner() {
   for (cudaEvent_t e : ev_join) if (e) cudaEventDestroy(e);
   for (cudaEvent_t e : ev_copy) cudaEventDestroy(e);
   cudaFree(scratch);
-  for (ChainDev& c : chains) cudaFree(c.d_layers);
   for (DevLayer& d : dl) {
     cudaFree(d.wpack); cudaFree(d.wfrag); cudaFree(d.tail_w); cudaFree(d.tail_bias); cudaFree(d.w16_rows); cudaFree(d.bias); cudaFree(d.w16); cudaFree(d.w32); cudaFree(d.w32_u8);
   }
@@ -1362,26 +1142,16 @@ int xrseg_create(const xrseg_config* cfg_in, xrseg_runner** out) {
     r->device = c.device;
     r->num_sms = prop.multiProcessorCount;
     XR_CUDA(cudaSetDevice(c.device));
-    {
-      // XRSEG_PRIO=1: the main stream (the dependent chain backbone -> neck -> P5 head) above the side branches (head / prototype
-      // chains), so that its small launches are not queued behind the branches' big ones; captured kernel nodes inherit the
-      // priority of the stream they were captured on
-      static const bool prio = [] { const char* e = getenv("XRSEG_PRIO"); return e && e[0] == '1'; }();
-      int lo = 0, hi = 0;
-      XR_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));        // lo = lowest priority (largest number)
-      XR_CUDA(cudaStreamCreateWithPriority(&r->stream, cudaStreamNonBlocking, prio ? hi : 0));
-      XR_CUDA(cudaStreamCreateWithFlags(&r->copy_stream, cudaStreamNonBlocking));
-      for (auto& s : r->side) XR_CUDA(cudaStreamCreateWithPriority(&s, cudaStreamNonBlocking, prio ? lo : 0));
-    }
+    XR_CUDA(cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking));
+    XR_CUDA(cudaStreamCreateWithFlags(&r->copy_stream, cudaStreamNonBlocking));
+    for (auto& s : r->side) XR_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
     for (auto& e : r->ev_tag) XR_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     for (auto& e : r->ev_join) XR_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     XR_CUDA(cudaEventCreateWithFlags(&r->ev_done, cudaEventDisableTiming));
     for (auto& e : r->ev) XR_CUDA(cudaEventCreate(&e));
     conv_umma_prepare_device();
     conv_tma_prepare_device();
-    conv_chain_prepare_device();
     bneck_prepare_device();
-    c3k2_prepare_device();
     XR_CUDA(cudaFuncSetAttribute(attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
     XR_CUDA(cudaFuncSetAttribute(nms_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 8));
     XR_CUDA(cudaFuncSetAttribute((nms_reduce_kernel<1, 4>), cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * 32 * 64 * 8));
@@ -1391,17 +1161,8 @@ int xrseg_create(const xrseg_config* cfg_in, xrseg_runner** out) {
     const char* fuse_env = getenv("XRSEG_FUSE");
     const bool fuse = c.conv_impl == XRSEG_CONV_UMMA && !(fuse_env && fuse_env[0] == '0');
     const char* bneck_env = getenv("XRSEG_FUSE_BNECK");
-    // whole-block C3k2 kernel: parity-tested but measured slower than cv1 + fused Bottleneck + cv2 (DESIGN.md 4): opt-in
-    const char* c3k2_env = getenv("XRSEG_FUSE_C3K2");
-    r->net.reset(new Net(c.model_scale, r->mb, 640, fuse, !(bneck_env && bneck_env[0] == '0'), c3k2_env && c3k2_env[0] == '1'));
+    r->net.reset(new Net(c.model_scale, r->mb, 640, fuse, !(bneck_env && bneck_env[0] == '0')));
     Net& net = *r->net;
-    if (c.conv_impl == XRSEG_CONV_UMMA && !chains_disabled()) {
-      const int mb = r->mb;
-      net.fuse_chains([mb](const Op& o) {
-        ConvParams tmp;
-        return plan_chain_layer(conv_desc_of(o, mb), tmp);
-      });
-    }
     r->A = net.fh[0] * net.fw[0] + net.fh[1] * net.fw[1] + net.fh[2] * net.fw[2];
     std::vector<HostLayerWeights> hw;
     try {
@@ -2221,14 +1982,6 @@ int xrseg_debug_conv(int device, int impl, const float* x, int b, int cin, int h
       const bool s2 = !tma && !flat && variant == 0 && plan_conv_s2_tma(cd, prop.multiProcessorCount, p);
       tma = tma || flat || s2;
       if (!tma) p = plan_conv(cd, prop.multiProcessorCount, variant & 1);
-      bool st_tma = false;
-      if (tma && variant == 0) {
-        const int mode = p.mode, nsm = prop.multiProcessorCount;
-        st_tma = plan_tma_store(p, 0, [&](ConvParams& q, int budget) {
-          return mode == MODE_HALO_TMA ? plan_conv_halo_tma(cd, nsm, q, true, budget)
-                 : mode == MODE_FLAT_TMA ? plan_conv_flat_tma(cd, nsm, q, budget) : plan_conv_s2_tma(cd, nsm, q, budget);
-        });
-      }
       std::vector<__half> wp;
       std::vector<float> bp;
       if (tma && p.sw) pack_conv_weights_sw<__half>(p, wgt, hb, cin, cout, wp, bp);
@@ -2256,7 +2009,6 @@ int xrseg_debug_conv(int device, int impl, const float* x, int b, int cin, int h
           if (s2) maps = make_s2_tensor_maps(d_x, b, h, w, cin_p, cin_p, p);
           else maps.m[0] = flat ? make_flat_tensor_map(d_x, static_cast<long>(b) * h * w, cin_p, cin_p, p)
                                 : make_halo_tensor_map(d_x, b, h, w, cin_p, cin_p, p.Wp, p.hbox, p.sw ? p.cb : 8, p.sw);
-          if (st_tma) maps.m[4] = make_store_tensor_map(d_y, p, b, cout_p, cout_p);
           launch_conv_halo_tma(p, maps, 0);
         } else {
           launch_conv_umma(p, 0);
@@ -2267,8 +2019,8 @@ int xrseg_debug_conv(int device, int impl, const float* x, int b, int cin, int h
       if (reps > 1) {
         float ms = 0;
         cudaEventElapsedTime(&ms, e0, e1);
-        fprintf(stderr, "xrseg_debug_conv: mode %d sw %d cb %d S %d nks %d nsub %d R %d grid %d smem %d tiles %d st_tma %d skip %d: %.1f us\n", p.mode, p.sw, p.cb,
-                p.S, p.nks, p.nsub, p.R, p.grid, p.smem_bytes, p.m_tiles * p.n_tiles, p.st_tma, p.dbg_skip, ms * 1e3f);
+        fprintf(stderr, "xrseg_debug_conv: mode %d sw %d cb %d S %d nks %d nsub %d R %d grid %d smem %d tiles %d skip %d: %.1f us\n", p.mode, p.sw, p.cb,
+                p.S, p.nks, p.nsub, p.R, p.grid, p.smem_bytes, p.m_tiles * p.n_tiles, p.dbg_skip, ms * 1e3f);
         if (d_clk) {
           std::vector<long long> h(static_cast<size_t>(p.grid) * 12);
           XR_CUDA(cudaMemcpy(h.data(), d_clk, sizeof(long long) * h.size(), cudaMemcpyDeviceToHost));
@@ -2389,81 +2141,7 @@ int xrseg_debug_bottleneck(int device, const float* x, int b, int c1, int h, int
   return XRSEG_OK;
 }
 
-// The whole-block C3k2 kernel on caller tensors (test hook): ab = silu(cv1 x), m = b + silu(m2 silu(m1 b)), y = silu(cv2 [a|b|m]).
-// x [b,cin,h,w]; w_cv1 [2c,cin], w_m1 [cm,c,3,3], w_m2 [c,cm,3,3], w_cv2 [cout,3c]; y [b,cout,h,w]; fp32 NCHW on the host.
-int xrseg_debug_c3k2(int device, const float* x, int b, int cin, int h, int w, int c, int cm, int cout, const float* w_cv1,
-                     const float* b_cv1, const float* w_m1, const float* b_m1, const float* w_m2, const float* b_m2,
-                     const float* w_cv2, const float* b_cv2, float* y) {
-  if (!x || !w_cv1 || !b_cv1 || !w_m1 || !b_m1 || !w_m2 || !b_m2 || !w_cv2 || !b_cv2 || !y) return XRSEG_ERR_INVALID;
-  try {
-    XR_CUDA(cudaSetDevice(device));
-    cudaDeviceProp prop{};
-    XR_CUDA(cudaGetDeviceProperties(&prop, device));
-    if (prop.major != 10) { g_create_error = "not an sm_100 device"; return XRSEG_ERR_NO_DEVICE; }
-    if (!c3k2_supported(cin, c, cm, cout)) { g_create_error = "unsupported channel counts"; return XRSEG_ERR_INVALID; }
-    c3k2_prepare_device();
-    const size_t nx = static_cast<size_t>(b) * cin * h * w, ny = static_cast<size_t>(b) * cout * h * w;
-    float* d_x32 = dev_alloc<float>(nx);
-    float* d_y32 = dev_alloc<float>(ny);
-    __half* d_x = dev_alloc<__half>(static_cast<size_t>(b) * h * w * cin);
-    __half* d_y = dev_alloc<__half>(static_cast<size_t>(b) * h * w * cout);
-    XR_CUDA(cudaMemcpy(d_x32, x, nx * sizeof(float), cudaMemcpyHostToDevice));
-    nchw_f32_to_nhwc_f16_kernel<<<grid_for(static_cast<long>(b) * h * w * cin), 256>>>(d_x32, d_x, b, cin, h, w, cin, cin);
-    XR_CUDA(cudaMemset(d_y, 0, static_cast<size_t>(b) * h * w * cout * sizeof(__half)));
-    const float* ws[4] = {w_cv1, w_m1, w_m2, w_cv2};
-    const float* bs[4] = {b_cv1, b_m1, b_m2, b_cv2};
-    const int kin[4] = {cin, c, cm, 3 * c}, nout[4] = {2 * c, cm, c, cout}, taps[4] = {1, 9, 9, 1};
-    uint32_t* d_f[4];
-    std::vector<float> bias;
-    for (int j = 0; j < 4; ++j) {
-      std::vector<uint32_t> f;
-      pack_bneck_weights(ws[j], kin[j], nout[j], kin[j], nout[j], f, taps[j]);
-      d_f[j] = dev_upload(f);
-      bias.insert(bias.end(), bs[j], bs[j] + nout[j]);
-    }
-    float* d_b = dev_upload(bias);
-    C3k2Params p{};
-    p.in = d_x; p.in_pitch = cin; p.out = d_y; p.out_pitch = cout;
-    p.w_cv1 = reinterpret_cast<uint2*>(d_f[0]); p.w_m1 = reinterpret_cast<uint2*>(d_f[1]);
-    p.w_m2 = reinterpret_cast<uint2*>(d_f[2]); p.w_cv2 = reinterpret_cast<uint2*>(d_f[3]);
-    p.bias = d_b; p.B = b; p.H = h; p.W = w;
-    const int reps = getenv("XRSEG_DBG_TIME") ? 5 : 1;
-    cudaEvent_t e0, e1;
-    XR_CUDA(cudaEventCreate(&e0));
-    XR_CUDA(cudaEventCreate(&e1));
-    for (int rep = 0; rep < reps; ++rep) {
-      if (rep == reps - 1) XR_CUDA(cudaEventRecord(e0, 0));
-      launch_c3k2(cin, c, cm, cout, p, 0);
-    }
-    XR_CUDA(cudaEventRecord(e1, 0));
-    XR_CUDA(cudaEventSynchronize(e1));
-    XR_CUDA(cudaGetLastError());
-    if (reps > 1) {
-      float ms = 0;
-      cudaEventElapsedTime(&ms, e0, e1);
-      fprintf(stderr, "xrseg_debug_c3k2: %d-%d-%d-%d %dx%d batch %d: %.1f us\n", cin, c, cm, cout, h, w, b, ms * 1e3f);
-    }
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    nhwc_f16_to_nchw_f32_kernel<<<grid_for(static_cast<long>(ny)), 256>>>(d_y, d_y32, b, cout, h, w, cout);
-    XR_CUDA(cudaDeviceSynchronize());
-    XR_CUDA(cudaMemcpy(y, d_y32, ny * sizeof(float), cudaMemcpyDeviceToHost));
-    cudaFree(d_x32); cudaFree(d_y32); cudaFree(d_x); cudaFree(d_y); cudaFree(d_b);
-    for (auto f : d_f) cudaFree(f);
-  } catch (const CudaError& e) {
-    g_create_error = e.msg;
-    return XRSEG_ERR_CUDA;
-  } catch (const std::exception& e) {   // nothing may unwind across the C boundary
-    g_create_error = std::string("unexpected exception: ") + e.what();
-    return XRSEG_ERR_CUDA;
-  } catch (...) {
-    g_create_error = "unknown exception";
-    return XRSEG_ERR_CUDA;
-  }
-  return XRSEG_OK;
-}
-
-// Host-only: the B-fragment weight packing of the fused Bottleneck / C3k2 kernels (bottleneck.cuh), for CPU tests of the
+// Host-only: the B-fragment weight packing of the fused Bottleneck kernel (bottleneck.cuh), for CPU tests of the
 // layout.  w [cout][cin][taps] fp32; out receives ceil(taps*C/16) * (N/8) * 64 words; returns the word count or < 0.
 int xrseg_debug_pack_bneck(const float* w, int cin, int cout, int C, int N, int taps, uint32_t* out, size_t cap_words) {
   if (!w || !out || cin < 1 || cout < 1 || C < cin || C % 8 || N < cout || N % 8 || (taps != 1 && taps != 9)) return XRSEG_ERR_INVALID;

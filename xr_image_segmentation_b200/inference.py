@@ -414,18 +414,6 @@ def debug_bottleneck(x, w1, b1, w2, b2, residual=True, device=0):
     return y
 
 
-def debug_c3k2(x, w_cv1, b_cv1, w_m1, b_m1, w_m2, b_m2, w_cv2, b_cv2, device=0):
-    """The whole-block C3k2 kernel (cv1 -> Bottleneck -> cv2 in one launch) on caller tensors (parity tests)."""
-    lib = _lib.load_library(True)
-    arrs = [np.ascontiguousarray(a, np.float32) for a in (x, w_cv1, b_cv1, w_m1, b_m1, w_m2, b_m2, w_cv2, b_cv2)]
-    B, cin, h, wd = arrs[0].shape
-    c, cm, cout = arrs[1].shape[0] // 2, arrs[3].shape[0], arrs[7].shape[0]
-    y = np.zeros((B, cout, h, wd), np.float32)
-    _lib.check(lib.xrseg_debug_c3k2(device, arrs[0].ctypes.data, B, cin, h, wd, c, cm, cout,
-                                    *[a.ctypes.data for a in arrs[1:]], y.ctypes.data), None, lib)
-    return y
-
-
 def debug_attention(qkv, heads, device=0, pe_w=None, pe_b=None, map_w=0):
     """The C2PSA attention kernel alone: qkv f32 [B,N,heads*128] (per head 32 q | 32 k | 64 v) -> [B,N,heads*64].
     pe_w [heads*64,3,3] / pe_b [heads*64] / map_w: the fused positional encoding (depthwise 3x3 on the V map) is added."""
