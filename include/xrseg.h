@@ -89,7 +89,9 @@ typedef struct xrseg_config {
   int32_t conv_impl;           /* xrseg_conv_impl */
   int32_t use_cuda_graph;      /* 1 = replay the captured pipeline (default 1) */
   int32_t micro_batch;         /* frames pushed through the network per pass, 0 -> auto */
-  int32_t reserved[8];
+  int32_t num_classes;         /* classes of the model (1..1024): 0 -> taken from the weights; any other value must equal
+                                  the weights' count, else xrseg_create fails with XRSEG_ERR_WEIGHTS */
+  int32_t reserved[7];
 } xrseg_config;
 
 /* Borrowed view of an output tensor: valid until the next xrseg_schedule (↔ Worker.PeekOutput, IEE:426). */
@@ -218,6 +220,16 @@ typedef struct xrseg_layer_info {
 } xrseg_layer_info;
 int xrseg_layer_count(int model_scale);
 int xrseg_layer_info_get(int model_scale, int index, xrseg_layer_info* info);
+/* The same for a model trained on num_classes classes (1..1024): the class branch is max(ch[2], min(num_classes, 100))
+ * wide and the three *.cls.2 convolutions have num_classes outputs; names and order do not change.  The two functions
+ * above are the num_classes = 80 case. */
+int xrseg_layer_count_nc(int model_scale, int num_classes);
+int xrseg_layer_info_get_nc(int model_scale, int num_classes, int index, xrseg_layer_info* info);
+/* Scale ('n' / 's', from the width of the first convolution) and class count (from the three *.cls.2 convolutions, which
+ * must agree and lie in 1..1024) of a weight pack or .sentis asset; host only.  XRSEG_ERR_WEIGHTS otherwise. */
+int xrseg_weights_info(const void* data, size_t bytes, int32_t* model_scale, int32_t* num_classes);
+/* Class count of a runner's model. */
+int xrseg_num_classes(const xrseg_runner* r);
 
 /* ---- .sentis asset introspection (↔ ModelLoader.Load, IEE:382; host only, no GPU needed) --------- */
 /* Number of biased convolutions in the asset and the thresholds baked into its NonMaxSuppression layer

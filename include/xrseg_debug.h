@@ -18,7 +18,8 @@ extern "C" {
  * names: "p3","p4","p5","box_logits","cls_logits","coefs","protos","input" and every layer name. */
 int xrseg_debug_fetch(xrseg_runner* r, const char* name, float* dst, size_t cap_floats, int64_t* shape4);
 /* Run ONLY the post-processing stage on caller-provided fp32 head tensors (the oracle's own tensors):
- * box_logits [batch,A,64], cls_logits [batch,A,80], coefs [batch,A,32], protos [batch,32,160*160]. */
+ * box_logits [batch,A,64], cls_logits [batch,A,nc] (nc = the runner's xrseg_num_classes), coefs [batch,A,32],
+ * protos [batch,32,160*160]. */
 int xrseg_debug_post(xrseg_runner* r, const float* box_logits, const float* cls_logits, const float* coefs,
                      const float* protos, int batch);
 /* Same tensors through the PRODUCT kernels: rounded to fp16 on the device (prototypes re-laid out NHWC like the network's),

@@ -24,7 +24,8 @@ public class IEExecutorNative : MonoBehaviour
         public IntPtr weights; public UIntPtr weightsBytes;
         public float iouThreshold, scoreThreshold, maskThreshold;
         public int maxDet, maxCandidates, resizeMode, convImpl, useCudaGraph, microBatch;
-        [MarshalAs(UnmanagedType.ByValArray, SizeConst = 8)] public int[] reserved;
+        public int numClasses;   // 0 = from the model; a custom-trained YOLO11-seg may have 1..1024 classes
+        [MarshalAs(UnmanagedType.ByValArray, SizeConst = 7)] public int[] reserved;
     }
     [StructLayout(LayoutKind.Sequential)]
     struct NativeBox { public float centerX, centerY, width, height; public int labelId, frame; }
@@ -69,7 +70,7 @@ public class IEExecutorNative : MonoBehaviour
         {
             structSize = (uint)Marshal.SizeOf<Config>(), device = 0, maxBatch = 1, modelScale = 'n',
             weights = _modelPin.AddrOfPinnedObject(), weightsBytes = (UIntPtr)model.Length,
-            maskThreshold = _confidenceThreshold, useCudaGraph = 1, reserved = new int[8]   // iou / score 0 = the asset's own 0.43 / 0.301
+            maskThreshold = _confidenceThreshold, useCudaGraph = 1, reserved = new int[7]   // iou / score 0 = the asset's own 0.43 / 0.301
         };
         if (xrseg_create(ref cfg, out _runner) < 0)
         {

@@ -1,6 +1,6 @@
 // Host-only developer tool: prints the launch plan of every convolution of the network (no GPU needed).
 //   nvcc -std=c++17 -gencode arch=compute_100a,code=sm_100a --expt-relaxed-constexpr -o /tmp/plan_dump tools/plan_dump.cu -lcuda
-//   /tmp/plan_dump [batch] [n|s]
+//   /tmp/plan_dump [batch] [n|s] [ops] [num_classes]
 #include <math.h>
 #include "../xr_image_segmentation_b200/csrc/conv_tma.cuh"
 #include "../xr_image_segmentation_b200/csrc/model.cuh"
@@ -8,8 +8,14 @@ using namespace xrseg;
 int main(int argc, char** argv) {
   const int B = argc > 1 ? atoi(argv[1]) : 64;
   const int scale = argc > 2 ? argv[2][0] : 'n';
-  if (argc > 3 && argv[3][0] == 'o') {   // "ops": the fused launch list (one line per network launch) instead of the conv plans
-    Net fused(scale, B, 640, true, true);
+  bool ops = false;
+  int nc = 80;
+  for (int i = 3; i < argc; ++i) {
+    if (argv[i][0] == 'o') ops = true;
+    else nc = atoi(argv[i]);
+  }
+  if (ops) {   // "ops": the fused launch list (one line per network launch) instead of the conv plans
+    Net fused(scale, B, 640, true, true, nc);
     const char* kind_name[] = {"stem", "conv", "dw", "sppf", "up", "attn", "bneck"};
     for (const Op& o : fused.ops) {
       std::string name = o.layer >= 0 ? fused.layers[o.layer].name : std::string("-");
@@ -19,7 +25,7 @@ int main(int argc, char** argv) {
     }
     return 0;
   }
-  Net net(scale, B, 640, true, false);   // Bottleneck fusion off: every convolution keeps its own plan
+  Net net(scale, B, 640, true, false, nc);   // Bottleneck fusion off: every convolution keeps its own plan
   const char* mode_name[] = {"gather", "halo", "halo_tma", "flat_tma", "s2_tma"};
   long total_smem_small = 0;
   for (const Op& o : net.ops) {

@@ -32,7 +32,8 @@ class Config(C.Structure):
         ("weights", C.c_void_p), ("weights_bytes", C.c_size_t),
         ("iou_threshold", C.c_float), ("score_threshold", C.c_float), ("mask_threshold", C.c_float),
         ("max_det", C.c_int32), ("max_candidates", C.c_int32), ("resize_mode", C.c_int32), ("conv_impl", C.c_int32),
-        ("use_cuda_graph", C.c_int32), ("micro_batch", C.c_int32), ("reserved", C.c_int32 * 8),
+        ("use_cuda_graph", C.c_int32), ("micro_batch", C.c_int32), ("num_classes", C.c_int32),
+        ("reserved", C.c_int32 * 7),
     ]
 
 
@@ -86,6 +87,10 @@ PRODUCT_SIGNATURES = {
     "xrseg_keep_indices": (C.c_int, [C.c_void_p, _P(C.c_int32), _P(C.c_float), C.c_int]),
     "xrseg_layer_count": (C.c_int, [C.c_int]),
     "xrseg_layer_info_get": (C.c_int, [C.c_int, C.c_int, _P(LayerInfo)]),
+    "xrseg_layer_count_nc": (C.c_int, [C.c_int, C.c_int]),
+    "xrseg_layer_info_get_nc": (C.c_int, [C.c_int, C.c_int, C.c_int, _P(LayerInfo)]),
+    "xrseg_weights_info": (C.c_int, [C.c_void_p, C.c_size_t, _P(C.c_int32), _P(C.c_int32)]),
+    "xrseg_num_classes": (C.c_int, [C.c_void_p]),
     "xrseg_last_timings": (C.c_int, [C.c_void_p, _P(C.c_float), C.c_int]),
     "xrseg_launch_count": (C.c_int, [C.c_void_p]),
     "xrseg_event_record": (C.c_int, [C.c_void_p, C.c_int]),

@@ -433,6 +433,17 @@ static inline TmapSet make_s2_tensor_maps(const __half* base, int B, int H, int 
   return t;
 }
 
+// N tiles of a flat-mode plan: one tile up to 256 columns, else two or four equal tiles of a multiple of 16 columns (the kernel
+// decodes work items for 1, 2 or 4 N tiles).  The class convolution's output pitch is padded to such a width (model.cuh
+// class_pitch) so that every class count gets a plan; every other layer is <= 256, 512 or 1024 columns wide.
+static inline bool tma_n_split(int ncols, int& Ntile, int& n_tiles) {
+  for (n_tiles = 1; n_tiles <= 4; n_tiles *= 2) {
+    Ntile = ncols / n_tiles;
+    if (ncols % n_tiles == 0 && Ntile <= 256 && (n_tiles == 1 || Ntile % 16 == 0)) return true;
+  }
+  return false;
+}
+
 // 1x1 stride-1 convolution = plain GEMM over the flattened [B*H*W, C] activation matrix ("flat" mode of the same
 // kernel): a work item is 128*nsub consecutive pixels, its A operand ONE (or two) 2-D TMA boxes of cb channels x <= 256
 // rows per K-block, swizzled like the halo boxes; taps = 1.  One mbarrier arrival per stage instead of one per producer
@@ -450,9 +461,7 @@ static inline bool plan_conv_flat_tma_impl(const ConvDesc& d, int num_sms, ConvP
   p.k = d.k; p.stride = d.stride; p.pad = 0; p.act = d.act; p.transposed = convt ? 1 : 0;
   p.Ho = convt ? 2 * d.H : d.H; p.Wo = convt ? 2 * d.W : d.W;
   const int ncols = convt ? 4 * d.Cout : d.Cout;
-  p.Ntile = ncols <= 256 ? ncols : 256;
-  if (ncols % p.Ntile) return false;
-  p.n_tiles = ncols / p.Ntile;
+  if (!tma_n_split(ncols, p.Ntile, p.n_tiles)) return false;
   if (!convt) tma_apply_split(p, ncols);
   p.idesc = umma_idesc_f16(p.Ntile, 0);
   p.mode = MODE_FLAT_TMA;
@@ -471,6 +480,9 @@ static inline bool plan_conv_flat_tma_impl(const ConvDesc& d, int num_sms, ConvP
   p.b_resident = (p.n_tiles == 1 && total_b <= 98304) ? 1 : 0;
   const int resident = p.b_resident ? static_cast<int>(total_b) : 0;
   const int tiles128 = ceil_div(p.flat_rows, 128);
+  // the kernel keeps the bias of all N tiles at [256, 256 + 4 * ncols) of the header: more than the standard header's 512
+  // entries only for the class convolution of a model with more than 512 classes
+  const int hdr = round_up(256 + 4 * ncols > CONV_HDR_BYTES ? 256 + 4 * ncols : static_cast<int>(CONV_HDR_BYTES), 1024);
   int nsub = 256 / p.Ntile;
   if (nsub > 4) nsub = 4;
   if (nsub == 3) nsub = 2;                         // an item is one or two FULL boxes of <= 256 rows: power-of-two sub-tiles only
@@ -489,7 +501,7 @@ static inline bool plan_conv_flat_tma_impl(const ConvDesc& d, int num_sms, ConvP
       p.nks = nkb / kps;
       p.a_stage_bytes = kps * p.slots * rb;          // multiple of 1024 for every cb
       p.b_stage_bytes = kps * b_block;
-      const int fixed = round_up(CONV_HDR_BYTES, 1024) + (p.b_resident ? round_up(resident, 1024) : 0);
+      const int fixed = hdr + (p.b_resident ? round_up(resident, 1024) : 0);
       S = (CONV_SMEM_MAX - fixed) / (p.a_stage_bytes + (p.b_resident ? 0 : round_up(p.b_stage_bytes, 1024)));
       if (S > CONV_MAX_STAGES) S = CONV_MAX_STAGES;
       if (S >= 2) break;                             // streamed weights of a wide layer: fewer K-blocks per stage
@@ -505,7 +517,7 @@ static inline bool plan_conv_flat_tma_impl(const ConvDesc& d, int num_sms, ConvP
   p.lbo_a = p.a_stage_bytes;
   p.M_total = ceil_div(p.flat_rows, p.slots);
   p.m_tiles = p.M_total;
-  p.smem_off_b = round_up(CONV_HDR_BYTES, 1024);
+  p.smem_off_b = hdr;
   const int b_region = p.b_resident ? resident : p.S * round_up(p.b_stage_bytes, 1024);
   p.smem_off_a = p.smem_off_b + round_up(b_region, 1024);
   p.smem_bytes = p.smem_off_a + p.S * p.a_stage_bytes;

@@ -61,16 +61,31 @@ struct Spec {
   int ch[5];
   int mid0, mid1;     // C3k2 output widths of layers 2 / 4 (n: 64 / 128)
   int cls_mid, box_mid, coef_mid, proto_mid, heads;
+  int nc;             // classes: outputs of the three cls.2 convolutions
 };
 
-static inline Spec make_spec(int scale) {
+constexpr int NC_MIN = 1, NC_MAX = 1024;   // supported class counts (csrc/post.cuh sizes its decode paths for them)
+
+// Channel pitch of the class-logit tensors: whole N tiles of the 1x1 convolution's TMA plan (conv_tma.cuh tma_n_split), so
+// that every class count gets one.  round_up(nc, 16) up to 256 classes (one tile; 80 stays 80), else two or four equal
+// tiles of a multiple of 16 channels (365 -> 2 x 192, 601 -> 4 x 160, 1024 -> 4 x 256).  The extra channels get zero
+// weights and bias; the decode never reads past nc.
+static inline int class_pitch(int nc) {
+  int nt = 1;
+  while (round_up(ceil_div(nc, nt), 16) > 256) nt *= 2;
+  return nt * round_up(ceil_div(nc, nt), 16);
+}
+
+static inline Spec make_spec(int scale, int nc = 80) {
   const int wnum = (scale == 's') ? 2 : 1;  // width = wnum / 4
   Spec s;
   const int base[5] = {64, 128, 256, 512, 1024};
   for (int i = 0; i < 5; ++i) s.ch[i] = base[i] * wnum / 4;
   s.mid0 = 256 * wnum / 4;
   s.mid1 = 512 * wnum / 4;
-  s.cls_mid = s.ch[2] > 80 ? s.ch[2] : 80;
+  s.nc = nc;
+  const int cls_floor = nc < 100 ? nc : 100;    // Ultralytics: c3 = max(ch[0], min(nc, 100))
+  s.cls_mid = s.ch[2] > cls_floor ? s.ch[2] : cls_floor;
   s.box_mid = 64;
   if (s.ch[2] / 4 > s.box_mid) s.box_mid = s.ch[2] / 4;
   s.coef_mid = s.ch[2] / 4 > 32 ? s.ch[2] / 4 : 32;
@@ -96,8 +111,11 @@ class Net {
   TV box[3], cls[3], coef[3], protos;
   int fh[3], fw[3];
 
-  Net(int scale, int batch, int in_hw = 640, bool fuse = true, bool bneck = true)
-      : B(batch), sp(make_spec(scale)), fuse_enabled(fuse), fuse_bneck(fuse && bneck), fuse_tail(fuse) { build(in_hw); }
+  Net(int scale, int batch, int in_hw = 640, bool fuse = true, bool bneck = true, int nc = 80)
+      : B(batch), sp(make_spec(scale, nc)), fuse_enabled(fuse), fuse_bneck(fuse && bneck), fuse_tail(fuse) {
+    XR_CHECK(nc >= NC_MIN && nc <= NC_MAX, "%d classes: supported are %d..%d", nc, NC_MIN, NC_MAX);
+    build(in_hw);
+  }
 
   TV alloc(int H, int W, int C, int pitch_override = 0) {
     TV t;
@@ -190,7 +208,8 @@ class Net {
     t = conv(t, sp.cls_mid, 1, 1, true, n + ".cls.0pw");
     t = dw(t, true, n + ".cls.1dw");
     t = conv(t, sp.cls_mid, 1, 1, true, n + ".cls.1pw");
-    cls[i] = conv(t, 80, 1, 1, false, n + ".cls.2");
+    TV logits = alloc(t.H, t.W, sp.nc, class_pitch(sp.nc));
+    cls[i] = conv(t, sp.nc, 1, 1, false, n + ".cls.2", &logits);
     cur_branch = 0;
   }
   void head_coef(const TV& p, int i, const std::string& n) {

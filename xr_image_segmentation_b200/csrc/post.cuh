@@ -14,7 +14,7 @@
 namespace xrseg {
 
 constexpr int NUM_ANCHORS_MAX = 8400;
-constexpr int NC = 80;
+constexpr int NC = 80;            // the COCO class count: decode_filter_kernel is specialised for it
 constexpr int NM = 32;
 constexpr int PROTO_HW = 160;
 constexpr int PROTO_PIX = PROTO_HW * PROTO_HW;
@@ -33,6 +33,7 @@ template <typename T>
 struct DecodeParams {
   ScaleSrc<T> s[3];
   int B, A;
+  int nc;                    // classes; class tensors carry cls_pitch >= nc channels per anchor, the rest is never counted
   float score_thr;
   float logit_floor;         // anchors whose largest class logit is <= this cannot reach score_thr
   float* boxes;              // [B,A,4] cx,cy,w,h  (rows of candidates only; the rest is never read)
@@ -153,13 +154,170 @@ __global__ void __launch_bounds__(256) decode_filter_kernel(const DecodeParams<T
   if (static_cast<int>(threadIdx.x) < n) p.filt_list[static_cast<long>(b) * p.A + s_base + threadIdx.x] = s_list[threadIdx.x];
 }
 
+// Largest of the first `valid` logits of a 16-byte chunk (all of them when valid >= the chunk's element count).
+template <typename T>
+__device__ __forceinline__ float chunk_max(const uint4 raw, int valid) {
+  constexpr int EPC = 16 / static_cast<int>(sizeof(T));
+  if (valid >= EPC) {
+    if (sizeof(T) == 2) {
+      const __half2* h = reinterpret_cast<const __half2*>(&raw);
+      const __half2 m2 = __hmax2(__hmax2(h[0], h[1]), __hmax2(h[2], h[3]));
+      return fmaxf(__low2float(m2), __high2float(m2));
+    }
+    const float* f = reinterpret_cast<const float*>(&raw);
+    return fmaxf(fmaxf(f[0], f[1]), fmaxf(f[2], f[3]));
+  }
+  const T* e = reinterpret_cast<const T*>(&raw);
+  float m = -3.0e38f;
+#pragma unroll
+  for (int k = 0; k < EPC; ++k)
+    if (k < valid) m = fmaxf(m, ldf(e + k));
+  return m;
+}
+
+// Per-thread walk over one anchor's nc logits (a warp whose 32 anchors straddle two scales).
+template <typename T>
+__device__ __forceinline__ float anchor_max_walk(const DecodeParams<T>& p, int b, int a) {
+  int sa = 0;
+  if (a >= p.s[1].a_off) sa = 1;
+  if (a >= p.s[2].a_off) sa = 2;
+  const ScaleSrc<T>& s = p.s[sa];
+  const T* cl = s.cls + b * s.cls_bstride + static_cast<long>(a - s.a_off) * s.cls_pitch;
+  float m = -3.0e38f;
+  for (int c = 0; c < p.nc; ++c) m = fmaxf(m, ldf(cl + c));
+  return m;
+}
+
+// Appends the block's survivors to the frame's list (one global atomic per block).
+__device__ __forceinline__ void filter_append(int* s_list, int& s_n, int& s_base, int* filt_count, int* filt_list, int A, int b) {
+  __syncthreads();
+  const int n = s_n;
+  if (n == 0) return;
+  if (threadIdx.x == 0) s_base = atomicAdd(&filt_count[b], n);
+  __syncthreads();
+  if (static_cast<int>(threadIdx.x) < n) filt_list[static_cast<long>(b) * A + s_base + threadIdx.x] = s_list[threadIdx.x];
+}
+
+// Any other class count, rows of at most 32 chunks (cls_pitch <= 256 fp16 / 128 fp32 channels): the same warp-coalesced run
+// as decode_filter_kernel with the chunks per anchor (cpa = cls_pitch / chunk) read at run time -- chunk gi of the run is
+// chunk gi % cpa of anchor gi / cpa -- and a segment table of 32 * cpa entries per warp in dynamic shared memory.  Only
+// channels < nc count: the padding channels of the class tensor hold logit 0 (probability 0.5, above the 0.301 threshold),
+// and chunks holding nothing but padding are not read.  cls_pitch is a multiple of the chunk (host-checked).
+template <typename T>
+__global__ void __launch_bounds__(256) decode_filter_nc_kernel(const DecodeParams<T> p) {
+  XR_PDL_ENTRY();
+  constexpr int EPC = 16 / static_cast<int>(sizeof(T));
+  extern __shared__ float s_seg[];                                // [8 warps][32 * cpa]
+  __shared__ int s_list[256];
+  __shared__ int s_n, s_base;
+  const int b = blockIdx.y;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (threadIdx.x == 0) s_n = 0;
+  __syncthreads();
+  const int a0 = blockIdx.x * 256 + warp * 32;
+  const int a = a0 + lane;
+  if (a0 < p.A) {
+    const int a_last = min(a0 + 31, p.A - 1);
+    int si = 0;
+    if (a0 >= p.s[1].a_off) si = 1;
+    if (a0 >= p.s[2].a_off) si = 2;
+    int sl = 0;
+    if (a_last >= p.s[1].a_off) sl = 1;
+    if (a_last >= p.s[2].a_off) sl = 2;
+    float lmax = -3.0e38f;
+    if (si == sl) {
+      const ScaleSrc<T>& s = p.s[si];
+      const int cpa = s.cls_pitch / EPC;
+      const int used = (p.nc + EPC - 1) / EPC;                    // chunks holding at least one class
+      const uint4* run = reinterpret_cast<const uint4*>(s.cls + b * s.cls_bstride + static_cast<long>(a0 - s.a_off) * s.cls_pitch);
+      const int n_chunks = (a_last - a0 + 1) * cpa;
+      float* seg = s_seg + warp * 32 * cpa;
+      for (int gi = lane; gi < n_chunks; gi += 32) {
+        const int j = gi / cpa, c = gi - j * cpa;
+        seg[gi] = c < used ? chunk_max<T>(run[gi], p.nc - c * EPC) : -3.0e38f;
+      }
+      __syncwarp();
+      if (a <= a_last)
+        for (int k = 0; k < cpa; ++k) lmax = fmaxf(lmax, seg[lane * cpa + k]);
+    } else if (a < p.A) {
+      lmax = anchor_max_walk(p, b, a);
+    }
+    if (a < p.A && lmax > p.logit_floor) s_list[atomicAdd(&s_n, 1)] = a;
+  }
+  filter_append(s_list, s_n, s_base, p.filt_count, p.filt_list, p.A, b);
+}
+
+// Wide rows (more than 32 chunks: over 256 fp16 classes), where 32 anchors' segment table no longer fits shared memory: a
+// warp reads its 32 anchors one row at a time (row j: lane l reads chunks l, l + 32, ... -- one contiguous, coalesced row),
+// keeps a per-lane partial maximum per anchor, and a butterfly reduce-scatter (31 shuffles for 32 anchors) leaves anchor
+// a0 + l's maximum in lane l.  Rows hold at most 1024 channels (the host checks cls_pitch against it).
+template <typename T>
+__global__ void __launch_bounds__(256) decode_filter_wide_kernel(const DecodeParams<T> p) {
+  XR_PDL_ENTRY();
+  constexpr int EPC = 16 / static_cast<int>(sizeof(T));
+  constexpr int ROW_ITERS = 1024 / EPC / 32;                      // chunk loads per lane and row at 1024 channels
+  __shared__ int s_list[256];
+  __shared__ int s_n, s_base;
+  const int b = blockIdx.y;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (threadIdx.x == 0) s_n = 0;
+  __syncthreads();
+  const int a0 = blockIdx.x * 256 + warp * 32;
+  const int a = a0 + lane;
+  if (a0 < p.A) {
+    const int a_last = min(a0 + 31, p.A - 1);
+    int si = 0;
+    if (a0 >= p.s[1].a_off) si = 1;
+    if (a0 >= p.s[2].a_off) si = 2;
+    int sl = 0;
+    if (a_last >= p.s[1].a_off) sl = 1;
+    if (a_last >= p.s[2].a_off) sl = 2;
+    float lmax = -3.0e38f;
+    if (si == sl) {
+      const ScaleSrc<T>& s = p.s[si];
+      const int used = (p.nc + EPC - 1) / EPC;
+      const T* base = s.cls + b * s.cls_bstride + static_cast<long>(a0 - s.a_off) * s.cls_pitch;
+      float v[32];
+#pragma unroll
+      for (int j = 0; j < 32; ++j) {
+        const uint4* row = reinterpret_cast<const uint4*>(base + static_cast<long>(min(j, a_last - a0)) * s.cls_pitch);
+        float m = -3.0e38f;
+#pragma unroll
+        for (int k = 0; k < ROW_ITERS; ++k) {
+          const int c = lane + 32 * k;
+          if (c < used) m = fmaxf(m, chunk_max<T>(row[c], p.nc - c * EPC));
+        }
+        v[j] = m;
+      }
+      // reduce-scatter: at step o a lane keeps the half of its anchors whose index has its own bit o, compacted to v[0, o)
+#pragma unroll
+      for (int o = 16; o >= 1; o >>= 1) {
+        const bool upper = (lane & o) != 0;
+#pragma unroll
+        for (int j = 0; j < o; ++j) {
+          const float send = upper ? v[j] : v[j + o];
+          const float keep = upper ? v[j + o] : v[j];
+          v[j] = fmaxf(keep, __shfl_xor_sync(0xffffffffu, send, o));
+        }
+      }
+      lmax = v[0];
+    } else if (a < p.A) {
+      lmax = anchor_max_walk(p, b, a);
+    }
+    if (a <= a_last && lmax > p.logit_floor) s_list[atomicAdd(&s_n, 1)] = a;
+  }
+  filter_append(s_list, s_n, s_base, p.filt_count, p.filt_list, p.A, b);
+}
+
 // ---- decode, kernel 2 of 2: exact arithmetic on the survivors ----------------------------------------------------------
-// One WARP per listed anchor: the 80 class sigmoids are spread over the lanes and reduced with the graph's first-maximum
+// One WARP per listed anchor: the nc class sigmoids are spread over the lanes and reduced with the graph's first-maximum
 // rule (max probability, lowest index on ties); the four DFL sides go to four lanes, each keeping the sequential 16-bin
 // order; lane 0 does the anchor / stride decode.  IEEE intrinsics in the oracle's operation order throughout.
-template <typename T>
+// NCT: the class count when fixed at compile time (80: the COCO models), 0: p.nc.
+template <typename T, int NCT>
 __global__ void __launch_bounds__(256) decode_exact_kernel(const DecodeParams<T> p) {
   XR_PDL_ENTRY();
+  const int nc = p.nc;
   const int b = blockIdx.y;
   const int n_list = min(p.filt_count[b], p.A);
   const int lane = threadIdx.x & 31;
@@ -183,12 +341,18 @@ __global__ void __launch_bounds__(256) decode_exact_kernel(const DecodeParams<T>
     const float l0 = ldf(bl + lane), l1 = ldf(bl + lane + 32);
     float best = -1.f;
     int besti = 0;
-    for (int c = lane; c < NC; c += 32) {
+    auto take = [&](int c) {
       const float pr = __fdiv_rn(1.0f, __fadd_rn(1.0f, expf(-ldf(cl + c))));
       if (pr > best) {
         best = pr;
         besti = c;
       }
+    };
+    if constexpr (NCT != 0) {
+      for (int c = lane; c < NCT; c += 32) take(c);
+    } else {
+#pragma unroll 1   // the compiler's partial unroll of the run-time trip count spilled
+      for (int c = lane; c < nc; c += 32) take(c);
     }
 #pragma unroll
     for (int o = 16; o >= 1; o >>= 1) {

@@ -103,6 +103,41 @@ T* dev_upload(const std::vector<T>& v) {
   return p;
 }
 
+// Scale and class count of an XRSW pack or .sentis asset: the scale from the first convolution's width (16 outputs: 'n',
+// 32: 's'), the class count from the three *.cls.2 convolutions (canonical indices of that scale's topology), which must agree.
+void weights_info(const void* data, size_t bytes, int& scale, int& nc) {
+  XR_CHECK(data != nullptr, "no weights");
+  std::vector<int> couts;   // output channels of every convolution, canonical order
+  if (looks_like_sentis(data, bytes)) {
+    const SentisWeights sw = sentis_load(data, bytes);
+    for (const SentisConv& cv : sw.convs) couts.push_back(cv.w_shape.size() == 4 ? cv.w_shape[cv.transposed ? 1 : 0] : -1);
+  } else {
+    XR_CHECK(bytes >= sizeof(XrswHeader), "weight pack too small");
+    XrswHeader h;
+    memcpy(&h, data, sizeof(h));
+    XR_CHECK(memcmp(h.magic, "XRSW", 4) == 0 && h.version == 1, "neither an XRSW v1 pack nor a .sentis asset");
+    XR_CHECK(h.n_layers <= 4096 && bytes >= sizeof(XrswHeader) + static_cast<size_t>(h.n_layers) * sizeof(XrswLayer), "truncated pack");
+    for (uint32_t i = 0; i < h.n_layers; ++i) {
+      XrswLayer l;
+      memcpy(&l, static_cast<const uint8_t*>(data) + sizeof(XrswHeader) + i * sizeof(XrswLayer), sizeof(l));
+      couts.push_back(static_cast<int>(l.cout));
+    }
+  }
+  XR_CHECK(!couts.empty() && (couts[0] == 16 || couts[0] == 32), "the first convolution has %d outputs: neither the n (16) nor the s (32) scale",
+           couts.empty() ? 0 : couts[0]);
+  scale = couts[0] == 16 ? 'n' : 's';
+  const Net net(scale, 1);                                   // layer names and order do not depend on the class count
+  XR_CHECK(couts.size() == net.layers.size(), "weights have %zu convolutions, the '%c' topology has %zu", couts.size(),
+           static_cast<char>(scale), net.layers.size());
+  std::vector<int> ncs;
+  for (size_t i = 0; i < net.layers.size(); ++i)
+    if (net.layers[i].name.size() > 6 && net.layers[i].name.compare(net.layers[i].name.size() - 6, 6, ".cls.2") == 0) ncs.push_back(couts[i]);
+  XR_CHECK(ncs.size() == 3 && ncs[0] == ncs[1] && ncs[1] == ncs[2], "the class convolutions disagree: %d / %d / %d classes", ncs[0],
+           ncs[1], ncs[2]);
+  XR_CHECK(ncs[0] >= NC_MIN && ncs[0] <= NC_MAX, "%d classes: supported are %d..%d", ncs[0], NC_MIN, NC_MAX);
+  nc = ncs[0];
+}
+
 }  // namespace
 
 struct xrseg_runner {
@@ -114,6 +149,7 @@ struct xrseg_runner {
   std::unique_ptr<Net> net;
   int mb = 1;                      // frames per network pass
   int A = 8400;
+  int nc = 80;                     // classes of the model (from the weights)
   std::vector<DevLayer> dl;
   __half* arena = nullptr;
   uint8_t* d_frames = nullptr;
@@ -539,7 +575,7 @@ void dense_scale_src(xrseg_runner* r, ScaleSrc<T> (&s)[3], const T* box, const T
   Net& net = *r->net;
   long bstr[3][3], off[3][3];
   int pitch[3][3];
-  const int ch[3] = {64, NC, NM};
+  const int ch[3] = {64, class_pitch(r->nc), NM};   // class rows padded like the network's (the decode reads nc of them)
   long a_off = 0;
   for (int i = 0; i < 3; ++i) {
     for (int j = 0; j < 3; ++j) {
@@ -573,7 +609,7 @@ void add_post_launches(xrseg_runner* r, int b0, int nb, const ScaleSrc<T> (&src)
   if (do_decode) {
     DecodeParams<T> dp{};
     for (int i = 0; i < 3; ++i) dp.s[i] = src[i];
-    dp.B = nb; dp.A = A; dp.score_thr = r->cfg.score_threshold;
+    dp.B = nb; dp.A = A; dp.nc = r->nc; dp.score_thr = r->cfg.score_threshold;
     {
       const double t = r->cfg.score_threshold;
       dp.logit_floor = t <= 0.0 ? -3.0e38f : (t >= 1.0 ? 3.0e38f : static_cast<float>(std::log(t / (1.0 - t)) - 0.01));
@@ -587,12 +623,26 @@ void add_post_launches(xrseg_runner* r, int b0, int nb, const ScaleSrc<T> (&src)
     dp.filt_list = r->d_filt_list + static_cast<long>(b0) * A;
     Launch L;
     L.name = "post.decode";
-    L.bytes = static_cast<double>(nb) * A * NC * sizeof(T);   // every anchor's class logits; box logits only for candidates
-    L.fn = [dp, A, nb](cudaStream_t st) { launch_k(decode_filter_kernel<T>, dim3(ceil_div(A, 256), nb), 256, 0, st, dp); };
+    // every anchor's class row (padding included: it shares the rows' sectors); box logits only for candidates
+    const int pitch = src[0].cls_pitch;
+    L.bytes = static_cast<double>(nb) * A * pitch * sizeof(T);
+    constexpr int EPC = 16 / static_cast<int>(sizeof(T));
+    for (int i = 0; i < 3; ++i)
+      XR_CHECK(src[i].cls_pitch == pitch && pitch % EPC == 0 && pitch >= r->nc && pitch <= NC_MAX, "class tensor pitch %d", src[i].cls_pitch);
+    const dim3 grid(ceil_div(A, 256), nb);
+    if (r->nc == NC) {            // the COCO models: the kernel specialised for 80 classes
+      L.fn = [dp, grid](cudaStream_t st) { launch_k(decode_filter_kernel<T>, grid, 256, 0, st, dp); };
+    } else if (pitch / EPC <= 32) {
+      const size_t smem = static_cast<size_t>(8) * 32 * (pitch / EPC) * sizeof(float);
+      L.fn = [dp, grid, smem](cudaStream_t st) { launch_k(decode_filter_nc_kernel<T>, grid, 256, smem, st, dp); };
+    } else {
+      L.fn = [dp, grid](cudaStream_t st) { launch_k(decode_filter_wide_kernel<T>, grid, 256, 0, st, dp); };
+    }
     out.push_back(std::move(L));
     Launch L2;
     L2.name = "post.decode_exact";
-    L2.fn = [dp, nb](cudaStream_t st) { launch_k(decode_exact_kernel<T>, dim3(8, nb), 256, 0, st, dp); };
+    if (r->nc == NC) L2.fn = [dp, nb](cudaStream_t st) { launch_k(decode_exact_kernel<T, NC>, dim3(8, nb), 256, 0, st, dp); };
+    else L2.fn = [dp, nb](cudaStream_t st) { launch_k(decode_exact_kernel<T, 0>, dim3(8, nb), 256, 0, st, dp); };
     out.push_back(std::move(L2));
   }
   SortParams sp{};
@@ -1019,10 +1069,12 @@ int xrseg_device_count(void) {
   return ok;
 }
 
-int xrseg_layer_count(int model_scale) {
+int xrseg_layer_count(int model_scale) { return xrseg_layer_count_nc(model_scale, 80); }
+
+int xrseg_layer_count_nc(int model_scale, int num_classes) {
   try {
-    if (model_scale != 'n' && model_scale != 's') return XRSEG_ERR_INVALID;
-    Net net(model_scale, 1);
+    if ((model_scale != 'n' && model_scale != 's') || num_classes < NC_MIN || num_classes > NC_MAX) return XRSEG_ERR_INVALID;
+    Net net(model_scale, 1, 640, true, true, num_classes);
     return static_cast<int>(net.layers.size());
   } catch (const CudaError& e) {
     g_create_error = e.msg;
@@ -1037,9 +1089,13 @@ int xrseg_layer_count(int model_scale) {
 }
 
 int xrseg_layer_info_get(int model_scale, int index, xrseg_layer_info* info) {
+  return xrseg_layer_info_get_nc(model_scale, 80, index, info);
+}
+
+int xrseg_layer_info_get_nc(int model_scale, int num_classes, int index, xrseg_layer_info* info) {
   try {
-    if ((model_scale != 'n' && model_scale != 's') || !info) return XRSEG_ERR_INVALID;
-    Net net(model_scale, 1);
+    if ((model_scale != 'n' && model_scale != 's') || num_classes < NC_MIN || num_classes > NC_MAX || !info) return XRSEG_ERR_INVALID;
+    Net net(model_scale, 1, 640, true, true, num_classes);
     if (index < 0 || index >= static_cast<int>(net.layers.size())) return XRSEG_ERR_INVALID;
     const LayerRec& l = net.layers[index];
     memset(info, 0, sizeof(*info));
@@ -1079,6 +1135,28 @@ int xrseg_sentis_info(const void* data, size_t bytes, int32_t* n_convs, float* i
     return XRSEG_ERR_WEIGHTS;
   }
 }
+
+int xrseg_weights_info(const void* data, size_t bytes, int32_t* model_scale, int32_t* num_classes) {
+  if (!data) return XRSEG_ERR_INVALID;
+  try {
+    int scale = 0, nc = 0;
+    weights_info(data, bytes, scale, nc);
+    if (model_scale) *model_scale = scale;
+    if (num_classes) *num_classes = nc;
+    return XRSEG_OK;
+  } catch (const CudaError& e) {
+    g_create_error = e.msg;
+    return XRSEG_ERR_WEIGHTS;
+  } catch (const std::exception& e) {   // nothing may unwind across the C boundary
+    g_create_error = std::string("unexpected exception: ") + e.what();
+    return XRSEG_ERR_WEIGHTS;
+  } catch (...) {
+    g_create_error = "unknown exception";
+    return XRSEG_ERR_WEIGHTS;
+  }
+}
+
+int xrseg_num_classes(const xrseg_runner* r) { return r ? r->nc : XRSEG_ERR_INVALID; }
 
 int xrseg_sentis_layer(const void* data, size_t bytes, int index, float* w, size_t w_cap, float* b, size_t b_cap,
                        int32_t* w_shape4, int32_t* transposed) {
@@ -1157,11 +1235,22 @@ int xrseg_create(const xrseg_config* cfg_in, xrseg_runner** out) {
     XR_CUDA(cudaFuncSetAttribute((nms_reduce_kernel<1, 4>), cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * 32 * 64 * 8));
     XR_CUDA(cudaFuncSetAttribute((nms_reduce_kernel<5, 2>), cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * 132 * 64 * 8));
 
+    try {   // the class count comes from the weights; a nonzero num_classes only confirms it
+      int wscale = 0;
+      weights_info(c.weights, c.weights_bytes, wscale, r->nc);
+      XR_CHECK(c.num_classes == 0 || c.num_classes == r->nc, "num_classes is %d, the weights have %d classes", c.num_classes, r->nc);
+    } catch (const CudaError& e) {
+      g_create_error = e.msg;
+      return XRSEG_ERR_WEIGHTS;
+    } catch (const std::exception& e) {
+      g_create_error = std::string("unexpected exception: ") + e.what();
+      return XRSEG_ERR_WEIGHTS;
+    }
     r->mb = c.micro_batch > 0 ? std::min(c.micro_batch, c.max_batch) : c.max_batch;
     const char* fuse_env = getenv("XRSEG_FUSE");
     const bool fuse = c.conv_impl == XRSEG_CONV_UMMA && !(fuse_env && fuse_env[0] == '0');
     const char* bneck_env = getenv("XRSEG_FUSE_BNECK");
-    r->net.reset(new Net(c.model_scale, r->mb, 640, fuse, !(bneck_env && bneck_env[0] == '0')));
+    r->net.reset(new Net(c.model_scale, r->mb, 640, fuse, !(bneck_env && bneck_env[0] == '0'), r->nc));
     Net& net = *r->net;
     r->A = net.fh[0] * net.fw[0] + net.fh[1] * net.fw[1] + net.fh[2] * net.fw[2];
     std::vector<HostLayerWeights> hw;
@@ -1748,15 +1837,18 @@ static int debug_post_impl(xrseg_runner* r, const float* box_logits, const float
     XR_CUDA(cudaSetDevice(r->device));
     const size_t A = r->A;
     const size_t B = r->cfg.max_batch;
+    const size_t nc = r->nc, pitch = class_pitch(r->nc);      // caller rows [A, nc] -> device rows of `pitch` (padding stays 0)
     if (!r->dbg_box) {
       r->dbg_box = dev_alloc<float>(B * A * 64);
-      r->dbg_cls = dev_alloc<float>(B * A * NC);
+      r->dbg_cls = dev_alloc<float>(B * A * pitch);
+      XR_CUDA(cudaMemset(r->dbg_cls, 0, sizeof(float) * B * A * pitch));
       r->dbg_coef = dev_alloc<float>(B * A * NM);
       r->dbg_proto = dev_alloc<float>(B * NM * PROTO_PIX);
     }
     cudaStream_t st = r->stream;
     XR_CUDA(cudaMemcpyAsync(r->dbg_box, box_logits, sizeof(float) * batch * A * 64, cudaMemcpyHostToDevice, st));
-    XR_CUDA(cudaMemcpyAsync(r->dbg_cls, cls_logits, sizeof(float) * batch * A * NC, cudaMemcpyHostToDevice, st));
+    XR_CUDA(cudaMemcpy2DAsync(r->dbg_cls, sizeof(float) * pitch, cls_logits, sizeof(float) * nc, sizeof(float) * nc, batch * A,
+                              cudaMemcpyHostToDevice, st));
     XR_CUDA(cudaMemcpyAsync(r->dbg_coef, coefs, sizeof(float) * batch * A * NM, cudaMemcpyHostToDevice, st));
     XR_CUDA(cudaMemcpyAsync(r->dbg_proto, protos, sizeof(float) * batch * NM * PROTO_PIX, cudaMemcpyHostToDevice, st));
     r->batch = batch;
@@ -1765,9 +1857,9 @@ static int debug_post_impl(xrseg_runner* r, const float* box_logits, const float
     std::vector<Launch> ls;
     if (as_f16) {
       // the product kernels (fp16 head tensors, NHWC prototypes, mma.sync mask assembly) on the caller's tensors
-      const size_t nb_ = batch * A * 64, nc_ = batch * A * NC, nm_ = batch * A * NM, np_ = static_cast<size_t>(batch) * NM * PROTO_PIX;
-      if (!r->dbg_h16) r->dbg_h16 = dev_alloc<__half>(B * (A * (64 + NC + NM) + static_cast<size_t>(NM) * PROTO_PIX));
-      __half *hb = r->dbg_h16, *hc = hb + B * A * 64, *hm = hc + B * A * NC, *hp = hm + B * A * NM;
+      const size_t nb_ = batch * A * 64, nc_ = batch * A * pitch, nm_ = batch * A * NM, np_ = static_cast<size_t>(batch) * NM * PROTO_PIX;
+      if (!r->dbg_h16) r->dbg_h16 = dev_alloc<__half>(B * (A * (64 + pitch + NM) + static_cast<size_t>(NM) * PROTO_PIX));
+      __half *hb = r->dbg_h16, *hc = hb + B * A * 64, *hm = hc + B * A * pitch, *hp = hm + B * A * NM;
       f32_to_f16_kernel<<<grid_for(static_cast<long>(nb_)), 256, 0, st>>>(r->dbg_box, hb, static_cast<long>(nb_));
       f32_to_f16_kernel<<<grid_for(static_cast<long>(nc_)), 256, 0, st>>>(r->dbg_cls, hc, static_cast<long>(nc_));
       f32_to_f16_kernel<<<grid_for(static_cast<long>(nm_)), 256, 0, st>>>(r->dbg_coef, hm, static_cast<long>(nm_));

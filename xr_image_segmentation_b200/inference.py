@@ -27,31 +27,27 @@ class BackendType:
 
 
 class Model:
-    """↔ Unity.InferenceEngine.Model: an XRSW weight pack + the topology scale."""
+    """↔ Unity.InferenceEngine.Model: an XRSW weight pack (or .sentis asset) + the topology scale and class count."""
 
-    def __init__(self, pack: bytes, scale: str = "n"):
+    def __init__(self, pack: bytes, scale: str = "n", nc: int = 80):
         self.pack = pack
         self.scale = scale
+        self.nc = nc
 
 
 class ModelLoader:
     @staticmethod
     def Load(asset) -> Model:
-        """↔ ModelLoader.Load(ModelAsset) IEE:382.  `asset`: path to / bytes of an XRSW pack."""
+        """↔ ModelLoader.Load(ModelAsset) IEE:382.  `asset`: path to / bytes of an XRSW pack or a .sentis asset (parsed
+        inside libxrseg.so); the scale and class count are read from the weights (xrseg_weights_info)."""
         data = asset if isinstance(asset, (bytes, bytearray)) else open(os.fspath(asset), "rb").read()
-        if data[:4] == b"XRSW":
-            return Model(bytes(data), chr(int.from_bytes(data[12:16], "little")))
-        # the sample's own .sentis asset: parsed (FlatBuffer walk + uint8 dequantization) inside libxrseg.so
         lib = _lib.load_library()
         buf = C.create_string_buffer(bytes(data), len(data))
-        n = C.c_int32()
-        rc = lib.xrseg_sentis_info(C.cast(buf, C.c_void_p), len(data), C.byref(n), None, None)
+        scale, nc = C.c_int32(), C.c_int32()
+        rc = lib.xrseg_weights_info(C.cast(buf, C.c_void_p), len(data), C.byref(scale), C.byref(nc))
         if rc < 0:
-            raise XrsegError(_lib.ERR_WEIGHTS, "neither an XRSW weight pack nor a .sentis asset")
-        scale = {100: "n"}.get(n.value)
-        if scale is None:
-            raise XrsegError(_lib.ERR_WEIGHTS, f".sentis asset with {n.value} convolutions does not match a known topology")
-        return Model(bytes(data), scale)
+            raise XrsegError(_lib.ERR_WEIGHTS, "not a usable XRSW weight pack or .sentis asset: " + lib.xrseg_last_error(None).decode())
+        return Model(bytes(data), chr(scale.value), nc.value)
 
 
 class Runner:
@@ -59,7 +55,7 @@ class Runner:
 
     def __init__(self, model: Model, device: int = 0, max_batch: int = 1, iou=0.0, score=0.0, mask_thr=0.0,
                  max_det=0, max_candidates=0, resize_mode=_lib.RESIZE_STRETCH, conv_impl=_lib.CONV_UMMA,
-                 use_cuda_graph=True, micro_batch=0, debug=False):
+                 use_cuda_graph=True, micro_batch=0, debug=False, num_classes=0):
         # debug=True: the runner lives in libxrseg_debug.so (same sources + the parity hooks of include/xrseg_debug.h:
         # fetch / debug_post / debug_nms / debug_mask_threshold); the product library exports none of them
         self.debug = debug
@@ -77,12 +73,18 @@ class Runner:
         cfg.resize_mode, cfg.conv_impl = resize_mode, conv_impl
         cfg.use_cuda_graph = 1 if use_cuda_graph else 0
         cfg.micro_batch = micro_batch
+        cfg.num_classes = num_classes
         self.h = C.c_void_p()
         _lib.check(self.lib.xrseg_create(C.byref(cfg), C.byref(self.h)), None, self.lib)
         self.max_batch = max_batch
         self.batch = 0
         self._max_det = max_det if max_det > 0 else 300          # the library's default cap per frame (xrseg_config.max_det)
         self._collect_buf = None
+
+    @property
+    def num_classes(self) -> int:
+        """Classes of the runner's model (labels are 0 .. num_classes - 1)."""
+        return self._ck(self.lib.xrseg_num_classes(self.h))
 
     def close(self):
         if getattr(self, "h", None) and self.h.value:
@@ -298,16 +300,22 @@ class Runner:
     def fetch(self, name: str) -> np.ndarray:
         self._need_debug()
         shp = (C.c_int64 * 4)()
-        cap = max(64, self.max_batch) * 1024 * 1024      # the largest tensor fetched by the tests: protos, 0.82 M floats per frame
-        buf = np.empty(cap, np.float32)
-        self._ck(self.lib.xrseg_debug_fetch(self.h, name.encode(), buf.ctypes.data, cap, shp))
+        probe = np.empty(1, np.float32)                  # a zero-capacity call reports the shape (class logits grow with nc)
+        rc = self.lib.xrseg_debug_fetch(self.h, name.encode(), probe.ctypes.data, 0, shp)
+        if rc != _lib.ERR_CAPACITY:
+            self._ck(rc)
         shape = [int(s) for s in shp]
-        return buf[:int(np.prod(shape))].reshape(shape).copy()
+        n = int(np.prod(shape))
+        buf = np.empty(max(n, 1), np.float32)
+        self._ck(self.lib.xrseg_debug_fetch(self.h, name.encode(), buf.ctypes.data, n, shp))
+        return buf[:n].reshape(shape)
 
     def debug_post(self, box_logits, cls_logits, coefs, protos, f16=False):
         """Post-processing alone on caller tensors: fp32 bit-exact kernels, or (f16) the product's fp16 kernels."""
         self._need_debug()
         arrs = [np.ascontiguousarray(a, np.float32) for a in (box_logits, cls_logits, coefs, protos)]
+        if arrs[1].shape[-1] != self.num_classes:
+            raise ValueError(f"cls_logits have {arrs[1].shape[-1]} classes, the runner's model {self.num_classes}")
         b = arrs[0].shape[0]
         self.batch = b
         fn = self.lib.xrseg_debug_post_f16 if f16 else self.lib.xrseg_debug_post

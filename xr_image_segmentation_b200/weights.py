@@ -45,14 +45,14 @@ class Layer:
         return (self.cout, self.cin // self.groups, self.k, self.k)
 
 
-def layer_table(scale: str) -> list[Layer]:
-    """The topology's convolution list, straight from the C library (single source of truth)."""
+def layer_table(scale: str, nc: int = 80) -> list[Layer]:
+    """The topology's convolution list for a model of `nc` classes, straight from the C library (single source of truth)."""
     lib = _lib.load_library()
-    n = _lib.check(lib.xrseg_layer_count(ord(scale)))
+    n = _lib.check(lib.xrseg_layer_count_nc(ord(scale), nc))
     out = []
     for i in range(n):
         info = _lib.LayerInfo()
-        _lib.check(lib.xrseg_layer_info_get(ord(scale), i, C.byref(info)))
+        _lib.check(lib.xrseg_layer_info_get_nc(ord(scale), nc, i, C.byref(info)))
         out.append(Layer(info.name.decode(), info.cin, info.cout, info.k, info.stride, info.groups, info.act,
                          info.transposed, info.h_in, info.w_in))
     return out
@@ -132,12 +132,16 @@ INIT_BIAS_STD = 0.2
 INIT_CLS_BIAS = {"n": -5.15, "s": -12.4}
 
 
-def random_weights(scale: str, seed: int, cls_bias: float | None = None):
+def random_weights(scale: str, seed: int, cls_bias: float | None = None, nc: int = 80):
     """Random-init network of BASELINE.json configs 2/3: w ~ N(0, (1.5/sqrt(fan_in))^2), b ~ N(0, 0.2^2), final class
-    conv biases N(cls_bias, 0.05^2).  Returns (layers, [(w, b)])."""
-    cls_bias = INIT_CLS_BIAS[scale] if cls_bias is None else cls_bias
+    conv biases N(cls_bias, 0.05^2).  Returns (layers, [(w, b)]).  INIT_CLS_BIAS was tuned for 80 classes: a network of
+    another class count needs its own cls_bias."""
+    if cls_bias is None:
+        if nc != 80:
+            raise ValueError(f"random_weights: pass cls_bias for a {nc}-class network (INIT_CLS_BIAS is tuned for 80 classes)")
+        cls_bias = INIT_CLS_BIAS[scale]
     rng = np.random.default_rng(seed)
-    layers = layer_table(scale)
+    layers = layer_table(scale, nc)
     out = []
     for l in layers:
         fan_in = l.cin if l.transposed else (l.cin // l.groups) * l.k * l.k
