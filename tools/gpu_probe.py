@@ -116,6 +116,7 @@ def step_layers():
     """Per-layer comparison UMMA vs DIRECT runner on one golden frame."""
     model, inputs, exp = load_golden()
     img = inputs["coco139"]
+    os.environ.setdefault("XRSEG_FUSE_UP", "0")     # fetch proto.up / proto.cv2 by name: keep them as their own launches
     ra = I.Runner(model, max_batch=1, conv_impl=_lib.CONV_DIRECT, use_cuda_graph=False)
     rb = I.Runner(model, max_batch=1, conv_impl=_lib.CONV_UMMA, use_cuda_graph=False)
     ra.schedule(img[None]); ra.wait()

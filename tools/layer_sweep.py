@@ -40,6 +40,7 @@ def main():
     weights = [(w, b) for _, w, b in layers]
     names = [n for n, _, _ in layers]
     inputs = np.load(os.path.join(g, "inputs.npz"))
+    os.environ.setdefault("XRSEG_FUSE_UP", "0")     # proto.up / proto.cv2 as their own launches: the merged launch has no such maps
     r = I.Runner(model, max_batch=1, debug=True)
     acc = {n: [0.0, 0.0, 0.0] for n in names}          # sum sq err, sum sq ref, max abs
     head = {k: [0.0, 0.0, 0.0] for k in ("box_logits", "cls_logits", "coefs", "protos")}

@@ -546,7 +546,78 @@ static inline bool plan_with_split(ConvParams& p, int num_sms, Plan plan) {
   }
   return true;
 }
+// ConvTranspose 2x2 / stride 2 + 3x3 stride 1 as ONE halo convolution over the map before the upsampling (ConvDesc::upm; the
+// n scale's proto.up -> proto.cv2, 64 -> 64 -> 64 channels, 80x80 -> 160x160).  Output pixel (2y + dy, 2x + dx) is a 2x2-tap
+// convolution of input rows y + dy - 1 .. y + dy and columns x + dx - 1 .. x + dx: in the 3x3 halo these are taps
+// (dy + {0,1}, dx + {0,1}).  Layout of a work item (R = 3 input rows of one image, one row parity dy = item & 1):
+//   * two 128-row sub-tiles of halo positions; each holds BOTH column parities: 2 x 64 accumulator columns, so that the
+//     accumulator set has 256 columns and the virtual sub-tile v = 2 u + dx is what the rest of the kernel calls a sub-tile
+//     (nsub = 4, Ntile = 64: TMEM, the four MMA warps, the fused-tail epilogue); 246 of 256 rows valid;
+//   * MMA warp v issues its parity's four taps x 4 k16 steps against resident weights [dx][tap][64][64] of its CTA's dy:
+//     a CTA only ever sees one row parity (the grid is even, items alternate dy), so it keeps 64 KB of the 128 KB resident;
+//   * the epilogue scatters halo position (y, x) of virtual sub-tile v to output pixel (2y + dy, 2x + dx); pixels on the
+//     border of the 160x160 map add a correction to the bias (cv2's zero padding drops the ConvTranspose bias there).
+// The K per output pixel falls from 576 to 256.  One K-block of 64 channels (Cin = 64), two stages (the 410-row halo box is
+// 52 KB), two accumulator sets = 512 TMEM columns.
+static inline bool plan_conv_upmerge_tma(const ConvDesc& d, int num_sms, ConvParams& p) {
+  if (!(d.upm && d.k == 3 && d.stride == 1 && !d.transposed && d.Cin == 64 && d.Cout == 64 && d.res_pitch == 0 && d.H >= 2)) return false;
+  p = ConvParams{};
+  p.B = d.B; p.H = d.H; p.W = d.W; p.Cin = d.Cin; p.in_pitch = d.in_pitch;
+  p.Cout = d.Cout; p.out_pitch = d.out_pitch; p.res_pitch = 0;
+  p.k = 3; p.stride = 1; p.pad = 1; p.act = d.act; p.transposed = 0; p.upm = 1;
+  p.Ho = 2 * d.H; p.Wo = 2 * d.W;
+  p.Ntile = 64; p.n_tiles = 1;
+  p.idesc = umma_idesc_f16(p.Ntile, 0);
+  p.mode = MODE_HALO_TMA;
+  p.Wp = d.W + 2;
+  p.Hp1 = d.H + 1;
+  if (p.Wp > 256) return false;
+  p.R = 256 / p.Wp < d.H ? 256 / p.Wp : d.H;    // the rows two 128-row sub-tiles hold
+  const int real_sub = ceil_div(p.R * p.Wp, 128);
+  p.nsub = 2 * real_sub;                          // virtual sub-tiles (sub-tile, column parity)
+  p.tpi = ceil_div(d.H, p.R);
+  p.hbox = p.R + 2;
+  p.slots = p.hbox * p.Wp;
+  p.cb = 64; p.cps = 8; p.nks = 1; p.kps = 1; p.sw = 3;
+  p.taps = 8;                                     // per row parity: 2 column parities x 4 taps
+  p.K_total = 4 * d.Cin;
+  p.nbuf = 2;
+  p.tmem_cols = pow2_ceil(p.nbuf * p.nsub * p.Ntile);
+  const int rb = p.cb * 2;
+  p.lbo_a = round_up(p.slots * 16, 128);
+  p.a_stage_bytes = round_up(p.slots * rb, 1024);
+  p.b_stage_bytes = p.taps * p.Ntile * rb;        // one row parity's weights; the image holds both
+  p.b_resident = 1;
+  p.M_total = 2 * d.B * p.tpi;                    // (row tile, row parity), parity fastest
+  p.m_tiles = p.M_total;
+  p.smem_off_b = round_up(CONV_HDR_BYTES, 1024);
+  p.smem_off_a = p.smem_off_b + round_up(p.b_stage_bytes, 1024) + 1024;   // one pad row block before the stages (row -1)
+  // rows read past the last stage: the second sub-tile's last position + the farthest tap (2 Wp + 1)
+  const int tail_rows = real_sub * 128 + 2 * p.Wp + 1 - p.slots;
+  const int tail = round_up((tail_rows > 0 ? tail_rows : 0) * rb, 1024);
+  const int corr = 9 * p.Ntile * 4;
+  const int fixed = p.smem_off_a + tail + corr + p.Ntile * 32 * 2 + 1024;   // + the fused tail's W2 (xrseg_api.cu) and its alignment
+  int S = (CONV_SMEM_MAX - fixed) / p.a_stage_bytes;
+  if (S > CONV_MAX_STAGES) S = CONV_MAX_STAGES;
+  if (S < 2) return false;
+  p.S = clamp_stages(S, p.m_tiles, num_sms, p.nks);
+  p.smem_off_corr = p.smem_off_a + p.S * p.a_stage_bytes + tail;
+  p.smem_bytes = p.smem_off_corr + corr;
+  if (p.smem_bytes > CONV_SMEM_MAX) return false;
+  const int grid = (p.m_tiles < num_sms ? p.m_tiles : num_sms) & ~1;   // even: a CTA's items all have one row parity
+  if (grid < 2) return false;
+  p.grid = grid;
+  p.fd_wp = make_fastdiv(p.Wp);
+  p.fd_hp1 = make_fastdiv(p.tpi);
+  p.fd_hw = make_fastdiv(1);
+  p.fd_wo = make_fastdiv(1);
+  p.fd_cin = make_fastdiv(d.Cin);
+  p.fd_cout = make_fastdiv(d.Cout);
+  return true;
+}
+
 static inline bool plan_conv_halo_tma(const ConvDesc& d, int num_sms, ConvParams& p, bool swizzled = true) {
+  if (d.upm) return swizzled && plan_conv_upmerge_tma(d, num_sms, p);
   if (!swizzled) return plan_conv_halo_tma_impl(d, num_sms, p, false);
   return plan_with_split(p, num_sms, [&](ConvParams& q) { return plan_conv_halo_tma_impl(d, num_sms, q); });
 }
@@ -572,7 +643,7 @@ static inline ConvParams replan_for_batch(const ConvParams& full, int nb, int nu
     p.flat_rows = nb * p.H * p.W;
     p.M_total = ceil_div(p.flat_rows, p.slots);
   } else if (p.mode == MODE_HALO_TMA || p.mode == MODE_S2_TMA) {
-    p.M_total = nb * p.tpi;
+    p.M_total = (nb * p.tpi) << (p.upm ? 1 : 0);     // merged ConvTranspose: (row tile, row parity) items
   } else if (p.mode == MODE_HALO) {
     p.M_total = nb * p.Hp1 * p.Wp;
   } else {
@@ -581,6 +652,7 @@ static inline ConvParams replan_for_batch(const ConvParams& full, int nb, int nu
   p.m_tiles = (p.mode == MODE_GATHER || p.mode == MODE_HALO) ? ceil_div(p.M_total, 128) : p.M_total;
   const int work = p.m_tiles * p.n_tiles;
   p.grid = work < num_sms ? work : num_sms;
+  if (p.upm) p.grid &= ~1;
   return p;
 }
 
@@ -626,6 +698,72 @@ static inline void pack_conv_weights_sw(const ConvParams& p, const float* w, con
   }
 }
 
+// ConvTranspose 2x2 / stride 2 (wt [ci][cm][2][2], bias bt [cm], no activation) followed by a 3x3 stride-1 convolution (w2
+// [co][cm][3][3], bias b2 [co]) on the 2H x 2W map, as the parity convolutions of plan_conv_upmerge_tma; fp64 throughout.
+// Tap (kh, kw) of output row 2y + dy reads upsampled row 2y + r, r = dy + kh - 1, i.e. input row y + floor(r / 2) at kernel
+// row a = r mod 2 of the ConvTranspose (the same for columns), so
+//   wm[dy][dx][th][tw][o][i] = sum over (kh, kw) landing on input tap (dy + th - 1, dx + tw - 1) of sum_c w2[o][c][kh][kw] wt[i][c][a][b].
+// cv2 zero-pads the UPSAMPLED map, so bt contributes only through cv2's taps inside it: bm[0, co) is the interior bias
+// b2 + sum_{kh,kw} w2[:, :, kh, kw] bt, bm[co (1 + cls) + o] the correction of border class cls = 3 rowc + colc (rowc: 0 inner
+// row, 1 first, 2 last; colc likewise; cls 0 = interior, zero) -- minus the terms of the taps that fall outside.  Out-of-range
+// taps of the INPUT need nothing: they are zeros (the TMA zero fill).
+static inline void merge_upconv_weights(const float* wt, const float* bt, const float* w2, const float* b2, int ci, int cm, int co,
+                                        std::vector<double>& wm, std::vector<double>& bm) {
+  wm.assign(static_cast<size_t>(16) * co * ci, 0.0);
+  bm.assign(static_cast<size_t>(10) * co, 0.0);
+  for (int dy = 0; dy < 2; ++dy)
+    for (int dx = 0; dx < 2; ++dx)
+      for (int kh = 0; kh < 3; ++kh)
+        for (int kw = 0; kw < 3; ++kw) {
+          const int r = dy + kh - 1, s = dx + kw - 1;
+          const int di = r < 0 ? -1 : r / 2, dj = s < 0 ? -1 : s / 2;
+          const int a = r - 2 * di, b = s - 2 * dj;
+          const int th = di - dy + 1, tw = dj - dx + 1;
+          double* dst = wm.data() + static_cast<size_t>(((dy * 2 + dx) * 2 + th) * 2 + tw) * co * ci;
+          for (int o = 0; o < co; ++o)
+            for (int c = 0; c < cm; ++c) {
+              const double w2v = w2[(static_cast<size_t>(o) * cm + c) * 9 + kh * 3 + kw];
+              for (int i = 0; i < ci; ++i) dst[static_cast<size_t>(o) * ci + i] += w2v * wt[((static_cast<size_t>(i) * cm + c) * 2 + a) * 2 + b];
+            }
+        }
+  std::vector<double> t(static_cast<size_t>(9) * co, 0.0);          // t[kh][kw][o] = sum_c w2[o][c][kh][kw] bt[c]
+  for (int o = 0; o < co; ++o)
+    for (int k = 0; k < 9; ++k)
+      for (int c = 0; c < cm; ++c) t[static_cast<size_t>(k) * co + o] += static_cast<double>(w2[(static_cast<size_t>(o) * cm + c) * 9 + k]) * bt[c];
+  for (int o = 0; o < co; ++o) {
+    double s = b2 ? b2[o] : 0.0;
+    for (int k = 0; k < 9; ++k) s += t[static_cast<size_t>(k) * co + o];
+    bm[o] = s;
+  }
+  for (int cls = 1; cls < 9; ++cls) {
+    const int rowc = cls / 3, colc = cls % 3;
+    const int bad_kh = rowc == 1 ? 0 : (rowc == 2 ? 2 : -1), bad_kw = colc == 1 ? 0 : (colc == 2 ? 2 : -1);
+    for (int o = 0; o < co; ++o) {
+      double s = 0.0;
+      for (int k = 0; k < 9; ++k)
+        if (k / 3 == bad_kh || k % 3 == bad_kw) s -= t[static_cast<size_t>(k) * co + o];
+      bm[static_cast<size_t>(co) * (1 + cls) + o] = s;
+    }
+  }
+}
+
+// Swizzled weight image of a merged plan: [dy][dx][tap = th * 2 + tw][n][64 channels], one row parity = one resident stage;
+// each fp64 weight is rounded to fp16 once.
+static inline void pack_upmerge_weights_sw(const ConvParams& p, const std::vector<double>& wm, int ci, int co, std::vector<__half>& wp) {
+  const size_t stage_elems = static_cast<size_t>(p.b_stage_bytes) / 2;
+  wp.assign(2 * stage_elems, __float2half(0.0f));
+  const int rb = p.cb * 2;
+  for (int dy = 0; dy < 2; ++dy)
+    for (int dx = 0; dx < 2; ++dx)
+      for (int tap = 0; tap < 4; ++tap)
+        for (int n = 0; n < co; ++n)
+          for (int c = 0; c < ci; ++c) {
+            const double v = wm[((static_cast<size_t>((dy * 2 + dx) * 4 + tap)) * co + n) * ci + c];
+            const size_t off = (static_cast<size_t>(dx * 4 + tap) * p.Ntile + n) * rb + static_cast<size_t>(c) * 2;
+            wp[dy * stage_elems + sw_phys(off, p.sw) / 2] = __double2half(v);
+          }
+}
+
 #ifdef __CUDACC__
 // ---- PTX: TMA + bulk copy ----------------------------------------------------------------------------------------
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
@@ -667,6 +805,23 @@ __device__ __forceinline__ void issue_taps(uint32_t d_tmem, uint32_t a_sub, uint
       a_sub += blk16;
       b_lo += tap16;
       asm volatile("" : "+r"(a_sub), "+r"(b_lo));   // the next K-block's descriptors are computed after these MMAs were issued
+    }
+    return;
+  }
+  if (MODE == 3) {   // merged ConvTranspose (plan_conv_upmerge_tma): a_sub is this parity's tap (0, 0); tap (th, tw) = th Wp + tw rows on
+#pragma unroll
+    for (int th = 0; th < 2; ++th) {
+#pragma unroll
+      for (int tw = 0; tw < 2; ++tw) {
+        const uint32_t a_tap = a_sub + th * wp16 + tw * row16;
+#pragma unroll
+        for (int j = 0; j < KJ; ++j) {
+          umma_f16(d_tmem, hi_a | (a_tap + 2u * j), hi_sw | (b_lo + 2u * j), idesc, acc);
+          acc = 1;
+        }
+        b_lo += tap16;
+        asm volatile("" : "+r"(a_sub), "+r"(b_lo));
+      }
     }
     return;
   }
@@ -964,7 +1119,10 @@ __device__ __forceinline__ void tma_epilogue_loop(const ConvParams& p, uint32_t 
 // In place (proto.cv2 -> cv3, TMEM full): packed columns 64u + {0, 24, 32, 56}, D2 as two N = 16 halves in the freed runs
 // [8, 24) and [40, 56) of the same 64 columns.  The intermediate never reaches shared or global memory.
 __device__ __forceinline__ uint32_t tail_pack_col(int c) { return c == 0 ? 0u : (c == 1 ? 24u : (c == 2 ? 32u : 56u)); }
-template <bool PROBE>
+// UPM (merged ConvTranspose, plan_conv_upmerge_tma): virtual sub-tile u = 2 (128-row sub-tile) + column parity, row parity dy =
+// item & 1; a lane's halo position (y, x) goes to output pixel (2y + dy, 2x + dx), and the 16 accumulators of a pixel on the
+// border of the output map get its class's correction (corr_s [9][64]) added before the bias -- only those lanes do it.
+template <bool PROBE, bool UPM>
 __device__ __forceinline__ void tma_epilogue_loop_tail(const ConvParams& p, uint32_t tmem_base, uint64_t* tfull, uint64_t* tempty,
                                                        uint64_t* tready, uint64_t* t2full, const float* bias_s, int warp, int lane,
                                                        int total_work) {
@@ -982,6 +1140,7 @@ __device__ __forceinline__ void tma_epilogue_loop_tail(const ConvParams& p, uint
   const FastDiv fd_wp = p.fd_wp, fd_tpi = p.fd_hp1;
   const uint32_t lane_taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
   const uint32_t pk_col = tail_pack_col(c1);
+  const float* corr_s = reinterpret_cast<const float*>(reinterpret_cast<const uint8_t*>(bias_s) - 256 + p.smem_off_corr);   // UPM only
   float hbr[16];
 #pragma unroll
   for (int i = 0; i < 16; ++i) hbr[i] = bias_s[c1 * 16 + i];
@@ -989,21 +1148,31 @@ __device__ __forceinline__ void tma_epilogue_loop_tail(const ConvParams& p, uint
   long long e_wait = 0, e_work = 0, t0 = 0;
   pdl_wait();
   for (int w = blockIdx.x; w < total_work; w += gridDim.x, ++tcount) {
-    const int tile = w;
+    const int tile = UPM ? w >> 1 : w;
     const int b = fd_div(fd_tpi, tile);
     const int y0 = (tile - b * tpi) * Rr;
     const int buf = tcount & 1;
     const uint32_t use = static_cast<uint32_t>(tcount >> 1);
     int pix[4];
+    uint32_t cls4 = 0;                 // UPM: border class of each virtual sub-tile's pixel, 4 bits each
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
       pix[u] = -1;
       if (u < nsub) {
-        const int j = 128 * u + q * 32 + lane;
+        const int j = 128 * (UPM ? u >> 1 : u) + q * 32 + lane;
         const int yy = fd_div(fd_wp, j);
         const int cc = j - yy * Wp;
         const int y = y0 + yy;
-        if (yy < Rr && y < Hh && cc >= 1 && cc <= Ww) pix[u] = (b * Hh + y) * Ww + (cc - 1);
+        if (yy < Rr && y < Hh && cc >= 1 && cc <= Ww) {
+          if (UPM) {
+            const int oy = 2 * y + (w & 1), ox = 2 * (cc - 1) + (u & 1), Ho = 2 * Hh, Wo = 2 * Ww;
+            pix[u] = (b * Ho + oy) * Wo + ox;
+            const uint32_t cls = 3u * (oy == 0 ? 1u : (oy == Ho - 1 ? 2u : 0u)) + (ox == 0 ? 1u : (ox == Wo - 1 ? 2u : 0u));
+            cls4 |= cls << (4 * u);
+          } else {
+            pix[u] = (b * Hh + y) * Ww + (cc - 1);
+          }
+        }
       }
     }
     if (PROBE) t0 = clock64();
@@ -1022,6 +1191,14 @@ __device__ __forceinline__ void tma_epilogue_loop_tail(const ConvParams& p, uint
         const int u = u1 + k * step1;
         if (u >= nsub) break;
         tmem_ld_wait();
+        if (UPM) {
+          const uint32_t cls = (cls4 >> (4 * u)) & 15u;
+          if (cls) {
+            const float* cv = corr_s + cls * 64u + c1 * 16;
+#pragma unroll
+            for (int i = 0; i < 16; ++i) v[i] = __float_as_uint(__uint_as_float(v[i]) + cv[i]);
+          }
+        }
         uint32_t o[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i)
@@ -1122,10 +1299,12 @@ conv_halo_tma_kernel(const __grid_constant__ ConvParams p, const __grid_constant
       const uint32_t bytes = static_cast<uint32_t>(p.nks) * p.b_stage_bytes;
       const uint32_t tail_bytes = p.tail_n ? static_cast<uint32_t>(p.tail_n) * static_cast<uint32_t>(p.Ntile) * 2u : 0u;   // W2: tail_n rows of Ntile channels
       const uint32_t b_dst = smem_u32(smem_b);
+      // merged ConvTranspose: the image holds both row parities; this CTA's items all have parity blockIdx.x & 1 (even grid)
+      const uint8_t* b_src = reinterpret_cast<const uint8_t*>(p.wpack) + (p.upm ? (blockIdx.x & 1u) * bytes : 0u);
       mbar_arrive_expect_tx(bres, bytes + tail_bytes);
       for (uint32_t off = 0; off < bytes; off += 32768u) {
         const uint32_t n = bytes - off < 32768u ? bytes - off : 32768u;
-        bulk_copy_g2s(b_dst + off, reinterpret_cast<const uint8_t*>(p.wpack) + off, n, bres);
+        bulk_copy_g2s(b_dst + off, b_src + off, n, bres);
       }
       if (tail_bytes) bulk_copy_g2s(smem_u32(smem + p.smem_off_w2), p.tail_w, tail_bytes, bres);
     }
@@ -1137,6 +1316,8 @@ conv_halo_tma_kernel(const __grid_constant__ ConvParams p, const __grid_constant
   // bias for the epilogue; activated layers keep 0.5 * bias (epilogue_chunk16_hb: h = 0.5 acc + 0.5 bias in one FFMA)
   for (int i = tid; i < p.n_tiles * p.Ntile; i += TMA_THREADS) bias_s[i] = p.act ? 0.5f * p.bias[i] : p.bias[i];
   for (int i = tid; i < p.tail_n; i += TMA_THREADS) bias_s[256 + i] = p.tail_act ? 0.5f * p.tail_bias[i] : p.tail_bias[i];
+  if (p.upm)   // merged ConvTranspose: the border corrections, added to the accumulator (tma_epilogue_loop_tail)
+    for (int i = tid; i < 9 * 64; i += TMA_THREADS) reinterpret_cast<float*>(smem + p.smem_off_corr)[i] = p.bias[p.n_tiles * p.Ntile + i];
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -1162,7 +1343,7 @@ conv_halo_tma_kernel(const __grid_constant__ ConvParams p, const __grid_constant
       const bool flat = p.mode == MODE_FLAT_TMA;
       const int S = p.S;
       for (int w = blockIdx.x; w < total_work; w += gridDim.x) {
-        const int tile = w >> (p.n_tiles == 4 ? 2 : (p.n_tiles == 2 ? 1 : 0));
+        const int tile = w >> (p.upm ? 1 : (p.n_tiles == 4 ? 2 : (p.n_tiles == 2 ? 1 : 0)));   // upm: (row tile, row parity)
         const int n_tile = w & (p.n_tiles - 1);
         const int b = fd_div(p.fd_hp1, tile);
         const int y0 = (tile - b * p.tpi) * p.R;
@@ -1293,6 +1474,14 @@ conv_halo_tma_kernel(const __grid_constant__ ConvParams p, const __grid_constant
       uint32_t c_sel = static_cast<uint32_t>((p.mode == MODE_HALO_TMA ? 0 : p.mode == MODE_S2_TMA ? 4 : 8) + (kj == 4 ? 2 : kj == 2 ? 1 : 0));
       uint32_t c_bres = p.b_resident ? 1u : 0u;
       const uint32_t c_wp16 = static_cast<uint32_t>(p.Wp) * row16;
+      if (p.upm) {
+        // merged ConvTranspose: warp my_u = 2 u + dx computes column parity dx of sub-tile u for the CTA's row parity dy; its tap
+        // (0, 0) is halo row j + dy Wp + dx - 1, its weights the dx half of the resident stage (four taps)
+        const uint32_t dy = blockIdx.x & 1u, dx = static_cast<uint32_t>(my_u) & 1u;
+        c_a_lo = (((a_u32 >> 4) & 0x3FFFu) | (1u << 16)) + (static_cast<uint32_t>(my_u) >> 1) * sub16 + dy * c_wp16 + dx * row16 - row16;
+        c_b_lo += dx * 4u * tap16;
+        c_sel = 12;
+      }
       const uint32_t c_planex16 = p.pair ? (rb >> 4) : static_cast<uint32_t>(p.lbo_a) >> 4;      // x parity: odd pixel inside the row / one plane buffer
       const uint32_t c_plane16 = p.pair ? static_cast<uint32_t>(p.lbo_a) >> 4 : 2u * (static_cast<uint32_t>(p.lbo_a) >> 4);   // y parity
       const uint32_t c_blk16 = static_cast<uint32_t>(p.slots) * row16;
@@ -1347,6 +1536,7 @@ conv_halo_tma_kernel(const __grid_constant__ ConvParams p, const __grid_constant
                   case 6: issue_taps<1, 4>(d_tmem, a_sub, b_lo, hi_sw, idesc, acc0, row16, tap16, c_wp16, c_plane16, c_blk16, c_kps, hi_a, c_planex16); break;
                   case 8: issue_taps<2, 1>(d_tmem, a_sub, b_lo, hi_sw, idesc, acc0, row16, tap16, c_wp16, c_plane16, c_blk16, c_kps, hi_a, c_planex16); break;
                   case 9: issue_taps<2, 2>(d_tmem, a_sub, b_lo, hi_sw, idesc, acc0, row16, tap16, c_wp16, c_plane16, c_blk16, c_kps, hi_a, c_planex16); break;
+                  case 12: issue_taps<3, 4>(d_tmem, a_sub, b_lo, hi_sw, idesc, acc0, row16, tap16, c_wp16, c_plane16, c_blk16, c_kps, hi_a, c_planex16); break;
                   default: issue_taps<2, 4>(d_tmem, a_sub, b_lo, hi_sw, idesc, acc0, row16, tap16, c_wp16, c_plane16, c_blk16, c_kps, hi_a, c_planex16); break;
                 }
               }
@@ -1403,8 +1593,10 @@ conv_halo_tma_kernel(const __grid_constant__ ConvParams p, const __grid_constant
   } else {
     // ======================================= epilogue ============================================
     // one specialised instantiation per (destination kind, activation, residual): see tma_epilogue_loop
-    if (p.tail_n) {
-      tma_epilogue_loop_tail<PROBE>(p, tmem_base, tfull, tempty, tready, t2full, bias_s, warp, lane, total_work);
+    if (p.tail_n && p.upm) {
+      tma_epilogue_loop_tail<PROBE, true>(p, tmem_base, tfull, tempty, tready, t2full, bias_s, warp, lane, total_work);
+    } else if (p.tail_n) {
+      tma_epilogue_loop_tail<PROBE, false>(p, tmem_base, tfull, tempty, tready, t2full, bias_s, warp, lane, total_work);
     } else {
     const int kind = p.transposed ? 2 : (p.split_n ? 1 : 0);
     const int nch_ = p.Ntile >> 4;
@@ -1444,6 +1636,8 @@ static inline void launch_conv_halo_tma(const ConvParams& p_in, const TmapSet& m
   ConvParams p = p_in;                        // values the kernel would otherwise compute and keep (or spill) per thread
   p.total_work = p.m_tiles * p.n_tiles;
   if (p.nbuf < 2) p.nbuf = 2;
+  if (p.upm) p.grid &= ~1;                    // a CTA's items must share one row parity (its resident weights)
+  XR_CHECK(!p.upm || (p.tail_n && p.grid >= 2), "a merged ConvTranspose launch needs the fused 1x1 tail and an even grid");
 #ifdef XRSEG_DEBUG_API
   if (p.dbg_skip || p.dbg_clk) {   // probe instantiation: only reachable through xrseg_debug_conv
     launch_k(conv_halo_tma_kernel<true>, p.grid, TMA_THREADS, p.smem_bytes, stream, p, maps);

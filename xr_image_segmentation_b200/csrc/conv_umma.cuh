@@ -107,6 +107,10 @@ struct ConvParams {
   int tail_n, tail_act, smem_off_w2;
   const __half* tail_w;             // [32][64] fp16, K-major 128-byte swizzle (pack_conv_weights_sw image of the 1x1 layer)
   const float* tail_bias;           // [32]
+  // ConvTranspose 2x2 / stride 2 merged into this 3x3 (conv_tma.cuh plan_conv_upmerge_tma): H / W are the map BEFORE the
+  // upsampling, Ho / Wo = 2H / 2W.  Virtual sub-tile v = 2 u + dx (u = 128-row sub-tile, dx = output column parity); the row
+  // parity dy of an item is w & 1.  The bias holds [Cout] interior values and nine [Cout] border corrections at smem_off_corr.
+  int upm, smem_off_corr;
 };
 
 struct ConvDesc {
@@ -114,6 +118,7 @@ struct ConvDesc {
   int Cout, out_pitch;
   int k, stride, act, transposed;
   int res_pitch;                    // 0 = no residual
+  int upm;                          // 1: a 2x2 / stride-2 ConvTranspose of this input runs inside the 3x3 (ConvParams::upm)
 };
 
 // ---------------------------------------------------------------------------------------------------------------

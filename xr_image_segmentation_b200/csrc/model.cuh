@@ -49,6 +49,9 @@ struct Op {
   // the kernel; ytail is its destination (y stays the never-materialised intermediate)
   int tail_layer = -1, tail_act = 0;
   TV ytail;
+  // merged leading ConvTranspose 2x2 / stride 2 (fuse_up_conv): x is that layer's input, the 3x3 `layer` runs on the
+  // upsampled map without it ever existing
+  int up_layer = -1;
 };
 
 // Channel triples (input, middle, output; as laid out in shared memory) the fused Bottleneck kernel is built for
@@ -107,12 +110,15 @@ class Net {
   bool fuse_bneck = true;                 // Bottleneck fusion (fuse_bottlenecks)
   bool fuse_pe = true;                    // C2PSA positional encoding inside the attention kernel (fuse_attention_pe)
   bool fuse_tail = true;                  // proto.cv3 (1x1, 64 -> 32) inside proto.cv2's launch (fuse_tail_1x1)
+  bool fuse_up = false;                   // proto.up inside that launch too (fuse_up_conv): requested by the caller, decided in build()
   TV input;                 // [B,640,640,4] fp16
   TV box[3], cls[3], coef[3], protos;
   int fh[3], fw[3];
 
-  Net(int scale, int batch, int in_hw = 640, bool fuse = true, bool bneck = true, int nc = 80)
-      : B(batch), sp(make_spec(scale, nc)), fuse_enabled(fuse), fuse_bneck(fuse && bneck), fuse_tail(fuse) {
+  // up: merge proto.up into proto.cv2's launch where that is supported (fuse_up_conv).  The runner asks for it; the default is the
+  // layer-per-launch list with only the sibling / Bottleneck / attention / tail fusions.
+  Net(int scale, int batch, int in_hw = 640, bool fuse = true, bool bneck = true, int nc = 80, bool up = false)
+      : B(batch), sp(make_spec(scale, nc)), fuse_enabled(fuse), fuse_bneck(fuse && bneck), fuse_tail(fuse), fuse_up(fuse && up) {
     XR_CHECK(nc >= NC_MIN && nc <= NC_MAX, "%d classes: supported are %d..%d", nc, NC_MIN, NC_MAX);
     build(in_hw);
   }
@@ -126,6 +132,24 @@ class Net {
     arena_elems += static_cast<size_t>(B) * H * W * t.pitch;
     arena_elems = (arena_elems + 127) / 128 * 128;
     return t;
+  }
+  // A view that no launch reads or writes (an intermediate a fusion pass removes): shape only, an offset far outside the arena.
+  static constexpr size_t NO_STORAGE = static_cast<size_t>(1) << 60;
+  TV unallocated(int H, int W, int C, int id) const {
+    TV t;
+    t.B = B; t.H = H; t.W = W; t.C = C;
+    t.Cp = t.pitch = round_up(C, 16);
+    t.off = NO_STORAGE + static_cast<size_t>(id) * 128;
+    return t;
+  }
+  int ops_reading_unallocated() const {
+    int n = 0;
+    for (const Op& o : ops) {
+      const bool tail = o.tail_layer >= 0;    // a fused tail's y is its never-materialised intermediate
+      n += o.x.off >= NO_STORAGE || (!tail && o.y.off >= NO_STORAGE) || (o.has_res && o.res.off >= NO_STORAGE) ||
+           (o.layer2 >= 0 && o.y2.off >= NO_STORAGE) || (tail && o.ytail.off >= NO_STORAGE);
+    }
+    return n;
   }
   static TV slice(const TV& t, int c0, int c) {
     XR_CHECK(c0 % 16 == 0 && c % 16 == 0 && c0 + c <= t.Cp, "bad slice %d+%d of %d", c0, c, t.Cp);
@@ -266,9 +290,12 @@ class Net {
   // accumulator columns are all in use).  The stride-2 stage pairs b1 -> b2.cv1 and b3 -> b4.cv1 were measured too: 76 + 43 ->
   // 113 us and 66 + 27 -> 88 us, frames/s unchanged -- these layers are bound by their epilogue, and two epilogue passes in one
   // launch cost what the second launch did.  Anything else keeps its two launches.
+  static bool tail_env_on() {
+    static const bool on = [] { const char* e = getenv("XRSEG_FUSE_TAIL"); return !(e && e[0] == '0'); }();
+    return on;
+  }
   void fuse_tail_1x1() {
-    static const bool env_on = [] { const char* e = getenv("XRSEG_FUSE_TAIL"); return !(e && e[0] == '0'); }();
-    if (!fuse_tail || !env_on) return;
+    if (!fuse_tail || !tail_env_on()) return;
     for (size_t i = 0; i + 1 < ops.size(); ++i) {
       Op& a = ops[i];
       const Op b = ops[i + 1];
@@ -286,6 +313,40 @@ class Net {
       a.signal_tag = b.signal_tag;
       ops.erase(ops.begin() + i + 1);
     }
+  }
+
+  // proto.up (ConvTranspose 2x2 / stride 2, bias, no activation) -> proto.cv2 (3x3, SiLU) is exact linear algebra before the
+  // SiLU: for each output parity (dy, dx) it is a 2x2-tap convolution of the 80x80 map with merged weights (K per output
+  // pixel 256 instead of 576), plus a bias that depends on which of cv2's taps fall inside the 160x160 map (conv_tma.cuh
+  // merge_upconv_weights).  The pair becomes one OP_CONV on the 80x80 map: layer = cv2, up_layer = up, x = up's input.  Only
+  // with the fused proto.cv3 tail (the kernel's parity-scatter epilogue is the tail's) and only for 64 channels (the n scale;
+  // the s scale's 128 would need four N tiles).  build() decides it up front (fuse_up) so that neither 160x160x64 map is
+  // allocated; XRSEG_FUSE_UP=0 (or XRSEG_FUSE_TAIL=0) keeps the three launches.
+  void fuse_up_conv() {
+    if (!fuse_up) return;
+    bool done = false;
+    for (size_t i = 0; i + 1 < ops.size(); ++i) {
+      Op& a = ops[i];
+      const Op b = ops[i + 1];
+      if (a.kind != OP_CONV || b.kind != OP_CONV || layers[a.layer].name != "proto.up" || layers[b.layer].name != "proto.cv2") continue;
+      const bool ok = a.transposed && a.k == 2 && a.stride == 2 && !a.act && !a.has_res && a.layer2 < 0 && a.tail_layer < 0 &&
+                      b.k == 3 && b.stride == 1 && !b.transposed && !b.has_res && b.layer2 < 0 && b.x.off == a.y.off &&
+                      a.x.Cp == 64 && b.y.Cp == 64 && a.y.Cp == 64 && a.branch == b.branch && b.wait_tag == 0 && a.signal_tag == 0;
+      XR_CHECK(ok, "proto.up -> proto.cv2 cannot be merged");
+      for (size_t j = 0; j < ops.size(); ++j)   // up's only consumer is cv2
+        XR_CHECK(j == i || j == i + 1 || (ops[j].x.off != a.y.off && !(ops[j].has_res && ops[j].res.off == a.y.off)),
+                 "proto.up has a second consumer");
+      const int wait = a.wait_tag;
+      ops[i + 1].up_layer = a.layer;
+      ops[i + 1].x = a.x;
+      ops[i + 1].wait_tag = wait;
+      ops.erase(ops.begin() + i);
+      done = true;
+      break;
+    }
+    XR_CHECK(done, "proto.up / proto.cv2 not found for the merge");
+    named.erase("proto.up");                  // never materialised
+    named.erase("proto.cv2");
   }
 
   // C2PSA: x = attention(q, k, v) + pe(v).  The depthwise 3x3 `attn.pe` reads V in place from the qkv tensor and adds the
@@ -415,15 +476,23 @@ class Net {
     head_coef(p5, 2, "h5");
     cur_branch = 4; pending_wait = 3;                // prototype chain: side stream 4, after P3
     t = conv(p3, sp.proto_mid, 3, 1, true, "proto.cv1");
-    t = conv(t, sp.proto_mid, 2, 2, false, "proto.up", nullptr, nullptr, true);
-    t = conv(t, sp.proto_mid, 3, 1, true, "proto.cv2");
+    {
+      // proto.up + proto.cv2 (+ cv3) as one launch (fuse_up_conv): the two 160x160 maps get no storage
+      const char* e = getenv("XRSEG_FUSE_UP");
+      fuse_up = fuse_up && fuse_tail && tail_env_on() && !(e && e[0] == '0') && sp.proto_mid == 64 && t.W + 2 <= 256;
+      TV up_y = unallocated(2 * t.H, 2 * t.W, sp.proto_mid, 0), cv2_y = unallocated(2 * t.H, 2 * t.W, sp.proto_mid, 1);
+      t = conv(t, sp.proto_mid, 2, 2, false, "proto.up", fuse_up ? &up_y : nullptr, nullptr, true);
+      t = conv(t, sp.proto_mid, 3, 1, true, "proto.cv2", fuse_up ? &cv2_y : nullptr);
+    }
     protos = conv(t, 32, 1, 1, true, "proto.cv3");
     cur_branch = 0;
     named["p3"] = p3; named["p4"] = p4; named["p5"] = p5;
     fuse_siblings();
     fuse_bottlenecks();
     fuse_attention_pe();
+    fuse_up_conv();
     fuse_tail_1x1();
+    XR_CHECK(!fuse_up || ops_reading_unallocated() == 0, "a launch touches a tensor without storage");
     fh[0] = p3.H; fw[0] = p3.W; fh[1] = p4.H; fw[1] = p4.W; fh[2] = p5.H; fw[2] = p5.W;
   }
 };

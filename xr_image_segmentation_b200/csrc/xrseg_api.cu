@@ -279,7 +279,9 @@ void upload_layers(xrseg_runner* r, const std::vector<HostLayerWeights>& hw) {
       cd.Cout = o.y.Cp + (o.layer2 >= 0 ? o.y2.Cp : 0); cd.out_pitch = o.y.pitch;
       cd.k = o.k; cd.stride = o.stride; cd.act = o.act; cd.transposed = o.transposed;
       cd.res_pitch = o.has_res ? o.res.pitch : 0;
+      cd.upm = o.up_layer >= 0 ? 1 : 0;
       d.use_tma = r->cfg.conv_impl == XRSEG_CONV_UMMA && plan_conv_halo_tma(cd, r->num_sms, d.cp);
+      XR_CHECK(!cd.upm || d.use_tma, "no launch plan for the merged ConvTranspose (%s)", l.name.c_str());
       if (d.use_tma) {
         d.tmaps.m[0] = make_halo_tensor_map(ptr_of(r, o.x), r->mb, o.x.H, o.x.W, o.x.Cp, o.x.pitch, d.cp.Wp, d.cp.hbox,
                                             d.cp.sw ? d.cp.cb : 8, d.cp.sw);
@@ -319,7 +321,18 @@ void upload_layers(xrseg_runner* r, const std::vector<HostLayerWeights>& hw) {
         std::vector<__half> wp;
         std::vector<float> bp;
         XR_CHECK(o.layer2 < 0 || (d.use_tma && d.cp.sw), "fused siblings need the TMA kernel (%s)", l.name.c_str());
-        if (d.use_tma && d.cp.sw) pack_conv_weights_sw<__half>(d.cp, wsrc.w.data(), wsrc.b.data(), l.cin, cout_real, wp, bp);
+        if (o.up_layer >= 0) {
+          // merged ConvTranspose (model.cuh fuse_up_conv): parity weights and border biases from the dequantized fp32 weights in
+          // fp64, each weight rounded to fp16 once; bias = [64 interior | 9 x 64 border corrections]
+          const LayerRec& lu = net.layers[o.up_layer];
+          const HostLayerWeights& wu = hw[o.up_layer];
+          XR_CHECK(lu.cin == 64 && lu.cout == l.cin && l.cout == 64 && !w.b.empty() && !wu.b.empty(),
+                   "merged ConvTranspose: unexpected shapes (%s)", l.name.c_str());
+          std::vector<double> wm, bm;
+          merge_upconv_weights(wu.w.data(), wu.b.data(), w.w.data(), w.b.data(), lu.cin, lu.cout, l.cout, wm, bm);
+          pack_upmerge_weights_sw(d.cp, wm, lu.cin, l.cout, wp);
+          bp.assign(bm.begin(), bm.end());
+        } else if (d.use_tma && d.cp.sw) pack_conv_weights_sw<__half>(d.cp, wsrc.w.data(), wsrc.b.data(), l.cin, cout_real, wp, bp);
         else pack_conv_weights<__half>(d.cp, wsrc.w.data(), wsrc.b.data(), l.cin, cout_real, wp, bp);
         d.wpack = dev_upload(wp);
         d.bias = dev_upload(bp);
@@ -422,8 +435,11 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
           L.name = l.name + "+" + net.layers[o.layer2].name.substr(net.layers[o.layer2].name.find('.') + 1);
           if (L.name.size() > 31) L.name.resize(31);
         }
-        L.flops = 2.0 * (o.transposed ? px_in * 4 : px_out) * cout_alg * l.cin * taps;
-        L.bytes = (px_in * l.cin + px_out * cout_alg * (o.has_res ? 2 : 1) + static_cast<double>(cout_alg) * l.cin * o.k * o.k) * 2;
+        // merged ConvTranspose: 4 taps per output pixel, weights of four parities x four taps
+        const bool upm = o.up_layer >= 0;
+        const double wtaps = upm ? 16.0 : static_cast<double>(o.k) * o.k;
+        L.flops = 2.0 * (o.transposed ? px_in * 4 : px_out) * cout_alg * l.cin * (upm ? 4.0 : taps);
+        L.bytes = (px_in * l.cin + px_out * cout_alg * (o.has_res ? 2 : 1) + static_cast<double>(cout_alg) * l.cin * wtaps) * 2;
         if (r->cfg.conv_impl == XRSEG_CONV_UMMA) {
           ConvParams p = d.cp;
           if (nb != p.B) p = replan_for_batch(d.cp, nb, r->num_sms);   // partial last chunk: same layout, fewer frames
@@ -453,8 +469,9 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
             p.out = ptr_of(r, o.ytail); p.out_pitch = o.ytail.pitch;
             p.tail_w = r->dl[o.tail_layer].tail_w; p.tail_bias = r->dl[o.tail_layer].tail_bias;
             L.name = l.name + "+" + lt.name.substr(lt.name.find('.') + 1);
+            if (upm) L.name = net.layers[o.up_layer].name + "+" + L.name.substr(L.name.find('.') + 1);   // "proto.up+cv2+cv3"
             L.flops += 2.0 * px_out * lt.cout * lt.cin;
-            L.bytes = (px_in * l.cin + px_out * lt.cout + static_cast<double>(cout_alg) * l.cin * o.k * o.k + static_cast<double>(lt.cout) * lt.cin) * 2;
+            L.bytes = (px_in * l.cin + px_out * lt.cout + static_cast<double>(cout_alg) * l.cin * wtaps + static_cast<double>(lt.cout) * lt.cin) * 2;
           }
           if (d.use_tma) {
             const TmapSet maps = d.tmaps;
@@ -1250,7 +1267,7 @@ int xrseg_create(const xrseg_config* cfg_in, xrseg_runner** out) {
     const char* fuse_env = getenv("XRSEG_FUSE");
     const bool fuse = c.conv_impl == XRSEG_CONV_UMMA && !(fuse_env && fuse_env[0] == '0');
     const char* bneck_env = getenv("XRSEG_FUSE_BNECK");
-    r->net.reset(new Net(c.model_scale, r->mb, 640, fuse, !(bneck_env && bneck_env[0] == '0'), r->nc));
+    r->net.reset(new Net(c.model_scale, r->mb, 640, fuse, !(bneck_env && bneck_env[0] == '0'), r->nc, true));
     Net& net = *r->net;
     r->A = net.fh[0] * net.fw[0] + net.fh[1] * net.fw[1] + net.fh[2] * net.fw[2];
     std::vector<HostLayerWeights> hw;
