@@ -14,8 +14,13 @@
 extern "C" {
 #endif
 
-/* Copy a named intermediate activation of the last run to host as f32 NCHW [batch,C,H,W].
- * names: "p3","p4","p5","box_logits","cls_logits","coefs","protos","input" and every layer name. */
+/* Copy a named intermediate activation of the last run to host as f32 NCHW [n,C,H,W].
+ * names: "p3","p4","p5","box_logits.i","cls_logits.i","coefs.i" (i = 0..2),"protos","input", every layer name, and the
+ * outputs of the copy / max-pool launches: "b9.pool" (the three chained SPPF max-pools), "up.13" / "up.16" (the nearest
+ * x2 upsamples feeding n13 / n16).
+ * A run of batch > micro_batch computes its frames in chunks of micro_batch that reuse one activation arena, so only the
+ * LAST chunk is resident: the fetched frames are (ceil(batch / micro_batch) - 1) * micro_batch .. batch - 1, and
+ * shape4[0] = n is their count.  A zero-capacity call reports the shape and returns XRSEG_ERR_CAPACITY. */
 int xrseg_debug_fetch(xrseg_runner* r, const char* name, float* dst, size_t cap_floats, int64_t* shape4);
 /* Run ONLY the post-processing stage on caller-provided fp32 head tensors (the oracle's own tensors):
  * box_logits [batch,A,64], cls_logits [batch,A,nc] (nc = the runner's xrseg_num_classes), coefs [batch,A,32],

@@ -2,6 +2,8 @@
 //   nvcc -std=c++17 -gencode arch=compute_100a,code=sm_100a --expt-relaxed-constexpr -o /tmp/plan_dump tools/plan_dump.cu -lcuda
 //   /tmp/plan_dump [batch] [n|s] [ops] [up] [num_classes]
 //   up: the runner's launch list, with proto.up merged into proto.cv2's launch (model.cuh fuse_up_conv)
+//   The launch list follows the fusion switches the runner reads at create time: XRSEG_FUSE, XRSEG_FUSE_BNECK (read here as
+//   xrseg_create reads them), XRSEG_FUSE_PE, XRSEG_FUSE_TAIL and XRSEG_FUSE_UP (read by model.cuh itself).
 #include <math.h>
 #include <string.h>
 #include "../xr_image_segmentation_b200/csrc/conv_tma.cuh"
@@ -18,7 +20,9 @@ int main(int argc, char** argv) {
     else nc = atoi(argv[i]);
   }
   if (ops) {   // "ops": the fused launch list (one line per network launch) instead of the conv plans
-    Net fused(scale, B, 640, true, true, nc, up);
+    const char* fuse_env = getenv("XRSEG_FUSE");
+    const char* bneck_env = getenv("XRSEG_FUSE_BNECK");
+    Net fused(scale, B, 640, !(fuse_env && fuse_env[0] == '0'), !(bneck_env && bneck_env[0] == '0'), nc, up);
     const char* kind_name[] = {"stem", "conv", "dw", "sppf", "up", "attn", "bneck"};
     for (const Op& o : fused.ops) {
       std::string name = o.layer >= 0 ? fused.layers[o.layer].name : std::string("-");
@@ -26,6 +30,7 @@ int main(int argc, char** argv) {
       printf("op %-6s %-28s in %3dx%-3d c%-3d out c%-3d res %d branch %d\n", kind_name[o.kind], name.c_str(), o.x.H, o.x.W, o.x.Cp,
              o.y.Cp, o.has_res ? 1 : 0, o.branch);
       if (o.kind == OP_CONV && o.up_layer >= 0) printf("   (merged: %s runs inside this launch)\n", fused.layers[o.up_layer].name.c_str());
+      if (o.kind == OP_CONV && o.tail_layer >= 0) printf("   (tail: %s runs inside this launch)\n", fused.layers[o.tail_layer].name.c_str());
     }
     return 0;
   }

@@ -60,6 +60,12 @@ static inline bool bneck_supported(int c1, int cm, int c2) {
   return (c1 == 16 && cm == 8 && c2 == 16) || (c1 == 32 && cm == 16 && c2 == 32);
 }
 
+// XRSEG_FLAT_TMA=0: keep the 1x1 convolutions on the thread-gather kernel (A/B measurements only)
+static inline bool flat_tma_disabled() {
+  const char* e = getenv("XRSEG_FLAT_TMA");
+  return e && e[0] == '0';
+}
+
 struct Spec {
   int ch[5];
   int mid0, mid1;     // C3k2 output widths of layers 2 / 4 (n: 64 / 128)
@@ -262,6 +268,8 @@ class Net {
     for (const auto& pr : pairs) {
       const int ia = find(pr.first), ib = find(pr.second);
       if (ia < 0 || ib < 0) continue;
+      // a fused pair needs a TMA plan (xrseg_api.cu upload_layers): with the flat TMA planner off, 1x1 pairs keep two launches
+      if (ops[ia].k == 1 && flat_tma_disabled()) continue;
       Op& a = ops[ia];
       const Op b = ops[ib];
       const bool same = a.kind == OP_CONV && b.kind == OP_CONV && a.x.off == b.x.off && a.x.C == b.x.C && a.x.pitch == b.x.pitch &&
@@ -423,6 +431,7 @@ class Net {
       TV cat = alloc(h32, h32, 4 * c_);
       TV y0 = slice(cat, 0, c_);
       conv(t, c_, 1, 1, true, "b9.cv1", &y0);
+      named["b9.pool"] = slice(cat, c_, 3 * c_);   // fetch-only name: the three max-pool outputs
       Op o;
       o.kind = OP_SPPF;
       o.x = cat; o.y = cat;
@@ -449,15 +458,16 @@ class Net {
       conv(f, c, 1, 1, false, "b10.ffn.1", &b, &b);                  // b += ffn(b)
       conv(cat, c5, 1, 1, true, "b10.cv2", &f10);
     }
-    auto upsample = [&](const TV& src, const TV& dst) {
+    auto upsample = [&](const TV& src, const TV& dst, const char* name) {
       Op o;
       o.kind = OP_UP; o.x = src; o.y = dst;
       ops.push_back(o);
+      named[name] = dst;                        // fetch-only name of the concat slice it fills
     };
-    upsample(f10, slice(cat13, 0, c5));
+    upsample(f10, slice(cat13, 0, c5), "up.13");
     TV f13 = slice(cat19, sp.mid0, sp.mid1);
     c3k2(cat13, sp.mid1, sp.mid1 / 2, false, "n13", &f13);
-    upsample(f13, slice(cat16, 0, sp.mid1));
+    upsample(f13, slice(cat16, 0, sp.mid1), "up.16");
     TV p3 = c3k2(cat16, sp.mid0, sp.mid0 / 2, false, "n16");
     ops.back().signal_tag = 3;
     head_box_cls(p3, 0, "h3");

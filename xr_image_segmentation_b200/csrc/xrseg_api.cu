@@ -71,12 +71,6 @@ void launch_bneck(int c1, int cm, int c2, const BneckParams& p, bool res, cudaSt
   else XR_CHECK(false, "no fused Bottleneck kernel for %d-%d-%d channels", c1, cm, c2);
 }
 
-// XRSEG_FLAT_TMA=0: keep the 1x1 convolutions on the thread-gather kernel (A/B measurements only)
-bool flat_tma_disabled() {
-  const char* e = getenv("XRSEG_FLAT_TMA");
-  return e && e[0] == '0';
-}
-
 bool branches_disabled() {   // XRSEG_BRANCHES=0: everything on one stream (A/B measurements)
   const char* e = getenv("XRSEG_BRANCHES");
   return e && e[0] == '0';
@@ -1821,7 +1815,8 @@ int xrseg_debug_fetch(xrseg_runner* r, const char* name, float* dst, size_t cap_
     t = it->second;
   }
   C = t.C;
-  const int nb = std::min(r->batch, r->mb);
+  // the arena holds the LAST micro-batch of the run: frames (n_chunks - 1) * mb .. batch - 1
+  const int nb = r->batch > 0 ? r->batch - (ceil_div(r->batch, r->mb) - 1) * r->mb : 0;
   const size_t n = static_cast<size_t>(nb) * C * t.H * t.W;
   if (shape4) { shape4[0] = nb; shape4[1] = C; shape4[2] = t.H; shape4[3] = t.W; }
   if (cap_floats < n) { r->err = "fetch buffer too small"; return XRSEG_ERR_CAPACITY; }
