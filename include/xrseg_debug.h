@@ -29,7 +29,8 @@ int xrseg_debug_post(xrseg_runner* r, const float* box_logits, const float* cls_
                      const float* protos, int batch);
 /* Same tensors through the PRODUCT kernels: rounded to fp16 on the device (prototypes re-laid out NHWC like the network's),
  * then the streaming decode filter, NMS and the mma.sync mask assembly of the per-frame path (tools/bench_post.py:
- * BASELINE.json configs[4], the post-processing stress shape). */
+ * BASELINE.json configs[4], the post-processing stress shape).  XRSEG_MASK_UPSAMPLE_640 then reads these prototypes; after
+ * xrseg_debug_post (fp32, planar) it returns XRSEG_ERR_STATE. */
 int xrseg_debug_post_f16(xrseg_runner* r, const float* box_logits, const float* cls_logits, const float* coefs,
                          const float* protos, int batch);
 /* Per-launch CUDA-event times of the last xrseg_debug_post* call made with XRSEG_DBG_TIME=1 in the environment

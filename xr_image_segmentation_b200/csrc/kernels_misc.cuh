@@ -46,8 +46,10 @@ __global__ void preprocess_kernel(const PreParams p) {
     inside = (xx >= 0 && xx < p.nw && yy >= 0 && yy < p.nh);
   }
   if (inside) {
-    const float fx = (static_cast<float>(xx) + 0.5f) * p.scale_x - 0.5f;
-    const float fy = (static_cast<float>(yy) + 0.5f) * p.scale_y - 0.5f;
+    // two roundings in the oracle's order (oracle/preprocess._axis); left to nvcc, the product and the subtraction contract
+    // into one FFMA
+    const float fx = __fsub_rn(__fmul_rn(static_cast<float>(xx) + 0.5f, p.scale_x), 0.5f);
+    const float fy = __fsub_rn(__fmul_rn(static_cast<float>(yy) + 0.5f, p.scale_y), 0.5f);
     const float x0f = floorf(fx), y0f = floorf(fy);
     const float tx = fx - x0f, ty = fy - y0f;
     int x0 = static_cast<int>(x0f), y0 = static_cast<int>(y0f);

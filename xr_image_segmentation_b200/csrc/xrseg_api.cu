@@ -183,7 +183,15 @@ struct xrseg_runner {
   // fused preprocess + stem: set by do_schedule when the frames are 640x640 (no resample), consumed by OP_STEM
   const uint8_t* fused_src = nullptr;
   int fused_stride = 0, fused_bpp = 0, fused_flip = 0;
-  int* h_overflow = nullptr;          // pinned: bit 0 = more candidates than max_candidates, bit 1 = more kept boxes than max_det
+  // NHWC fp16 prototypes the last post-processing stage read, which xrseg_masks' 640-px mode reads again: the network arena
+  // after xrseg_schedule*, the caller's tensors after xrseg_debug_post_f16.  ptr == nullptr: none usable, `why` says why.
+  struct ProtoSrc {
+    const __half* ptr = nullptr;
+    long bstride = 0;
+    int pitch = 0;
+    const char* why = "no run scheduled";
+  } mask_protos;
+  int* h_overflow = nullptr;         // pinned: bit 0 = more candidates than max_candidates, bit 1 = more kept boxes than max_det
 
   ~xrseg_runner();
 };
@@ -906,6 +914,11 @@ int do_schedule(xrseg_runner* r, const uint8_t* src, bool src_on_device, int w, 
       d_src = r->d_frames;
     }
     r->batch = batch;
+    const TV& pr = r->net->protos;
+    if (batch > r->mb)
+      r->mask_protos = {nullptr, 0, 0, "640-px masks need the prototypes of every frame resident: use micro_batch >= batch"};
+    else
+      r->mask_protos = {ptr_of(r, pr), static_cast<long>(pr.H) * pr.W * pr.pitch, pr.pitch, nullptr};
     r->timed = !r->cfg.use_cuda_graph;
     if (r->timed) XR_CUDA(cudaEventRecord(r->ev[0], st));
     reset_counters(r, batch, st);
@@ -1523,8 +1536,8 @@ static int masks_enqueue(xrseg_runner* r, const xrseg_mask_params* mp, uint8_t* 
   try {
     XR_CUDA(cudaSetDevice(r->device));
     uint8_t* d_out = static_cast<uint8_t*>(ensure_scratch(r, per * count));
-    if (mp->mode == XRSEG_MASK_UPSAMPLE_640 && r->batch > r->mb) {
-      r->err = "640-px masks need the prototypes of every frame resident: use micro_batch >= batch";
+    if (mp->mode == XRSEG_MASK_UPSAMPLE_640 && !r->mask_protos.ptr) {
+      r->err = r->mask_protos.why;
       return XRSEG_ERR_STATE;
     }
     // gridDim.y / .z hold the detection index: at most 65535 per launch (batch 512 x 300 detections = 153600)
@@ -1532,8 +1545,7 @@ static int masks_enqueue(xrseg_runner* r, const xrseg_mask_params* mp, uint8_t* 
       const int n = std::min(65535, count - s0);
       uint8_t* slice_out = d_out + per * s0;
       if (mp->mode == XRSEG_MASK_UPSAMPLE_640) {
-        const TV& pr = r->net->protos;
-        Mask640Params p{ptr_of(r, pr), static_cast<long>(pr.H) * pr.W * pr.pitch, pr.pitch, r->o_coefs, r->o_boxes,
+        Mask640Params p{r->mask_protos.ptr, r->mask_protos.bstride, r->mask_protos.pitch, r->o_coefs, r->o_boxes,
                         r->o_frame, first + s0, slice_out,
                         thr <= 0.f ? -3.0e38f : (thr >= 1.f ? 3.0e38f : logf(thr / (1.f - thr)))};
         if (thr == 0.5f) p.logit_thr = 0.f;
@@ -1879,7 +1891,9 @@ static int debug_post_impl(xrseg_runner* r, const float* box_logits, const float
       ScaleSrc<__half> src[3];
       dense_scale_src<__half>(r, src, hb, hc, hm);
       add_post_launches<__half, false>(r, 0, batch, src, hp, static_cast<long>(NM) * PROTO_PIX, NM, true, false, ls);
+      r->mask_protos = {hp, static_cast<long>(NM) * PROTO_PIX, NM, nullptr};
     } else {
+      r->mask_protos = {nullptr, 0, 0, "640-px masks after xrseg_debug_post: its prototypes are fp32 planar, use xrseg_debug_post_f16"};
       ScaleSrc<float> src[3];
       dense_scale_src<float>(r, src, r->dbg_box, r->dbg_cls, r->dbg_coef);
       add_post_launches<float, true>(r, 0, batch, src, r->dbg_proto, static_cast<long>(NM) * PROTO_PIX, 0, true, false, ls);

@@ -105,25 +105,31 @@ class Runner:
             raise XrsegError(_lib.ERR_STATE, "parity hook: create the Runner with debug=True (libxrseg_debug.so)")
 
     # ---- per-frame path ----
-    def schedule(self, frames: np.ndarray, fmt=None, bottom_up=False):
+    def schedule(self, frames: np.ndarray, fmt=None, bottom_up=False, stride_bytes=None):
         """frames uint8 [B,H,W,3|4] (host).  Asynchronous.  bottom_up: memory row 0 is the BOTTOM of the picture (Unity's
-        GetPixels32 order, XRSEG_FMT_BOTTOM_UP)."""
-        assert frames.dtype == np.uint8 and frames.ndim == 4 and frames.flags.c_contiguous
+        GetPixels32 order, XRSEG_FMT_BOTTOM_UP).  stride_bytes: row pitch of padded rows (default w * c); frames is then a
+        view whose rows lie stride_bytes apart and whose frames lie h * stride_bytes apart."""
+        assert frames.dtype == np.uint8 and frames.ndim == 4
         b, h, w, c = frames.shape
+        stride_bytes = w * c if stride_bytes is None else stride_bytes
+        want = (h * stride_bytes, stride_bytes, c, 1)
+        assert all(n == 1 or s == t for n, s, t in zip(frames.shape, frames.strides, want)), (frames.strides, stride_bytes)
         fmt = (_lib.FMT_RGBA8 if c == 4 else _lib.FMT_RGB8) if fmt is None else fmt
         if bottom_up:
             fmt |= _lib.FMT_BOTTOM_UP
         self._keep = frames
         self.batch = b
-        self._ck(self.lib.xrseg_schedule(self.h, frames.ctypes.data, w, h, w * c, fmt, b))
+        self._ck(self.lib.xrseg_schedule(self.h, frames.ctypes.data, w, h, stride_bytes, fmt, b))
 
     def schedule_ptr(self, host_ptr: int, b, h, w, c):
         self.batch = b
         self._ck(self.lib.xrseg_schedule(self.h, host_ptr, w, h, w * c, _lib.FMT_RGBA8 if c == 4 else _lib.FMT_RGB8, b))
 
-    def schedule_device(self, dev_ptr: int, b, h, w, c):
+    def schedule_device(self, dev_ptr: int, b, h, w, c, stride_bytes=None):
+        """dev_ptr: frames already on the runner's GPU, rows stride_bytes apart (default w * c), frames h * stride_bytes apart."""
         self.batch = b
-        self._ck(self.lib.xrseg_schedule_device(self.h, dev_ptr, w, h, w * c, _lib.FMT_RGBA8 if c == 4 else _lib.FMT_RGB8, b))
+        stride_bytes = w * c if stride_bytes is None else stride_bytes
+        self._ck(self.lib.xrseg_schedule_device(self.h, dev_ptr, w, h, stride_bytes, _lib.FMT_RGBA8 if c == 4 else _lib.FMT_RGB8, b))
 
     def poll(self) -> int:
         return self._ck(self.lib.xrseg_poll(self.h))
