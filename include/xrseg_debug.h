@@ -22,6 +22,16 @@ extern "C" {
  * LAST chunk is resident: the fetched frames are (ceil(batch / micro_batch) - 1) * micro_batch .. batch - 1, and
  * shape4[0] = n is their count.  A zero-capacity call reports the shape and returns XRSEG_ERR_CAPACITY. */
 int xrseg_debug_fetch(xrseg_runner* r, const char* name, float* dst, size_t cap_floats, int64_t* shape4);
+/* Same as xrseg_debug_fetch, for `count` frames starting at frame `first` of the resident chunk (first = 0 is its first
+ * frame; count = -1: to its end).  At large batches a whole layer is gigabytes of fp32: a test that checks a few frames
+ * copies only those.  Frames outside the resident chunk: XRSEG_ERR_INVALID. */
+int xrseg_debug_fetch_frames(xrseg_runner* r, const char* name, int first, int count, float* dst, size_t cap_floats,
+                             int64_t* shape4);
+/* The launch list of the last run's resident (last) chunk, in launch order: per launch the CTAs of its grid, its work items
+ * and, for a convolution on the tcgen05 engine, its mode (conv_umma.cuh MODE_*; -1 for every other launch).  grid and items
+ * are 0 for the stem, whose kernel is chosen when it is launched.  names: cap * 32 bytes (may be NULL).  Returns the number
+ * of launches, XRSEG_ERR_CAPACITY when cap is smaller. */
+int xrseg_debug_launches(xrseg_runner* r, int* grid, int* items, int* mode, char* names, int cap);
 /* Run ONLY the post-processing stage on caller-provided fp32 head tensors (the oracle's own tensors):
  * box_logits [batch,A,64], cls_logits [batch,A,nc] (nc = the runner's xrseg_num_classes), coefs [batch,A,32],
  * protos [batch,32,160*160]. */

@@ -113,9 +113,10 @@ class LocalCheck(Y._ConvFeed):
     """Teacher-forced float64 reference.  provider(name) -> float64 tensor [F,C,H,W] of the sampled frames (the GPU's tensor);
     provider None simulates a GPU that stores every checked value rounded to fp16 (`synth` keeps those tensors)."""
 
-    def __init__(self, weights, provider, fusion: Fusion, heads: int):
+    def __init__(self, weights, provider, fusion: Fusion, heads: int, targets: set[str] | None = None):
         super().__init__(weights=weights)
         self.provider = provider
+        self.targets = targets                          # None: check every tensor; else only these (see __call__)
         self.fu = fusion
         self.heads = heads
         self.results: dict[str, dict] = {}
@@ -150,6 +151,12 @@ class LocalCheck(Y._ConvFeed):
                            f"({int(bad.sum())} of {ratio.numel()} elements out of bound)")
         self.results[name] = res
 
+    def _stored(self, name):
+        """The GPU stores this layer's own output under its name, unchanged by a later launch: targets mode may take it as
+        is.  Not so for a fused Bottleneck's cv1 (shared memory), the C2PSA block's in-place chain and attention, and the
+        prototype launches whose intermediates never leave the SM."""
+        return name not in self.fu.bneck_cv1 and not name.startswith("b10.") and not name.startswith("proto.")
+
     # ---- arithmetic ----
     def _w(self, name, w):
         w = torch.as_tensor(w)
@@ -168,10 +175,14 @@ class LocalCheck(Y._ConvFeed):
             return super().__call__(x, cout, k, s, act, groups, transposed, name)
         w, b = self.weights[self.i]
         self.i += 1
+        self.last_in[name] = x
+        if self.targets is not None and name not in self.targets and self._stored(name):
+            self.pending.pop(name, None)
+            gpu = self.provider(name)
+            return gpu - self.last_in[name[:-1] + "1"] if name in RESIDUAL else gpu
         w, b = self._w(name, w), torch.as_tensor(b).double()
         conv = lambda xx, ww, bb: self._conv(xx, ww, bb, s, k, groups, transposed)   # noqa: E731
         K = (x.shape[1] // groups) * (1 if transposed else k * k)
-        self.last_in[name] = x
         z = conv(x, w, b)
         S = conv(x.abs(), w.abs(), b.abs())
         ref = Y.silu(z) if act else z
@@ -294,9 +305,10 @@ def parity_conv(x, wms):
     return out
 
 
-def run_reference(weights, sp: Y.Spec, fusion: Fusion, provider, x):
-    """One teacher-forced pass plus the bit-exact checks of the copy / max kernels.  Returns the LocalCheck."""
-    chk = LocalCheck(weights, provider, fusion, sp.heads)
+def run_reference(weights, sp: Y.Spec, fusion: Fusion, provider, x, targets: set[str] | None = None):
+    """One teacher-forced pass plus the bit-exact checks of the copy / max kernels.  Returns the LocalCheck.  targets: check
+    only these tensors (LocalCheck targets mode)."""
+    chk = LocalCheck(weights, provider, fusion, sp.heads, targets)
     feed = _Hook(chk)
     with torch.no_grad():
         Y.forward_raw(x, feed, sp, taps=feed.taps)
@@ -349,6 +361,32 @@ def failures(chk: LocalCheck) -> list[str]:
 
 
 # ---- launch-list coverage ---------------------------------------------------------------------------------------------
+def launch_tensors(o: dict, ups: int) -> tuple[list[str], set[str]] | None:
+    """(layers computed by launch o, tensors the checker compares for it); ups = nearest-upsample launches before it.
+    None for an unknown launch kind."""
+    kind, name = o["kind"], o["name"]
+    if kind in ("stem", "conv", "dw"):
+        layers = name.split("+")                         # sibling fusion: "b6.m0.cv1+b6.m0.cv2"
+        if o["tail"]:
+            layers.append(o["tail"])
+        if o["merged"]:
+            layers.append(o["merged"])
+        # hidden and in-place outputs are checked through the tensor that carries them
+        keys = {"b10.attn.proj": "b10.ffn.1"}
+        if o["tail"]:
+            keys.update({"proto.up": "proto.cv3", "proto.cv2": "proto.cv3"})
+        return layers, {keys.get(l, l) for l in layers}
+    if kind == "bneck":
+        return [name, name[:-1] + "2"], {name[:-1] + "2"}
+    if kind == "attn":
+        return ([name] if name != "-" else []), {"b10.attn.pe"}   # attention alone (pe unfused): through pe's residual
+    if kind == "sppf":
+        return [], {"b9.pool"}
+    if kind == "up":
+        return [], {("up.13", "up.16")[ups]}
+    return None
+
+
 def launch_coverage(ops: list[dict], checked: set[str], layer_names: list[str]) -> list[str]:
     """Every launch of the op list maps to at least one checked tensor, and every layer is computed by a checked launch.
     Returns the problems (empty: covered)."""
@@ -356,31 +394,12 @@ def launch_coverage(ops: list[dict], checked: set[str], layer_names: list[str]) 
     ups = 0
     for o in ops:
         kind, name = o["kind"], o["name"]
-        if kind in ("stem", "conv", "dw"):
-            layers = name.split("+")                     # sibling fusion: "b6.m0.cv1+b6.m0.cv2"
-            if o["tail"]:
-                layers.append(o["tail"])
-            if o["merged"]:
-                layers.append(o["merged"])
-            # hidden and in-place outputs are checked through the tensor that carries them
-            keys = {"b10.attn.proj": "b10.ffn.1"}
-            if o["tail"]:
-                keys.update({"proto.up": "proto.cv3", "proto.cv2": "proto.cv3"})
-            tensors = {keys.get(l, l) for l in layers}
-        elif kind == "bneck":
-            layers = [name, name[:-1] + "2"]
-            tensors = {layers[1]}
-        elif kind == "attn":
-            layers = [name] if name != "-" else []
-            tensors = {"b10.attn.pe"}                    # attention alone (pe unfused) is checked through pe's residual
-        elif kind == "sppf":
-            layers, tensors = [], {"b9.pool"}
-        elif kind == "up":
-            layers, tensors = [], {("up.13", "up.16")[ups]}
-            ups += 1
-        else:
+        lt = launch_tensors(o, ups)
+        ups += kind == "up"
+        if lt is None:
             problems.append(f"unknown launch kind {kind} ({name})")
             continue
+        layers, tensors = lt
         missing = tensors - checked
         if not tensors or missing:
             problems.append(f"launch {kind} {name}: no checked tensor ({sorted(missing)})")

@@ -111,6 +111,8 @@ PRODUCT_SIGNATURES = {
 # include/xrseg_debug.h: exported by libxrseg_debug.so only
 DEBUG_SIGNATURES = {
     "xrseg_debug_fetch": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_size_t, _P(C.c_int64)]),
+    "xrseg_debug_fetch_frames": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int, C.c_int, C.c_void_p, C.c_size_t, _P(C.c_int64)]),
+    "xrseg_debug_launches": (C.c_int, [C.c_void_p, _P(C.c_int), _P(C.c_int), _P(C.c_int), C.c_char_p, C.c_int]),
     "xrseg_debug_post": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "xrseg_debug_post_f16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "xrseg_debug_nms": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int]),

@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "conv_tma.cuh"
 #include "conv_umma.cuh"
 
 namespace xrseg {
@@ -83,6 +84,14 @@ static inline int class_pitch(int nc) {
   int nt = 1;
   while (round_up(ceil_div(nc, nt), 16) > 256) nt *= 2;
   return nt * round_up(ceil_div(nc, nt), 16);
+}
+
+// The post-processing decode filter of a class tensor (xrseg_api.cu add_post_launches, tools/plan_dump sig): the kernel
+// specialised for 80 classes (post.cuh NC), the segment-table kernel while a class row is at most 32 chunks of epc elements
+// (16 bytes each), else the wide kernel.
+enum { DECODE_80, DECODE_TABLE, DECODE_WIDE };
+static inline int decode_variant(int nc, int pitch, int epc) {
+  return nc == 80 ? DECODE_80 : (pitch / epc <= 32 ? DECODE_TABLE : DECODE_WIDE);
 }
 
 static inline Spec make_spec(int scale, int nc = 80) {
@@ -506,6 +515,56 @@ class Net {
     fh[0] = p3.H; fw[0] = p3.W; fh[1] = p4.H; fw[1] = p4.W; fh[2] = p5.H; fw[2] = p5.W;
   }
 };
+
+// ---------------------------------------------------------------------------------------------------------------
+// A convolution launch's parameters.  The runner (xrseg_api.cu) and tools/plan_dump both derive them here, so that a
+// listing of the plans cannot drift from what the runner launches.
+// ---------------------------------------------------------------------------------------------------------------
+// XRSEG_S2_TMA=0: keep the stride-2 3x3 convolutions on the thread-gather kernel (A/B measurements only)
+static inline bool s2_tma_disabled() {
+  const char* e = getenv("XRSEG_S2_TMA");
+  return e && e[0] == '0';
+}
+
+// The plan of conv op `o` for micro-batch mb on the tcgen05 engine: the halo TMA planner (which also takes the merged
+// ConvTranspose), else the flat one (1x1 and ConvTranspose 2x2), else the stride-2 one, else the thread-gather kernel.
+// Returns true for a TMA plan.
+static inline bool plan_conv_op(const Op& o, int mb, int num_sms, ConvParams& p) {
+  ConvDesc cd{};
+  cd.B = mb; cd.H = o.x.H; cd.W = o.x.W; cd.Cin = o.x.Cp; cd.in_pitch = o.x.pitch;
+  cd.Cout = o.y.Cp + (o.layer2 >= 0 ? o.y2.Cp : 0); cd.out_pitch = o.y.pitch;
+  cd.k = o.k; cd.stride = o.stride; cd.act = o.act; cd.transposed = o.transposed;
+  cd.res_pitch = o.has_res ? o.res.pitch : 0;
+  cd.upm = o.up_layer >= 0 ? 1 : 0;
+  if (plan_conv_halo_tma(cd, num_sms, p)) return true;
+  if (!flat_tma_disabled() && plan_conv_flat_tma(cd, num_sms, p)) return true;
+  if (!s2_tma_disabled() && plan_conv_s2_tma(cd, num_sms, p)) return true;
+  p = plan_conv(cd, num_sms, 0);
+  return false;
+}
+
+// The parameters one launch of a layer planned by plan_conv_op runs with, for a chunk of nb frames: a partial last chunk
+// keeps the plan's layout with fewer frames (replan_for_batch), then a small TMA launch gets at most half the SMs.
+static inline ConvParams conv_launch_params(const ConvParams& plan, bool tma, int nb, int num_sms) {
+  ConvParams p = plan;
+  if (nb != p.B) p = replan_for_batch(plan, nb, num_sms);
+  // Small launches use at most HALF the SMs (XRSEG_TINY_GRID=0 turns it off): 3x3 layers with at most two work items
+  // per SM (296: every 20x20 layer, the 3x3 convs of the 40x40 stage) and 1x1 layers with at most 800 items (the 40x40
+  // stage).  These kernels are latency-bound -- most of their ~10 us is fill
+  // and drain -- and a throughput caller keeps several runners in flight: with half-width grids the small kernels of
+  // two steps sit side by side on disjoint SMs instead of taking turns on all of them.  Measured (B200, batch 64, four
+  // runners, profiles/r2_experiments.md): 34.5k -> 36.7k frames/s, e2e 32.4k -> 34.0k; one runner alone 30.2k -> 29.9k;
+  // batch-1 latency unchanged (its grids are smaller than the cap anyway).
+  // Tensor-heavy layers stay at half width too: keeping them on all SMs (b7: 256 items of 72 N = 256 MMAs each, 21 us of
+  // tensor time on half the SMs against 10.5 us on all of them; h5.box.0, n20, h4.box.1, n13.cv1, b9.cv2 likewise) made
+  // those launches alone 43 -> 28, 30 -> 21, 27 -> 21, 27 -> 19, 37 -> 28, 24 -> 21 us and one runner alone 32.0k -> 32.5k
+  // frames/s, but four runners 39.1k -> 38.2k and e2e 35.9k -> 35.6k: side by side on disjoint SMs beats taking turns.
+  static const bool tiny_on = [] { const char* e = getenv("XRSEG_TINY_GRID"); return !(e && e[0] == '0'); }();
+  const int cap = num_sms / 2;
+  const int work = p.m_tiles * p.n_tiles;
+  if (tiny_on && tma && p.grid > cap && work <= (p.mode == MODE_FLAT_TMA ? 800 : 296)) p.grid = cap;
+  return p;
+}
 
 // ---------------------------------------------------------------------------------------------------------------
 // XRSW weight pack (written by xr_image_segmentation_b200/weights.py)

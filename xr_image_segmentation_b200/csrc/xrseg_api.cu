@@ -25,6 +25,7 @@
 #include "bottleneck.cuh"
 
 using namespace xrseg;
+static_assert(NC == 80, "model.cuh decode_variant names the class count decode_filter_kernel is specialised for");
 
 namespace {
 
@@ -48,10 +49,12 @@ struct DevLayer {
 };
 
 // ---- fused Bottleneck (bottleneck.cuh): one instantiation per supported channel triple ---------------------------------
+constexpr int BNECK_TH = 14;   // output rows per CTA of every instantiation
+dim3 bneck_grid(const BneckParams& p, int th) { return dim3(ceil_div(p.W, BNECK_TW), ceil_div(p.H, th), p.B); }
 template <int C1, int CM, int C2, int TH>
 void bneck_launch_t(const BneckParams& p, bool res, cudaStream_t st) {
   using Cfg = BneckCfg<C1, CM, C2, TH>;
-  const dim3 grid(ceil_div(p.W, BNECK_TW), ceil_div(p.H, TH), p.B);
+  const dim3 grid = bneck_grid(p, TH);
   if (res) launch_k(bottleneck_mma_kernel<C1, CM, C2, TH, true>, grid, 256, Cfg::SMEM_BYTES, st, p);
   else launch_k(bottleneck_mma_kernel<C1, CM, C2, TH, false>, grid, 256, Cfg::SMEM_BYTES, st, p);
 }
@@ -62,12 +65,12 @@ void bneck_prepare_t() {
   XR_CUDA(cudaFuncSetAttribute(bottleneck_mma_kernel<C1, CM, C2, TH, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
 }
 void bneck_prepare_device() {
-  bneck_prepare_t<16, 8, 16, 14>();
-  bneck_prepare_t<32, 16, 32, 14>();
+  bneck_prepare_t<16, 8, 16, BNECK_TH>();
+  bneck_prepare_t<32, 16, 32, BNECK_TH>();
 }
 void launch_bneck(int c1, int cm, int c2, const BneckParams& p, bool res, cudaStream_t st) {
-  if (c1 == 16 && cm == 8 && c2 == 16) bneck_launch_t<16, 8, 16, 14>(p, res, st);
-  else if (c1 == 32 && cm == 16 && c2 == 32) bneck_launch_t<32, 16, 32, 14>(p, res, st);
+  if (c1 == 16 && cm == 8 && c2 == 16) bneck_launch_t<16, 8, 16, BNECK_TH>(p, res, st);
+  else if (c1 == 32 && cm == 16 && c2 == 32) bneck_launch_t<32, 16, 32, BNECK_TH>(p, res, st);
   else XR_CHECK(false, "no fused Bottleneck kernel for %d-%d-%d channels", c1, cm, c2);
 }
 
@@ -78,10 +81,6 @@ bool branches_disabled() {   // XRSEG_BRANCHES=0: everything on one stream (A/B 
 bool mask_mma_enabled() {
   const char* e = getenv("XRSEG_MASK_MMA");
   return !(e && e[0] == '0');
-}
-bool s2_tma_disabled() {
-  const char* e = getenv("XRSEG_S2_TMA");
-  return e && e[0] == '0';
 }
 
 template <typename T>
@@ -276,25 +275,15 @@ void upload_layers(xrseg_runner* r, const std::vector<HostLayerWeights>& hw) {
         cout_real = o.y.Cp + l2.cout;
       }
       const HostLayerWeights& wsrc = o.layer2 >= 0 ? fused : w;
-      ConvDesc cd{};
-      cd.B = r->mb; cd.H = o.x.H; cd.W = o.x.W; cd.Cin = o.x.Cp; cd.in_pitch = o.x.pitch;
-      cd.Cout = o.y.Cp + (o.layer2 >= 0 ? o.y2.Cp : 0); cd.out_pitch = o.y.pitch;
-      cd.k = o.k; cd.stride = o.stride; cd.act = o.act; cd.transposed = o.transposed;
-      cd.res_pitch = o.has_res ? o.res.pitch : 0;
-      cd.upm = o.up_layer >= 0 ? 1 : 0;
-      d.use_tma = r->cfg.conv_impl == XRSEG_CONV_UMMA && plan_conv_halo_tma(cd, r->num_sms, d.cp);
-      XR_CHECK(!cd.upm || d.use_tma, "no launch plan for the merged ConvTranspose (%s)", l.name.c_str());
-      if (d.use_tma) {
+      d.use_tma = r->cfg.conv_impl == XRSEG_CONV_UMMA && plan_conv_op(o, r->mb, r->num_sms, d.cp);
+      XR_CHECK(o.up_layer < 0 || (d.use_tma && d.cp.upm), "no launch plan for the merged ConvTranspose (%s)", l.name.c_str());
+      if (d.use_tma && d.cp.mode == MODE_HALO_TMA) {
         d.tmaps.m[0] = make_halo_tensor_map(ptr_of(r, o.x), r->mb, o.x.H, o.x.W, o.x.Cp, o.x.pitch, d.cp.Wp, d.cp.hbox,
                                             d.cp.sw ? d.cp.cb : 8, d.cp.sw);
-      } else if (r->cfg.conv_impl == XRSEG_CONV_UMMA && !flat_tma_disabled() && plan_conv_flat_tma(cd, r->num_sms, d.cp)) {
-        d.use_tma = true;
+      } else if (d.use_tma && d.cp.mode == MODE_FLAT_TMA) {
         d.tmaps.m[0] = make_flat_tensor_map(ptr_of(r, o.x), static_cast<long>(r->mb) * o.x.H * o.x.W, o.x.Cp, o.x.pitch, d.cp);
-      } else if (r->cfg.conv_impl == XRSEG_CONV_UMMA && !s2_tma_disabled() && plan_conv_s2_tma(cd, r->num_sms, d.cp)) {
-        d.use_tma = true;
+      } else if (d.use_tma) {
         d.tmaps = make_s2_tensor_maps(ptr_of(r, o.x), r->mb, o.x.H, o.x.W, o.x.Cp, o.x.pitch, d.cp);
-      } else {
-        d.cp = plan_conv(cd, r->num_sms, 0);
       }
       if (o.tail_layer >= 0) {
         // fused trailing 1x1 (model.cuh: fuse_tail_1x1): W2 as the 128-byte-swizzled image of a 1x1 layer with Ntile = 32, cb = 64
@@ -372,6 +361,7 @@ struct Launch {
   std::function<void(cudaStream_t)> fn;
   double flops = 0, bytes = 0;   // algorithmic work of the launch (real channel counts, fp16 activations)
   int branch = 0, wait_tag = 0, signal_tag = 0;   // see model.cuh Op::branch
+  int grid = 0, items = 0, mode = -1;            // CTAs, work items and conv mode (-1: not a convolution) for xrseg_debug_launches
 };
 
 void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
@@ -443,25 +433,8 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
         L.flops = 2.0 * (o.transposed ? px_in * 4 : px_out) * cout_alg * l.cin * (upm ? 4.0 : taps);
         L.bytes = (px_in * l.cin + px_out * cout_alg * (o.has_res ? 2 : 1) + static_cast<double>(cout_alg) * l.cin * wtaps) * 2;
         if (r->cfg.conv_impl == XRSEG_CONV_UMMA) {
-          ConvParams p = d.cp;
-          if (nb != p.B) p = replan_for_batch(d.cp, nb, r->num_sms);   // partial last chunk: same layout, fewer frames
-          {
-            // Small launches use at most HALF the SMs (XRSEG_TINY_GRID=0 turns it off): 3x3 layers with at most two work items
-            // per SM (296: every 20x20 layer, the 3x3 convs of the 40x40 stage) and 1x1 layers with at most 800 items (the 40x40
-            // stage).  These kernels are latency-bound -- most of their ~10 us is fill
-            // and drain -- and a throughput caller keeps several runners in flight: with half-width grids the small kernels of
-            // two steps sit side by side on disjoint SMs instead of taking turns on all of them.  Measured (B200, batch 64, four
-            // runners, profiles/r2_experiments.md): 34.5k -> 36.7k frames/s, e2e 32.4k -> 34.0k; one runner alone 30.2k -> 29.9k;
-            // batch-1 latency unchanged (its grids are smaller than the cap anyway).
-            // Tensor-heavy layers stay at half width too: keeping them on all SMs (b7: 256 items of 72 N = 256 MMAs each, 21 us of
-            // tensor time on half the SMs against 10.5 us on all of them; h5.box.0, n20, h4.box.1, n13.cv1, b9.cv2 likewise) made
-            // those launches alone 43 -> 28, 30 -> 21, 27 -> 21, 27 -> 19, 37 -> 28, 24 -> 21 us and one runner alone 32.0k -> 32.5k
-            // frames/s, but four runners 39.1k -> 38.2k and e2e 35.9k -> 35.6k: side by side on disjoint SMs beats taking turns.
-            static const bool tiny_on = [] { const char* e = getenv("XRSEG_TINY_GRID"); return !(e && e[0] == '0'); }();
-            const int cap = r->num_sms / 2;
-            const int work = p.m_tiles * p.n_tiles;
-            if (tiny_on && d.use_tma && p.grid > cap && work <= (p.mode == MODE_FLAT_TMA ? 800 : 296)) p.grid = cap;
-          }
+          ConvParams p = conv_launch_params(d.cp, d.use_tma, nb, r->num_sms);
+          L.grid = p.grid; L.items = p.m_tiles * p.n_tiles; L.mode = p.mode;
           p.in = ptr_of(r, o.x); p.out = ptr_of(r, o.y);
           if (o.layer2 >= 0) { p.out2 = ptr_of(r, o.y2); p.split_n = o.y.Cp; p.out2_pitch = o.y2.pitch; }
           p.res = o.has_res ? ptr_of(r, o.res) : nullptr;
@@ -504,6 +477,10 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
         L.name = l.name.substr(0, l.name.size() - 4);          // "b2.m0"
         L.flops = 2.0 * px_out * 9 * (static_cast<double>(l.cin) * l.cout + static_cast<double>(l2.cin) * l2.cout);
         L.bytes = (px_in * l.cin + px_out * l2.cout + 9.0 * (l.cin * l.cout + l2.cin * l2.cout)) * 2;
+        {
+          const dim3 g = bneck_grid(p, BNECK_TH);
+          L.grid = L.items = static_cast<int>(g.x * g.y * g.z);
+        }
         L.fn = [p, c1, cm, c2, res](cudaStream_t st) { launch_bneck(c1, cm, c2, p, res, st); };
         break;
       }
@@ -520,6 +497,7 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
         L.flops = 2.0 * px_out * l.cout * 9;
         L.bytes = (px_in * l.cin + px_out * l.cout * (o.has_res ? 2 : 1)) * 2;
         const dim3 grid(ceil_div(p.W * (p.C / 8), 128), ceil_div(p.H, p.rows), nb);
+        L.grid = L.items = static_cast<int>(grid.x * grid.y * grid.z);
         L.fn = [p, grid](cudaStream_t st) { launch_k(dwconv3x3_kernel<4>, grid, 128, 0, st, p); };
         break;
       }
@@ -528,7 +506,9 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
         const size_t smem = static_cast<size_t>(o.x.H) * o.x.W * 32;
         L.name = "sppf.pool";
         L.bytes = px_in * p.C * 4 * 2;
-        L.fn = [p, nb, smem](cudaStream_t st) { launch_k(sppf_pool_kernel, nb * (p.C / 8), 256, smem, st, p); };
+        const int ctas = nb * (p.C / 8);
+        L.grid = L.items = ctas;
+        L.fn = [p, ctas, smem](cudaStream_t st) { launch_k(sppf_pool_kernel, ctas, 256, smem, st, p); };
         break;
       }
       case OP_UP: {
@@ -536,6 +516,7 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
         const dim3 grid(ceil_div(o.x.W * (o.x.Cp / 8), 256), o.x.H, nb);
         L.name = "upsample2x";
         L.bytes = px_in * o.x.C * 5 * 2;
+        L.grid = L.items = static_cast<int>(grid.x * grid.y * grid.z);
         L.fn = [p, grid](cudaStream_t st) { launch_k(upsample2x_kernel, grid, 256, 0, st, p); };
         break;
       }
@@ -551,6 +532,7 @@ void add_network_launches(xrseg_runner* r, int nb, std::vector<Launch>& out) {
         L.flops = 2.0 * nb * o.heads * static_cast<double>(p.N) * p.N * (ATT_KD + ATT_HD) +
                   (o.layer >= 0 ? 2.0 * px_out * o.y.C * 9 : 0.0);
         L.bytes = px_in * (o.x.C + o.y.C) * 2;
+        L.grid = L.items = static_cast<int>(g.x * g.y);
         L.fn = [p, g, smem, threads](cudaStream_t st) { launch_k(attention_kernel, g, threads, smem, st, p); };
         break;
       }
@@ -649,9 +631,10 @@ void add_post_launches(xrseg_runner* r, int b0, int nb, const ScaleSrc<T> (&src)
     for (int i = 0; i < 3; ++i)
       XR_CHECK(src[i].cls_pitch == pitch && pitch % EPC == 0 && pitch >= r->nc && pitch <= NC_MAX, "class tensor pitch %d", src[i].cls_pitch);
     const dim3 grid(ceil_div(A, 256), nb);
-    if (r->nc == NC) {            // the COCO models: the kernel specialised for 80 classes
+    const int variant = decode_variant(r->nc, pitch, EPC);
+    if (variant == DECODE_80) {   // the COCO models: the kernel specialised for 80 classes
       L.fn = [dp, grid](cudaStream_t st) { launch_k(decode_filter_kernel<T>, grid, 256, 0, st, dp); };
-    } else if (pitch / EPC <= 32) {
+    } else if (variant == DECODE_TABLE) {
       const size_t smem = static_cast<size_t>(8) * 32 * (pitch / EPC) * sizeof(float);
       L.fn = [dp, grid, smem](cudaStream_t st) { launch_k(decode_filter_nc_kernel<T>, grid, 256, smem, st, dp); };
     } else {
@@ -1809,7 +1792,12 @@ int xrseg_profile_ops(xrseg_runner* r, int iters, float* ms, char* names, double
 // ---- debug / parity: exported by libxrseg_debug.so only (include/xrseg_debug.h) -----------------------------------------
 #ifdef XRSEG_DEBUG_API
 int xrseg_debug_fetch(xrseg_runner* r, const char* name, float* dst, size_t cap_floats, int64_t* shape4) {
-  if (!r || !name || !dst) return XRSEG_ERR_INVALID;
+  return xrseg_debug_fetch_frames(r, name, 0, -1, dst, cap_floats, shape4);
+}
+
+int xrseg_debug_fetch_frames(xrseg_runner* r, const char* name, int first, int count, float* dst, size_t cap_floats,
+                             int64_t* shape4) {
+  if (!r || !name || !dst || first < 0) return XRSEG_ERR_INVALID;
   int rc = finish(r);
   if (rc < 0) return rc;
   Net& net = *r->net;
@@ -1828,15 +1816,18 @@ int xrseg_debug_fetch(xrseg_runner* r, const char* name, float* dst, size_t cap_
   }
   C = t.C;
   // the arena holds the LAST micro-batch of the run: frames (n_chunks - 1) * mb .. batch - 1
-  const int nb = r->batch > 0 ? r->batch - (ceil_div(r->batch, r->mb) - 1) * r->mb : 0;
+  const int resident = r->batch > 0 ? r->batch - (ceil_div(r->batch, r->mb) - 1) * r->mb : 0;
+  if (count < 0) count = resident - first;
+  if (count <= 0 || first + count > resident) { r->err = "no frames, or frames outside the resident chunk"; return XRSEG_ERR_INVALID; }
+  const int nb = count;
   const size_t n = static_cast<size_t>(nb) * C * t.H * t.W;
   if (shape4) { shape4[0] = nb; shape4[1] = C; shape4[2] = t.H; shape4[3] = t.W; }
   if (cap_floats < n) { r->err = "fetch buffer too small"; return XRSEG_ERR_CAPACITY; }
   try {
     XR_CUDA(cudaSetDevice(r->device));
     float* d = dev_alloc<float>(n);
-    nhwc_f16_to_nchw_f32_kernel<<<grid_for(static_cast<long>(n)), 256, 0, r->stream>>>(ptr_of(r, t), d, nb, C, t.H, t.W,
-                                                                                      t.pitch);
+    const __half* src = ptr_of(r, t) + static_cast<size_t>(first) * t.H * t.W * t.pitch;
+    nhwc_f16_to_nchw_f32_kernel<<<grid_for(static_cast<long>(n)), 256, 0, r->stream>>>(src, d, nb, C, t.H, t.W, t.pitch);
     XR_CUDA(cudaMemcpyAsync(dst, d, n * sizeof(float), cudaMemcpyDeviceToHost, r->stream));
     XR_CUDA(cudaStreamSynchronize(r->stream));
     cudaFree(d);
@@ -1851,6 +1842,25 @@ int xrseg_debug_fetch(xrseg_runner* r, const char* name, float* dst, size_t cap_
     return XRSEG_ERR_CUDA;
   }
   return XRSEG_OK;
+}
+
+int xrseg_debug_launches(xrseg_runner* r, int* grid, int* items, int* mode, char* names, int cap) {
+  if (!r || !grid || !items || !mode) return XRSEG_ERR_INVALID;
+  int rc = finish(r);
+  if (rc < 0) return rc;
+  if (r->batch < 1) { r->err = "no run"; return XRSEG_ERR_STATE; }
+  const int b0 = (ceil_div(r->batch, r->mb) - 1) * r->mb, nb = r->batch - b0;
+  const std::vector<Launch>* ls = nullptr;
+  for (auto& c : r->launch_cache)
+    if (c.b0 == b0 && c.nb == nb) ls = static_cast<const std::vector<Launch>*>(c.list);
+  if (!ls) { r->err = "the last chunk ran without a launch list"; return XRSEG_ERR_STATE; }
+  if (static_cast<int>(ls->size()) > cap) { r->err = "launch buffers too small"; return XRSEG_ERR_CAPACITY; }
+  for (size_t i = 0; i < ls->size(); ++i) {
+    const Launch& L = (*ls)[i];
+    grid[i] = L.grid; items[i] = L.items; mode[i] = L.mode;
+    if (names) { memset(names + i * 32, 0, 32); strncpy(names + i * 32, L.name.c_str(), 31); }
+  }
+  return static_cast<int>(ls->size());
 }
 
 static int debug_post_impl(xrseg_runner* r, const float* box_logits, const float* cls_logits, const float* coefs,

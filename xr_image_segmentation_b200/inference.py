@@ -303,18 +303,28 @@ class Runner:
         return [(names.raw[i * 32:(i + 1) * 32].split(b"\0")[0].decode(), ms[i], fl[i], by[i]) for i in range(n)]
 
     # ---- parity / debug ----
-    def fetch(self, name: str) -> np.ndarray:
+    def fetch(self, name: str, first: int = 0, count: int = -1) -> np.ndarray:
+        """A named activation of the last run, frames [first, first + count) of the resident chunk (count -1: all)."""
         self._need_debug()
         shp = (C.c_int64 * 4)()
         probe = np.empty(1, np.float32)                  # a zero-capacity call reports the shape (class logits grow with nc)
-        rc = self.lib.xrseg_debug_fetch(self.h, name.encode(), probe.ctypes.data, 0, shp)
+        rc = self.lib.xrseg_debug_fetch_frames(self.h, name.encode(), first, count, probe.ctypes.data, 0, shp)
         if rc != _lib.ERR_CAPACITY:
             self._ck(rc)
         shape = [int(s) for s in shp]
         n = int(np.prod(shape))
         buf = np.empty(max(n, 1), np.float32)
-        self._ck(self.lib.xrseg_debug_fetch(self.h, name.encode(), buf.ctypes.data, n, shp))
+        self._ck(self.lib.xrseg_debug_fetch_frames(self.h, name.encode(), first, count, buf.ctypes.data, n, shp))
         return buf[:n].reshape(shape)
+
+    def launches(self) -> list[tuple[str, int, int, int]]:
+        """The last run's launch list (resident chunk): (name, grid CTAs, work items, conv mode or -1) per launch."""
+        self._need_debug()
+        cap = 512
+        g, it, md = (C.c_int * cap)(), (C.c_int * cap)(), (C.c_int * cap)()
+        names = C.create_string_buffer(cap * 32)
+        n = self._ck(self.lib.xrseg_debug_launches(self.h, g, it, md, names, cap))
+        return [(names.raw[i * 32:(i + 1) * 32].split(b"\0")[0].decode(), g[i], it[i], md[i]) for i in range(n)]
 
     def debug_post(self, box_logits, cls_logits, coefs, protos, f16=False):
         """Post-processing alone on caller tensors: fp32 bit-exact kernels, or (f16) the product's fp16 kernels."""
